@@ -73,6 +73,9 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--small", action="store_true", help="reduced tessellation (debugging only; reported in config)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned to its caller as DIR/<name>.npy "
+                         "(the float32 accumulation image), so that two builds can be compared output for output")
     args = ap.parse_args()
     scenes = importlib.import_module("path-tracing_b200.scenes")
     _, _, w, h, spp, depth = scenes.WORKLOADS[args.workload]
@@ -153,6 +156,23 @@ class ClockSampler:
             "samples": len(sm),
             "reasons": sorted(reasons),
         }
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(directory: str, arrays: dict):
+    """Writes each (H, W, C) array as directory/<name>.npy in float32.  Arrays of more than DUMP_BYTES in all are each
+    replaced by a fixed, seeded sample of their pixels, the same on every run (rows of the (H*W, C) view, in pixel order)."""
+    os.makedirs(directory, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        a = np.asarray(a, np.float32)
+        if total > DUMP_BYTES:
+            flat = a.reshape(a.shape[0] * a.shape[1], -1)
+            keep = int(len(flat) * DUMP_BYTES / total)
+            a = flat[np.sort(np.random.default_rng(0).choice(len(flat), keep, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 class CudaArray:
@@ -299,10 +319,12 @@ def run_reference(args):
     rays = samples = 0
     t0 = time.perf_counter()
     for k in range(args.steps):
-        _, cnt = o.render(params, args.width, args.height, k * step_spp, step_spp, tiles=tiles, threads=threads)
+        image, cnt = o.render(params, args.width, args.height, k * step_spp, step_spp, tiles=tiles, threads=threads)
         rays += cnt["rays_closest"] + cnt["rays_shadow"]
         samples += cnt["samples"]
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"accumulation": image})
     value = rays / dt / 1e6
     line = {
         "impl": "reference",
@@ -428,6 +450,9 @@ def run_ours(args):
 
     head_kind = "weak" if (args.scaling == "weak" and world > 1) else "strong"
     head = measure(head_kind)
+    if args.dump_outputs and rank == 0:
+        # the last timed step's (reduced) image, written before the weak arrangement reads back into host_img
+        dump_outputs(args.dump_outputs, {"accumulation": host_img.numpy()})
     other = None
     if world > 1 and args.scaling == "both":
         other = measure("weak")

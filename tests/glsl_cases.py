@@ -1,7 +1,11 @@
 """The cases the oracle is compared on with the reference's compiled shaders (oracle/_ref/libglsl_ref.so):
 shared by tests/test_oracle_vs_glsl.py (live comparison, where the library exists) and
-tests/golden/make_glsl_vectors.py (golden vectors that travel to machines without the reference)."""
+tests/golden/make_glsl_vectors.py (golden vectors that travel to machines without the reference), and the recorded
+digests that let the live comparisons of test_oracle_vs_glsl.py and test_oracle_vs_glsl_compute.py run without it."""
+import hashlib
 import importlib
+import json
+import os
 
 import numpy as np
 
@@ -62,3 +66,33 @@ DEBUG_GOLDEN = (("default", "color", 0, 0), ("feature", "color", 0, 0), ("featur
 
 def debug_key(scene, mode, raygen_flags, hit_flags):
     return f"dbg_{scene}_{mode}_{raygen_flags}_{hit_flags}"
+
+
+# ---- recorded outputs of the compiled shaders (tests/golden/glsl_digests.json, make_glsl_digests.py) --------------------
+DIGESTS_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "glsl_digests.json")
+RECORD = os.environ.get("PT_RECORD_GLSL_DIGESTS") == "1"
+
+
+def digest(a) -> str:
+    """SHA-256 of a float32 array's shape and bits, every NaN written as one NaN (the comparisons let any NaN equal any NaN)."""
+    a = np.array(a, np.float32)
+    a[np.isnan(a)] = np.nan
+    return hashlib.sha256(repr(a.shape).encode() + a.tobytes()).hexdigest()
+
+
+def check_recorded(key, got, want, compare, what):
+    """`got` (the oracle's) against the compiled shaders' output on the same input.  Where the library is built, `want` is
+    that output: compare(got, want, what), and the digest recorded under `key` must still be want's.  Without the library
+    `want` is None and got's digest must be the recorded one."""
+    if want is not None:
+        compare(got, want, what)
+    value = digest(got if want is None else want)
+    recorded = json.load(open(DIGESTS_PATH)) if os.path.exists(DIGESTS_PATH) else {}
+    if RECORD:
+        recorded[key] = value
+        with open(DIGESTS_PATH, "w") as f:
+            json.dump(recorded, f, indent=1, sort_keys=True)
+            f.write("\n")
+        return
+    assert value == recorded[key], (f"{what}: not the compiled shaders' output recorded in tests/golden/glsl_digests.json "
+                                    f"under '{key}'" + (" (the record is stale: tests/golden/make_glsl_digests.py)" if want is not None else ""))

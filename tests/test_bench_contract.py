@@ -4,6 +4,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 import conftest
 
 
@@ -21,6 +23,20 @@ def test_reference_arm_line():
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] == line["value"] and "96x54" in cb["sample"]
     assert line["e2e"] == {"value": line["value"], "unit": "Mrays/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert line["gpu_launches"] == 0
+
+
+def test_reference_arm_dumps_the_last_step(tmp_path):
+    outs = []
+    for run in ("a", "b"):
+        out = subprocess.run([sys.executable, os.path.join(conftest.ROOT, "bench.py"), "--impl", "reference", "--small", "--width", "96",
+                              "--height", "54", "--steps", "2", "--warmup", "1", "--dump-outputs", str(tmp_path / run)],
+                             capture_output=True, text=True, timeout=300, cwd=conftest.ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert os.listdir(tmp_path / run) == ["accumulation.npy"]
+        outs.append(np.load(tmp_path / run / "accumulation.npy"))
+    assert outs[0].dtype == np.float32 and outs[0].shape == (54, 96, 4)
+    assert np.isfinite(outs[0]).all() and outs[0][..., :3].max() > 0
+    assert np.array_equal(outs[0], outs[1])
 
 
 def test_reference_arm_other_ranks_exit_quietly():

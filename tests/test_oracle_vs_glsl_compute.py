@@ -13,12 +13,15 @@ This pin found one discrepancy when it was first run: `boneWeight * vec4(Positio
 groups from the left — the weighted point goes through the matrix — where oracle and core weighted the transformed
 point (last bit of x / y on every second vertex).  Both follow the shader now.
 
-Without the reference checkout the committed vectors of tests/golden/glsl_compute_vectors.npz pin the oracle."""
+Without the reference checkout the committed vectors of tests/golden/glsl_compute_vectors.npz pin the oracle, and the
+comparisons with the compiled shaders compare with the SHA-256 of their output on the same inputs, recorded in
+tests/golden/glsl_digests.json (make_glsl_digests.py)."""
 import os
 
 import numpy as np
 import pytest
 
+import glsl_cases as gc
 import glsl_compute_cases as cc
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -27,11 +30,17 @@ GOLDEN = os.path.join(ROOT, "tests", "golden", "glsl_compute_vectors.npz")
 
 @pytest.fixture(scope="module")
 def glsl():
+    """The compiled shaders, or None where libglsl_comp_ref.so is not built: the recorded digests stand in for their outputs."""
     from oracle import glsl_ref
 
-    if not glsl_ref.comp_available():
+    return glsl_ref if glsl_ref.comp_available() else None
+
+
+@pytest.fixture(scope="module")
+def live_glsl(glsl):
+    if glsl is None:
         pytest.skip("libglsl_comp_ref.so not built and no reference checkout (golden vectors still pin the oracle)")
-    return glsl_ref
+    return glsl
 
 
 @pytest.fixture(scope="module")
@@ -45,6 +54,11 @@ def assert_same_bits(got, want, what):
     diff = got.view(np.uint32) != want.view(np.uint32)
     diff &= ~(np.isnan(got) & np.isnan(want))  # any NaN equals any NaN
     assert not diff.any(), f"{what}: {int(diff.sum())} of {diff.size} floats differ, first at {np.argwhere(diff)[:4].tolist()}"
+
+
+def assert_shader_bits(key, got, want, what):
+    """got == want bit for bit; with want None (no library), got == the compiled shaders' output recorded under key."""
+    gc.check_recorded(key, got, want, assert_same_bits, what)
 
 
 def oracle_post(oracle_mod, name):
@@ -68,44 +82,49 @@ def test_skinning_matches_the_golden_vectors(oracle_mod, golden, angle):
     assert_same_bits(oracle_mod.skin_vertices(*cc.skin_case(angle)), golden[f"skin_{angle}"], f"skinning.comp at {angle} degrees")
 
 
-# ---- the compiled shaders themselves (where the reference checkout is) ----------------------------------------------
-def test_golden_vectors_are_current(glsl, golden):
+# ---- the compiled shaders: live where the library is built, else their recorded digests ----------------------------
+def test_golden_vectors_are_current(live_glsl, golden):
     for name in cc.GOLDEN_POST:
         acc, total, exposure, threshold, intensity = cc.post_case(name)
-        b0, composed, final = glsl.postprocess(acc, total, exposure, threshold, intensity, tone_mapping_hdr=False)
+        b0, composed, final = live_glsl.postprocess(acc, total, exposure, threshold, intensity, tone_mapping_hdr=False)
         assert_same_bits(composed, golden[f"post_{name}_composed"], name)
         assert_same_bits(final, golden[f"post_{name}_final"], name)
         assert_same_bits(b0, golden[f"post_{name}_bloom0"], name)
     for angle in cc.SKIN_ANGLES:
-        assert_same_bits(glsl.skin_vertices(*cc.skin_case(angle)), golden[f"skin_{angle}"], f"skin {angle}")
+        assert_same_bits(live_glsl.skin_vertices(*cc.skin_case(angle)), golden[f"skin_{angle}"], f"skin {angle}")
 
 
 @pytest.mark.parametrize("case", [c[0] for c in cc.POST_CASES])
 def test_postprocess_chain_bitwise(glsl, oracle_mod, case):
     acc, total, exposure, threshold, intensity = cc.post_case(case)
     composed, final = oracle_post(oracle_mod, case)
-    _, g_composed, g_final = glsl.postprocess(acc, total, exposure, threshold, intensity, tone_mapping_hdr=False)
-    assert_same_bits(composed[..., :3], g_composed[..., :3], f"{case}: after composition.comp")
-    assert_same_bits(final[..., :3], g_final[..., :3], f"{case}: after toneMapping.comp")
-    # toneMapping.comp in HDR mode is the identity
-    _, _, g_hdr = glsl.postprocess(acc, total, exposure, threshold, intensity, tone_mapping_hdr=True)
-    assert_same_bits(g_hdr, g_composed, f"{case}: HDR tone mapping")
+    g = glsl and glsl.postprocess(acc, total, exposure, threshold, intensity, tone_mapping_hdr=False)
+    assert_shader_bits(f"post_{case}_composed", composed[..., :3], g and g[1][..., :3], f"{case}: after composition.comp")
+    assert_shader_bits(f"post_{case}_final", final[..., :3], g and g[2][..., :3], f"{case}: after toneMapping.comp")
+    if glsl:
+        # toneMapping.comp in HDR mode is the identity
+        _, _, g_hdr = glsl.postprocess(acc, total, exposure, threshold, intensity, tone_mapping_hdr=True)
+        assert_same_bits(g_hdr, g[1], f"{case}: HDR tone mapping")
 
 
-def test_postprocess_marks_nan_and_inf_like_the_shader(glsl):
+def test_postprocess_marks_nan_and_inf_like_the_shader(glsl, oracle_mod):
+    """On the shader's image where the library is built, and on the oracle's."""
     acc, total, exposure, threshold, intensity = cc.post_case("defaults_96x54")
-    _, composed, _ = glsl.postprocess(acc, total, exposure, 1e9, 0.0, tone_mapping_hdr=True)  # no bloom contribution
+    images = [oracle_mod.postprocess(acc, total, exposure, 1e9, 0.0, hdr=True)]  # no bloom contribution
+    if glsl:
+        images.append(glsl.postprocess(acc, total, exposure, 1e9, 0.0, tone_mapping_hdr=True)[1])
     h, w = acc.shape[:2]
-    assert composed[h // 2, w // 3, :3].tolist() == [5000.0, 0.0, 0.0]  # NaN -> red (postprocess.comp:24-25)
-    assert composed[h // 3, w // 2, :3].tolist() == [0.0, 5000.0, 0.0]  # Inf -> green (:26-27)
-    assert np.isinf(composed[h - 1, w - 1, :3]).all()  # finite in fp32, beyond binary16: the store overflows
+    for composed in images:
+        assert composed[h // 2, w // 3, :3].tolist() == [5000.0, 0.0, 0.0]  # NaN -> red (postprocess.comp:24-25)
+        assert composed[h // 3, w // 2, :3].tolist() == [0.0, 5000.0, 0.0]  # Inf -> green (:26-27)
+        assert np.isinf(composed[h - 1, w - 1, :3]).all()  # finite in fp32, beyond binary16: the store overflows
 
 
 @pytest.mark.parametrize("angle", [0.0, 5.0, 12.0, 47.5, 90.0, -33.0])
 def test_skinning_bitwise(glsl, oracle_mod, angle):
     animated, idx, bones = cc.skin_case(angle)
-    assert_same_bits(oracle_mod.skin_vertices(animated, idx, bones), glsl.skin_vertices(animated, idx, bones),
-                     f"skinning.comp at {angle} degrees")
+    assert_shader_bits(f"skin_{angle}", oracle_mod.skin_vertices(animated, idx, bones), glsl and glsl.skin_vertices(animated, idx, bones),
+                       f"skinning.comp at {angle} degrees")
 
 
 def test_skinning_random_bones_bitwise(glsl, oracle_mod):
@@ -116,4 +135,5 @@ def test_skinning_random_bones_bitwise(glsl, oracle_mod):
     animated["bone_weights"] = rng.random(animated["bone_weights"].shape, dtype=np.float32) * 0.6
     bones = (rng.standard_normal((4, 12)) * 0.7).astype(np.float32)
     bones[:, [0, 5, 10]] += 1.5  # keep the linear part invertible
-    assert_same_bits(oracle_mod.skin_vertices(animated, idx, bones), glsl.skin_vertices(animated, idx, bones), "random bones")
+    assert_shader_bits("skin_random_bones", oracle_mod.skin_vertices(animated, idx, bones), glsl and glsl.skin_vertices(animated, idx, bones),
+                       "random bones")
