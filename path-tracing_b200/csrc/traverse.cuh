@@ -110,7 +110,14 @@ struct RaySetup
 #endif
 };
 
-PT_DEV float comp(vec3 v, int k) { return k == 0 ? v.x : (k == 1 ? v.y : v.z); }
+// v[k] as two selects (FSEL) on predicates that depend on the ray only.  Written as the nested
+// k == 0 ? v.x : (k == 1 ? v.y : v.z), ptxas made every one of the watertight test's nine components a divergent
+// branch (BSSY / BRA / BSYNC; 7.6 % of k_extend's instructions at 14 of 32 lanes).
+PT_DEV float comp(vec3 v, int k)
+{
+    const float yz = k == 1 ? v.y : v.z;
+    return k == 0 ? v.x : yz;
+}
 
 PT_DEV RaySetup setupRay(vec3 o, vec3 d)
 {
@@ -336,15 +343,14 @@ PT_DEV void intersectNode(const BvhNode *__restrict__ node, const RaySetup &r, f
 
 #endif
 
+// distances by min / max, references by one compare and two selects (an if-swap compiled to eight moves);
+// the distances are never NaN, so min / max order them as the compare does
 #define PT_CSWAP(i, j)                                                                                                \
-    if (d[j] < d[i])                                                                                                  \
     {                                                                                                                 \
-        const float td = d[i];                                                                                        \
-        d[i] = d[j];                                                                                                  \
-        d[j] = td;                                                                                                    \
-        const int tc = c[i];                                                                                          \
-        c[i] = c[j];                                                                                                  \
-        c[j] = tc;                                                                                                    \
+        const bool sw = d[j] < d[i];                                                                                  \
+        const int ci = sw ? c[j] : c[i], cj = sw ? c[i] : c[j];                                                       \
+        const float di = fminf(d[i], d[j]), dj = fmaxf(d[i], d[j]);                                                   \
+        d[i] = di, d[j] = dj, c[i] = ci, c[j] = cj;                                                                   \
     }
 
 // cur value "take the next entry off the stack": popping is a step of the state machine of its own
@@ -489,6 +495,26 @@ template <bool CLOSEST, bool ALPHA, bool STATS, int SMEM = 0, bool CULL = false>
             return;
         }
         cur = c[0];
+        // the hit children are d[0 .. m]: the rest goes on the stack farthest first, as predicated stores below one
+        // bound check (three conditional pushes were three branches with a bound check each)
+        const bool h1 = d[1] != INFINITY, h2 = d[2] != INFINITY, h3 = d[3] != INFINITY;
+        const int m = (int)h1 + (int)h2 + (int)h3;
+        if (SMEM == 0 && sp + m <= PT_STACK_SIZE)
+        {
+            unsigned long long *top = stack + sp + m; // one past the new top
+            if (h1)
+                top[-1] = ((unsigned long long)__float_as_uint(d[1]) << 32) | (uint32_t)c[1];
+            if (h2)
+                top[-2] = ((unsigned long long)__float_as_uint(d[2]) << 32) | (uint32_t)c[2];
+            if (h3)
+                top[-3] = ((unsigned long long)__float_as_uint(d[3]) << 32) | (uint32_t)c[3];
+            sp += m;
+#if PT_PREFETCH_PUSH
+            if (h1 && c[1] >= 0)
+                prefetchL1(s.nodes + c[1]);
+#endif
+            return;
+        }
         // push the rest, farthest first
         if (d[3] != INFINITY)
             push(c[3], d[3]);
