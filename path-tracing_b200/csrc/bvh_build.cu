@@ -120,18 +120,14 @@ __global__ void k_bake(const MeshInstance *__restrict__ mis, uint32_t miCount, c
     ts.a[6] = make_float4(bit[2][0], bit[2][1], bit[2][2], uv[0][0]);
     ts.a[7] = make_float4(uv[0][1], uv[1][0], uv[1][1], uv[2][0]);
     ts.a[8] = make_float4(uv[2][1], __uint_as_float(mi.instance), __uint_as_float(mi.geometry), __uint_as_float(prim));
-#if PT_SHADE_UNIT_NORMALS
-    {
-        const vec3 u0 = normalize(V3(nrm[0][0], nrm[0][1], nrm[0][2])), u1 = normalize(V3(nrm[1][0], nrm[1][1], nrm[1][2]));
-        const vec3 u2 = normalize(V3(nrm[2][0], nrm[2][1], nrm[2][2]));
-        const vec3 w0 = V3(pos[0][0], pos[0][1], pos[0][2]), w1 = V3(pos[1][0], pos[1][1], pos[1][2]);
-        const vec3 w2 = V3(pos[2][0], pos[2][1], pos[2][2]);
-        const vec3 g = normalize(cross(w1 - w0, w2 - w0));
-        ts.a[9] = make_float4(u0.x, u0.y, u0.z, u1.x);
-        ts.a[10] = make_float4(u1.y, u1.z, u2.x, u2.y);
-        ts.a[11] = make_float4(u2.z, g.x, g.y, g.z);
-    }
-#endif
+    const vec3 u0 = normalize(V3(nrm[0][0], nrm[0][1], nrm[0][2])), u1 = normalize(V3(nrm[1][0], nrm[1][1], nrm[1][2]));
+    const vec3 u2 = normalize(V3(nrm[2][0], nrm[2][1], nrm[2][2]));
+    const vec3 w0 = V3(pos[0][0], pos[0][1], pos[0][2]), w1 = V3(pos[1][0], pos[1][1], pos[1][2]);
+    const vec3 w2 = V3(pos[2][0], pos[2][1], pos[2][2]);
+    const vec3 g = normalize(cross(w1 - w0, w2 - w0));
+    ts.a[9] = make_float4(u0.x, u0.y, u0.z, u1.x);
+    ts.a[10] = make_float4(u1.y, u1.z, u2.x, u2.y);
+    ts.a[11] = make_float4(u2.z, g.x, g.y, g.z);
     triShade[tri] = ts;
 
     Aabb b;
@@ -566,10 +562,9 @@ __global__ void k_ploc_merge(const int *__restrict__ clusters, uint32_t m, const
 }
 
 // Writes one wide node from the exact child boxes (empty slots: lo = +inf, hi = -inf, ref = PT_CHILD_EMPTY).
-__device__ __forceinline__ void writeWideNode(BvhNode *dst, const float lo[3][4], const float hi[3][4], const int ref[4], int cc)
+__device__ __forceinline__ void writeWideNode(BvhNode *dst, const float lo[3][4], const float hi[3][4], const int ref[4])
 {
     BvhNode out;
-#if PT_QNODES
     float o[3], step[3];
     uint32_t qlo[3] = { 0, 0, 0 }, qhi[3] = { 0, 0, 0 };
     for (int j = 0; j < 3; j++)
@@ -613,17 +608,6 @@ __device__ __forceinline__ void writeWideNode(BvhNode *dst, const float lo[3][4]
     out.qlox = qlo[0], out.qloy = qlo[1], out.qloz = qlo[2];
     out.qhix = qhi[0], out.qhiy = qhi[1], out.qhiz = qhi[2];
     out.child = make_int4(ref[0], ref[1], ref[2], ref[3]);
-    (void)cc;
-#else
-    out.lox = make_float4(lo[0][0], lo[0][1], lo[0][2], lo[0][3]);
-    out.loy = make_float4(lo[1][0], lo[1][1], lo[1][2], lo[1][3]);
-    out.loz = make_float4(lo[2][0], lo[2][1], lo[2][2], lo[2][3]);
-    out.hix = make_float4(hi[0][0], hi[0][1], hi[0][2], hi[0][3]);
-    out.hiy = make_float4(hi[1][0], hi[1][1], hi[1][2], hi[1][3]);
-    out.hiz = make_float4(hi[2][0], hi[2][1], hi[2][2], hi[2][3]);
-    out.child = make_int4(ref[0], ref[1], ref[2], ref[3]);
-    out.pad = make_int4(cc, 0, 0, 0);
-#endif
     *dst = out;
 }
 
@@ -631,7 +615,7 @@ __device__ __forceinline__ void writeWideNode(BvhNode *dst, const float lo[3][4]
 // final order).  Children are opened largest-area first until the node is 4 wide; sub-trees of
 // <= PT_MAX_LEAF_TRIS primitives become leaves.  The triangles are laid out depth first: child k
 // starts where child k - 1 ends, and a leaf writes the source indices of its triangles to
-// order[first ...] (k_gather moves the triangle data afterwards).
+// order[first ...] (k_gather moves the triangle positions afterwards).
 __global__ void k_collapse(Bvh2 t, int n, const uint4 *__restrict__ work, uint32_t workCount, uint4 *__restrict__ next,
                            uint32_t *__restrict__ nextCount, BvhNode *__restrict__ nodes, uint32_t *__restrict__ nodeCount,
                            const uint32_t *__restrict__ sortedIdx, uint32_t *__restrict__ order)
@@ -719,7 +703,7 @@ __global__ void k_collapse(Bvh2 t, int n, const uint4 *__restrict__ work, uint32
         }
         first += count;
     }
-    writeWideNode(nodes + dst, lo, hi, ref, cc);
+    writeWideNode(nodes + dst, lo, hi, ref);
 }
 
 // root of a scene whose whole BVH2 is one leaf (1..PT_MAX_LEAF_TRIS primitives)
@@ -746,12 +730,11 @@ __global__ void k_single_leaf_root(const Aabb *__restrict__ primBoxes, const uin
             lo[j][i] = i == 0 ? m.lo[j] : INFINITY;
             hi[j][i] = i == 0 ? m.hi[j] : -INFINITY;
         }
-    writeWideNode(nodes, lo, hi, ref, 1);
+    writeWideNode(nodes, lo, hi, ref);
 }
 
 __global__ void k_gather(const uint32_t *__restrict__ sortedIdx, const uint32_t *__restrict__ refTri, uint32_t n,
-                         const float4 *__restrict__ posIn, const TriShade *__restrict__ shadeIn, float4 *__restrict__ posOut,
-                         TriShade *__restrict__ shadeOut)
+                         const float4 *__restrict__ posIn, float4 *__restrict__ posOut)
 {
     const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= n)
@@ -761,8 +744,6 @@ __global__ void k_gather(const uint32_t *__restrict__ sortedIdx, const uint32_t 
     posOut[3 * (size_t)k + 0] = posIn[3 * (size_t)src + 0];
     posOut[3 * (size_t)k + 1] = posIn[3 * (size_t)src + 1];
     posOut[3 * (size_t)k + 2] = posIn[3 * (size_t)src + 2];
-    if (shadeOut)
-        shadeOut[k] = shadeIn[src];
 }
 
 
@@ -892,16 +873,12 @@ pt_status buildAccel(Context *ctx, const std::vector<MeshInstance> &mis, uint32_
         const uint32_t *dIndices = ctx->dIndices;
         MeshInstance *dMis;
         float4 *posUnsorted;
-        TriShade *shadeUnsorted;
+        TriShade *triShade;
         Aabb *primBoxes;
         uint32_t *sceneBounds;
         PT_TRY(devAllocPool(ctx, &dMis, mis.size(), temp));
         PT_TRY(devAllocPool(ctx, &posUnsorted, (size_t)n * 3, temp));
-#if PT_SHADE_BY_FLAT
-        PT_TRY(devAllocPool(ctx, &shadeUnsorted, (size_t)n, ctx->accelAllocs)); // stays: the scene's shading records
-#else
-        PT_TRY(devAllocPool(ctx, &shadeUnsorted, (size_t)n, temp));
-#endif
+        PT_TRY(devAllocPool(ctx, &triShade, (size_t)n, ctx->accelAllocs)); // stays: the scene's shading records
         PT_TRY(devAllocPool(ctx, &primBoxes, (size_t)n, temp));
         PT_TRY(devAllocPool(ctx, &sceneBounds, 7, temp)); // 6 bounds + the bad-index counter of k_bake
         PT_CUDA_CHECK(ctx, cudaMemcpyAsync(dMis, mis.data(), mis.size() * sizeof(MeshInstance), cudaMemcpyHostToDevice, ctx->stream));
@@ -910,7 +887,7 @@ pt_status buildAccel(Context *ctx, const std::vector<MeshInstance> &mis, uint32_
         PT_CUDA_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
         const uint32_t T = 256;
         uint32_t G = (n + T - 1) / T;
-        k_bake<<<G, T, 0, ctx->stream>>>(dMis, (uint32_t)mis.size(), dVertices, dIndices, n, posUnsorted, shadeUnsorted,
+        k_bake<<<G, T, 0, ctx->stream>>>(dMis, (uint32_t)mis.size(), dVertices, dIndices, n, posUnsorted, triShade,
                                          primBoxes, sceneBounds, sceneBounds + 6);
         {
             uint32_t badIndices = 0;
@@ -1073,15 +1050,8 @@ pt_status buildAccel(Context *ctx, const std::vector<MeshInstance> &mis, uint32_
 
         // ---- final triangle streams, in leaf order ------------------------------------------------
         float4 *triPos;
-        TriShade *triShade;
         PT_TRY(devAllocPool(ctx, &triPos, (size_t)n * 3, ctx->accelAllocs));
-#if PT_SHADE_BY_FLAT
-        triShade = shadeUnsorted;
-        k_gather<<<G, T, 0, ctx->stream>>>(order, refTri, n, posUnsorted, shadeUnsorted, triPos, nullptr);
-#else
-        PT_TRY(devAllocPool(ctx, &triShade, (size_t)n, ctx->accelAllocs));
-        k_gather<<<G, T, 0, ctx->stream>>>(order, refTri, n, posUnsorted, shadeUnsorted, triPos, triShade);
-#endif
+        k_gather<<<G, T, 0, ctx->stream>>>(order, refTri, n, posUnsorted, triPos);
         s.triPos = triPos;
         s.triShade = triShade;
         BvhNode *nodes;
@@ -1089,11 +1059,7 @@ pt_status buildAccel(Context *ctx, const std::vector<MeshInstance> &mis, uint32_
         PT_CUDA_CHECK(ctx, cudaMemcpyAsync(nodes, wide, (size_t)wideCount * sizeof(BvhNode), cudaMemcpyDeviceToDevice, ctx->stream));
         s.nodes = nodes;
         ctx->nodeCount = wideCount;
-#if PT_SHADE_BY_FLAT
         ctx->bvhBytes = (uint64_t)wideCount * sizeof(BvhNode) + (uint64_t)n * 48 + ctx->triangleCount * sizeof(TriShade);
-#else
-        ctx->bvhBytes = (uint64_t)wideCount * sizeof(BvhNode) + (uint64_t)n * (48 + sizeof(TriShade));
-#endif
         ctx->referenceCount = n;
     }
     PT_CUDA_CHECK(ctx, cudaStreamSynchronize(ctx->stream));

@@ -5,13 +5,13 @@
 //     space once (the reference re-derives the 4x4 transform and inverts it four times per hit,
 //     PT/Shaders/sampling.glsl:5-15).  Flattened triangle id order = instance, mesh-in-model,
 //     primitive (this id breaks ties in t, so results do not depend on the BVH).
-//   * triangles are stored in BVH leaf order in two streams:
-//       TriPos   48 B  — three float4: world positions, .w lanes carry flat id / flags / material
-//                        id; read by the intersection loop (coalesced 16-B loads);
-//       TriShade 144 B — nine float4: un-normalised world normals / tangents / bitangents of
-//                        the three corners, the three UVs and the (instance, geometry,
-//                        primitive) triple; read once per shaded hit.
-//   * wide BVH nodes are 128 B (one L2 line): SoA child boxes + 4 child references.
+//   * triangles are stored in two streams:
+//       TriPos   48 B  — three float4 per BVH reference, in BVH leaf order: world positions, .w lanes carry
+//                        flat id / flags / material id; read by the intersection loop (coalesced 16-B loads);
+//       TriShade 192 B — twelve float4 per triangle, in flattened order, reached through the flat id:
+//                        world normals / tangents / bitangents of the three corners, the three UVs, the
+//                        (instance, geometry, primitive) triple and the unit normals; read once per shaded hit.
+//   * wide BVH nodes are 64 B: child boxes quantised to 8 bits per plane + 4 child references.
 //   * textures: RGBA8 (or float) mip chains, one allocation per texture, sampled in software (bilinear x
 //     trilinear, repeat) so that CPU oracle and GPU agree; sRGB decode through a 256-entry LUT.
 #pragma once
@@ -21,16 +21,11 @@ namespace pt
 {
 
 // ---------------------------------------------------------------------------------------------
-// BVH4 node.  PT_QNODES = 0: 128 bytes, fp32 child boxes (SoA).  PT_QNODES = 1: 64 bytes — the child
-// boxes quantised to 8 bits per plane on a per-node grid (origin = min corner of the node, one power-of-two
-// step per axis; Ylitie, Karras, Laine 2017 in 4-wide form), rounded OUTWARDS so that a quantised box
-// always contains the exact one: traversal stays conservative, hits are unchanged, and a node costs
-// half the cache footprint (the trace kernels live on L1 / L2 capacity for nodes, DESIGN.md §3).
+// BVH4 node, 64 bytes: the child boxes quantised to 8 bits per plane on a per-node grid (origin = min corner of
+// the node, one power-of-two step per axis; Ylitie, Karras, Laine 2017 in 4-wide form), rounded OUTWARDS so that a
+// quantised box always contains the exact one: traversal stays conservative, hits are unchanged, and a node costs
+// half the cache footprint of fp32 boxes (the trace kernels live on L1 / L2 capacity for nodes, DESIGN.md §3).
 // ---------------------------------------------------------------------------------------------
-#ifndef PT_QNODES
-#define PT_QNODES 1
-#endif
-#if PT_QNODES
 struct __align__(16) BvhNode
 {
     float ox, oy, oz; // grid origin
@@ -41,54 +36,29 @@ struct __align__(16) BvhNode
     int4 child; // >= 0: internal node index; < 0: leaf, ~child = (firstTri << 2) | (count - 1)
 };
 static_assert(sizeof(BvhNode) == 64, "quantised BvhNode must be 64 bytes");
-#else
-struct __align__(16) BvhNode
-{
-    float4 lox, loy, loz; // child i: lo = (lox[i], loy[i], loz[i])
-    float4 hix, hiy, hiz;
-    int4 child;           // >= 0: internal node index; < 0: leaf, ~child = (firstTri << 2) | (count - 1)
-    int4 pad;
-};
-static_assert(sizeof(BvhNode) == 128, "BvhNode must be one 128-byte line");
-#endif
 
 #define PT_CHILD_EMPTY 0x7fffffff
-#ifndef PT_MAX_LEAF_TRIS
 #define PT_MAX_LEAF_TRIS 4 // the leaf code has two bits for the count
-#endif
 
 PT_HD int encodeLeaf(uint32_t first, uint32_t count) { return ~(int)((first << 2) | (count - 1)); }
-
-// The shading records (TriShade, 144 B) stay in FLATTENED triangle order and are reached through the flat id a leaf entry
-// carries (triPos[3 * k].w) — one record per triangle however many references the BVH holds to it (1) — or are copied into
-// leaf order next to the positions (0: 192 B per leaf entry, the round-1 layout).
-#ifndef PT_SHADE_BY_FLAT
-#define PT_SHADE_BY_FLAT 1
-#endif
-// index of the shading record of leaf entry `tri` whose first position word is q0
-#if PT_SHADE_BY_FLAT
-#define PT_SHADE_INDEX(tri, q0w) (__float_as_uint(q0w))
-#else
-#define PT_SHADE_INDEX(tri, q0w) (tri)
-#endif
 
 #define PT_TRI_FLAG_OPAQUE 1u
 #define PT_TRI_FLAG_MIRRORED 2u // the instance transform has a negative determinant: object-space winding = world-space winding reversed
 
-#ifndef PT_SHADE_UNIT_NORMALS
-#define PT_SHADE_UNIT_NORMALS 1 // a[9..11]: what k_shade would normalise per HIT is normalised once per TRIANGLE by k_bake
-#endif
+// The shading records stay in FLATTENED triangle order and are reached through the flat id a leaf entry carries
+// (__float_as_uint(triPos[3 * k].w)): one record per triangle however many references the BVH holds to it.
 struct __align__(16) TriShade
 {
-    float4 a[PT_SHADE_UNIT_NORMALS ? 12 : 9];
+    float4 a[12];
     // a[0] = n0.xyz, n1.x   a[1] = n1.yz, n2.xy   a[2] = n2.z, t0.xyz
     // a[3] = t1.xyz, t2.x   a[4] = t2.yz, b0.xy   a[5] = b0.z, b1.xyz
     // a[6] = b2.xyz, uv0.x  a[7] = uv0.y, uv1.xy, uv2.x   a[8] = uv2.y, instance, geometry, primitive (bits)
     // a[9] = normalize(n0).xyz, normalize(n1).x   a[10] = normalize(n1).yz, normalize(n2).xy
-    // a[11] = normalize(n2).z, normalize(cross(p1 - p0, p2 - p0)).xyz — the same device functions on the same
-    //         values k_shade would apply (closestHit.rchit:60-66, 76-78), so the bits are those of the per-hit evaluation
+    // a[11] = normalize(n2).z, normalize(cross(p1 - p0, p2 - p0)).xyz — what k_shade would normalise per HIT, normalised
+    //         once per TRIANGLE by k_bake with the same device functions on the same values (closestHit.rchit:60-66,
+    //         76-78), so the bits are those of the per-hit evaluation
 };
-static_assert(sizeof(TriShade) == (PT_SHADE_UNIT_NORMALS ? 192 : 144), "TriShade must be 144 / 192 bytes");
+static_assert(sizeof(TriShade) == 192, "TriShade must be 192 bytes");
 
 // ---------------------------------------------------------------------------------------------
 // materials: the reference's 96-byte structs, verbatim (PT/Shaders/ShaderTypes.incl:61-118)
@@ -126,8 +96,8 @@ struct LightBlock
 struct DeviceScene
 {
     const BvhNode *nodes;
-    const float4 *triPos;     // 3 per triangle, leaf order
-    const TriShade *triShade; // leaf order
+    const float4 *triPos;     // 3 per BVH reference, leaf order
+    const TriShade *triShade; // flattened order, indexed by the flat id
     const MaterialRaw *materials[3]; // by material type
     const DevTexture *textures;
     const float *lut; // [0..255] unorm, [256..511] sRGB -> linear
@@ -293,18 +263,10 @@ PT_DEV float4 sampleTrilinear(const DeviceScene &s, const DevTexture &t, uint32_
     return lerp4(a, b, frac);
 }
 
-// Inlined by default.  An out-of-line copy (PT_TEX_INLINE=0) shrinks k_shade from 300 KB to 100 KB
-// of SASS and removes the instruction-cache stalls, but the calls cost more than that saves
-// (measured on the B200: shade 46.4 ms out of line vs 41.6 ms inlined, 32 spp of the chess scene).
-#ifndef PT_TEX_INLINE
-#define PT_TEX_INLINE 1
-#endif
-#if PT_TEX_INLINE
-static __device__ __forceinline__ float4 textureGrad(
-#else
-static __device__ __noinline__ float4 textureGrad(
-#endif
-const DeviceScene &s, uint32_t slot, float u, float v, float4 deriv)
+// Inlined.  An out-of-line copy shrinks k_shade from 300 KB to 100 KB of SASS and removes the instruction-cache
+// stalls, but the calls cost more than that saves (measured on the B200: shade 46.4 ms out of line vs 41.6 ms
+// inlined, 32 spp of the chess scene).
+static __device__ __forceinline__ float4 textureGrad(const DeviceScene &s, uint32_t slot, float u, float v, float4 deriv)
 {
     const DevTexture &t = s.textures[slot];
     const GradFootprint g = gradFootprint(t, deriv, s.maxAnisotropy);

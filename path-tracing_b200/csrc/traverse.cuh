@@ -12,55 +12,16 @@ namespace pt
 {
 
 #define PT_STACK_SIZE 96 // >= 3 entries per level of the wide BVH + 1 (depths seen: 14-21); an overflow fails the call
-// PT_SMEM_STACK > 0 puts the first PT_SMEM_STACK entries of a wavefront lane's traversal stack in SHARED
-// memory, laid out [entry][thread] (64-bit words: conflict-free whatever the lanes' depths), deeper
-// entries in the local-memory array.  Measured on the B200 (chess / street / atrium, 8 blocks per SM):
-// 8 entries = no change, 16 entries = 1-3 % SLOWER, 24 entries = 8 % slower in k_extend — the hot top of
-// a local-memory stack already sits in L1, and the shared-memory carve-out takes that L1 away from
-// the BVH nodes.  Off by default.
-#ifndef PT_SMEM_STACK
-#define PT_SMEM_STACK 0
-#endif
-#define PT_TRACE_THREADS 128
-
-// tuning switches (A/B-tested on the B200, see DESIGN.md)
-#ifndef PT_PREFETCH_LEAF
-#define PT_PREFETCH_LEAF 1 // prefetch a leaf's first triangle into L1 when the leaf is postponed
-#endif
-#ifndef PT_PREFETCH_PUSH
-#define PT_PREFETCH_PUSH 0 // prefetch the nearest pushed child node into L1
-#endif
+// The stack lives in local memory.  Its first entries in SHARED memory instead were measured on the B200 (chess /
+// street / atrium, 8 blocks per SM): 8 entries = no change, 16 entries = 1-3 % SLOWER, 24 entries = 8 % slower in
+// k_extend — the hot top of a local-memory stack already sits in L1, and the shared-memory carve-out takes that L1
+// away from the BVH nodes.
 
 // the node phase of a warp goes on while more than this many lanes still look for their first leaf
 // (0 = until every lane has one; lanes cut short idle through the triangle phase)
 #ifndef PT_NODE_LOOP_LANES
 #define PT_NODE_LOOP_LANES 4 // measured on chess: 0 -> 4 = k_extend -1.5 %, k_shadow -6 %; 8 = no further gain
 #endif
-// leafStep also tests a second leaf the lane found while the first was postponed (1) or leaves it
-// to the next round of the warp (0)
-#ifndef PT_LEAF_SECOND
-#define PT_LEAF_SECOND 0 // measured: 1 -> 0 = +2.3 % chess, +2.5 % street, +2.4 % dragon
-#endif
-#ifndef PT_LEAF_SECOND_ALPHA
-#define PT_LEAF_SECOND_ALPHA 1
-#endif
-// the leaf phase tests ONE triangle per lane and trip of the warp instead of the whole leaf
-#ifndef PT_POP_TWICE
-#define PT_POP_TWICE 0
-#endif
-#ifndef PT_LEAF_ONE
-#define PT_LEAF_ONE 0
-#endif
-
-#ifndef PT_SHADOW_NOSORT
-#define PT_SHADOW_NOSORT 0 // occlusion rays: skip the front-to-back sort of a node's children (measured: k_shadow -3 % on
-                           // chess, -1 % dragon, +8 % street: near-first order finds occluders sooner; off)
-#endif
-
-#ifndef PT_BOX_FMA
-#define PT_BOX_FMA 0 // slab distances as one FMA per plane (precomputed org / dir, error folded into the planes)
-#endif
-
 // Entries a traversal could not push because its stack (PT_STACK_SIZE entries) was full.  A dropped entry is a lost
 // sub-tree, i.e. possibly a missed hit: the host reads this counter after every call and FAILS the call when it is
 // non-zero (checkStackOverflow).  The build also reports the depth of the wide BVH (pt_stats::bvh_max_depth).
@@ -99,15 +60,9 @@ struct RaySetup
     float idx, idy, idz; // 1 / dir
     float Sx, Sy, Sz;
     int kx, ky, kz;
-    // float4 index (0 = lo planes, 3 = hi planes) of the slab planes the ray enters through, per axis:
-    // chosen by the SIGN BIT of the direction (so that -0 pairs with idx = -inf)
+    // non-zero when the ray enters the slab of that axis through its hi plane: chosen by the SIGN BIT of the
+    // direction (so that -0 pairs with idx = -inf)
     int nearX, nearY, nearZ;
-#if PT_BOX_FMA
-    // rn(org * idir) pushed outwards by its own rounding error (and one more ulp for the FMA's), per
-    // axis, for the entry (N) and exit (F) planes: fma(plane, idir, -oidN) <= true entry distance and
-    // fma(plane, idir, -oidF) >= true exit distance, so the box test stays conservative
-    float oidNx, oidNy, oidNz, oidFx, oidFy, oidFz;
-#endif
 };
 
 // v[k] as two selects (FSEL) on predicates that depend on the ray only.  Written as the nested
@@ -143,16 +98,6 @@ PT_DEV RaySetup setupRay(vec3 o, vec3 d)
     r.nearX = __float_as_int(d.x) < 0 ? 3 : 0;
     r.nearY = __float_as_int(d.y) < 0 ? 3 : 0;
     r.nearZ = __float_as_int(d.z) < 0 ? 3 : 0;
-#if PT_BOX_FMA
-    {
-        // |error| of fma(p, id, -rn(o * id)) against (p - o) * id is at most ulp(o * id) / 2 + ulp(result) / 2;
-        // the second term is covered by the relative factor of the test, the first by e below
-        const float ox = o.x * r.idx, oy = o.y * r.idy, oz = o.z * r.idz;
-        const float ex = fabsf(ox) * 1.8e-7f, ey = fabsf(oy) * 1.8e-7f, ez = fabsf(oz) * 1.8e-7f;
-        r.oidNx = ox + ex, r.oidNy = oy + ey, r.oidNz = oz + ez;
-        r.oidFx = ox - ex, r.oidFy = oy - ey, r.oidFz = oz - ez;
-    }
-#endif
     return r;
 }
 
@@ -276,10 +221,8 @@ PT_DEV vec3 anyHitRgb(const DeviceScene &s, const AnyHitSample &a)
 }
 
 // One BVH4 node: tests the four child boxes, returns entry distances (INF if missed / empty).
-// The entry / exit planes of every slab are picked by the ray's direction signs when the node is
-// LOADED (per-ray float4 offsets), so a box costs 6 subtractions, 6 multiplications and two
-// four-input max / min (FMNMX + FMNMX3) instead of twelve more two-input min / max.
-#if PT_QNODES
+// The entry / exit plane words of every slab are picked once per node by the ray's direction signs,
+// so a box costs six byte conversions, six FMAs and two four-input max / min.
 PT_DEV void intersectNode(const BvhNode *__restrict__ node, const RaySetup &r, float tmin, float tmax, float d[4],
                           int c[4])
 {
@@ -309,39 +252,6 @@ PT_DEV void intersectNode(const BvhNode *__restrict__ node, const RaySetup &r, f
         d[i] = (c[i] != PT_CHILD_EMPTY && t0 <= t1 * 1.0000008f) ? t0 : INFINITY;
     }
 }
-#else
-PT_DEV void intersectNode(const BvhNode *__restrict__ node, const RaySetup &r, float tmin, float tmax, float d[4],
-                          int c[4])
-{
-    const float4 *q = reinterpret_cast<const float4 *>(node);
-    const float4 nx4 = __ldg(q + r.nearX), ny4 = __ldg(q + 1 + r.nearY), nz4 = __ldg(q + 2 + r.nearZ);
-    const float4 fx4 = __ldg(q + 3 - r.nearX), fy4 = __ldg(q + 4 - r.nearY), fz4 = __ldg(q + 5 - r.nearZ);
-    const int4 ch = __ldg(&node->child);
-    const float nx[4] = { nx4.x, nx4.y, nx4.z, nx4.w }, ny[4] = { ny4.x, ny4.y, ny4.z, ny4.w };
-    const float nz[4] = { nz4.x, nz4.y, nz4.z, nz4.w }, fx[4] = { fx4.x, fx4.y, fx4.z, fx4.w };
-    const float fy[4] = { fy4.x, fy4.y, fy4.z, fy4.w }, fz[4] = { fz4.x, fz4.y, fz4.z, fz4.w };
-    c[0] = ch.x, c[1] = ch.y, c[2] = ch.z, c[3] = ch.w;
-#pragma unroll
-    for (int i = 0; i < 4; i++)
-    {
-#if PT_BOX_FMA
-        const float ax = fmaf(nx[i], r.idx, -r.oidNx), bx = fmaf(fx[i], r.idx, -r.oidFx);
-        const float ay = fmaf(ny[i], r.idy, -r.oidNy), by = fmaf(fy[i], r.idy, -r.oidFy);
-        const float az = fmaf(nz[i], r.idz, -r.oidNz), bz = fmaf(fz[i], r.idz, -r.oidFz);
-#else
-        const float ax = (nx[i] - r.org.x) * r.idx, bx = (fx[i] - r.org.x) * r.idx;
-        const float ay = (ny[i] - r.org.y) * r.idy, by = (fy[i] - r.org.y) * r.idy;
-        const float az = (nz[i] - r.org.z) * r.idz, bz = (fz[i] - r.org.z) * r.idz;
-#endif
-        // fminf/fmaxf drop NaNs (0 * inf when the origin lies in a slab plane of an axis-parallel ray)
-        const float t0 = fmaxf(fmaxf(ax, ay), fmaxf(az, tmin));
-        const float t1 = fminf(fminf(bx, by), fminf(bz, tmax));
-        // conservative (Ize 2013): never cull a box the triangle test could still hit
-        d[i] = (c[i] != PT_CHILD_EMPTY && t0 <= t1 * 1.0000004f) ? t0 : INFINITY;
-    }
-}
-
-#endif
 
 // distances by min / max, references by one compare and two selects (an if-swap compiled to eight moves);
 // the distances are never NaN, so min / max order them as the compare does
@@ -367,11 +277,10 @@ PT_DEV void intersectNode(const BvhNode *__restrict__ node, const RaySetup &r, f
 //                    candidates at all.  Vulkan decides the facing in OBJECT space: front = the vertices appear
 //                    clockwise from the ray origin, i.e. dot((v1 - v0) x (v2 - v0), d) < 0 there; a mirroring
 //                    instance transform reverses the world-space winding (PT_TRI_FLAG_MIRRORED).
-template <bool CLOSEST, bool ALPHA, bool STATS, int SMEM = 0, bool CULL = false> struct Traverser
+template <bool CLOSEST, bool ALPHA, bool STATS, bool CULL = false> struct Traverser
 {
     vec3 cullDir; // world ray direction (CULL only)
     static constexpr bool kClosest = CLOSEST, kAlpha = ALPHA, kStats = STATS;
-    unsigned long long *sstack; // this thread's column of the block's shared stack (SMEM > 0)
     RaySetup r;
     float tmin, tmax, best;
     uint32_t bestFlat;
@@ -436,19 +345,15 @@ template <bool CLOSEST, bool ALPHA, bool STATS, int SMEM = 0, bool CULL = false>
     PT_DEV unsigned long long take()
     {
         --sp;
-        if (SMEM > 0 && sp < SMEM)
-            return sstack[sp * PT_TRACE_THREADS];
-        return stack[sp - SMEM];
+        return stack[sp];
     }
 
     PT_DEV void push(int node, float dist)
     {
         const unsigned long long e = ((unsigned long long)__float_as_uint(dist) << 32) | (uint32_t)node;
-        if (SMEM > 0 && sp < SMEM)
-            sstack[sp++ * PT_TRACE_THREADS] = e;
-        else if (sp < PT_STACK_SIZE + SMEM)
+        if (sp < PT_STACK_SIZE)
         {
-            stack[sp - SMEM] = e;
+            stack[sp] = e;
             sp++;
         }
         else
@@ -466,24 +371,9 @@ template <bool CLOSEST, bool ALPHA, bool STATS, int SMEM = 0, bool CULL = false>
             st.boxTests += 4;
             visits++;
         }
-#if PT_SHADOW_NOSORT
-        if (!CLOSEST)
-        {
-            // any hit will do: no front-to-back order, take the hit children as they are stored
-            int next = PT_CHILD_POP;
-#pragma unroll
-            for (int i = 3; i >= 0; i--)
-                if (d[i] != INFINITY)
-                {
-                    if (next != PT_CHILD_POP)
-                        push(next, 0.0f);
-                    next = c[i];
-                }
-            cur = next;
-            return;
-        }
-#endif
-        // sorting network, ascending by distance (missed children carry INF)
+        // sorting network, ascending by distance (missed children carry INF).  Occlusion rays are sorted too:
+        // taking the hit children in stored order was measured k_shadow -3 % on chess, -1 % dragon, +8 % street —
+        // near-first order finds occluders sooner.
         PT_CSWAP(0, 1)
         PT_CSWAP(2, 3)
         PT_CSWAP(0, 2)
@@ -499,7 +389,7 @@ template <bool CLOSEST, bool ALPHA, bool STATS, int SMEM = 0, bool CULL = false>
         // bound check (three conditional pushes were three branches with a bound check each)
         const bool h1 = d[1] != INFINITY, h2 = d[2] != INFINITY, h3 = d[3] != INFINITY;
         const int m = (int)h1 + (int)h2 + (int)h3;
-        if (SMEM == 0 && sp + m <= PT_STACK_SIZE)
+        if (sp + m <= PT_STACK_SIZE)
         {
             unsigned long long *top = stack + sp + m; // one past the new top
             if (h1)
@@ -509,10 +399,6 @@ template <bool CLOSEST, bool ALPHA, bool STATS, int SMEM = 0, bool CULL = false>
             if (h3)
                 top[-3] = ((unsigned long long)__float_as_uint(d[3]) << 32) | (uint32_t)c[3];
             sp += m;
-#if PT_PREFETCH_PUSH
-            if (h1 && c[1] >= 0)
-                prefetchL1(s.nodes + c[1]);
-#endif
             return;
         }
         // push the rest, farthest first
@@ -521,13 +407,7 @@ template <bool CLOSEST, bool ALPHA, bool STATS, int SMEM = 0, bool CULL = false>
         if (d[2] != INFINITY)
             push(c[2], d[2]);
         if (d[1] != INFINITY)
-        {
             push(c[1], d[1]);
-#if PT_PREFETCH_PUSH
-            if (c[1] >= 0)
-                prefetchL1(s.nodes + c[1]);
-#endif
-        }
     }
 
     // result of another lane that traversed part of this ray's tree (straggler splitting)
@@ -560,29 +440,20 @@ template <bool CLOSEST, bool ALPHA, bool STATS, int SMEM = 0, bool CULL = false>
         if (cur < 0 && leaf == PT_CHILD_EMPTY)
         {
             leaf = cur;
-#if PT_PREFETCH_LEAF
-            prefetchL1(sPrefetchTri + 3 * (size_t)(((uint32_t)~cur) >> 2));
-#endif
+            prefetchL1(sPrefetchTri + 3 * (size_t)(((uint32_t)~cur) >> 2)); // the leaf's first triangle, into L1
             cur = PT_CHILD_POP;
         }
     }
 
-    // tests the triangles of the postponed leaf (and of a second leaf waiting in cur)
+    // tests the triangles of the postponed leaf (and, if ALPHA, of a second leaf waiting in cur)
     PT_DEV void leafStep(const DeviceScene &s)
     {
         while (leaf != PT_CHILD_EMPTY)
         {
             const uint32_t code = (uint32_t)~leaf;
             const uint32_t first = code >> 2, count = (code & 3u) + 1;
-#if PT_LEAF_ONE
-            // one triangle per trip of the warp: the rest of the leaf waits for the next leaf phase
-            leaf = count > 1 ? encodeLeaf(first + 1, count - 1) : PT_CHILD_EMPTY;
-            const uint32_t trips = 1;
-#else
             leaf = PT_CHILD_EMPTY;
-            const uint32_t trips = count;
-#endif
-            for (uint32_t i = 0; i < trips; i++)
+            for (uint32_t i = 0; i < count; i++)
             {
                 const uint32_t tri = first + i;
                 const float4 q0 = __ldg(s.triPos + 3 * (size_t)tri);
@@ -617,7 +488,7 @@ template <bool CLOSEST, bool ALPHA, bool STATS, int SMEM = 0, bool CULL = false>
                     if (STATS)
                         st.alphaTests++;
                     AnyHitSample ah;
-                    const float alpha = anyHitAlpha(s, PT_SHADE_INDEX(tri, q0.w), __float_as_uint(q2.w), b1, b2, ah);
+                    const float alpha = anyHitAlpha(s, __float_as_uint(q0.w), __float_as_uint(q2.w), b1, b2, ah);
                     if (CLOSEST)
                     {
                         if (alpha < 0.5f)
@@ -647,17 +518,14 @@ template <bool CLOSEST, bool ALPHA, bool STATS, int SMEM = 0, bool CULL = false>
                 best = t;
                 bestFlat = flat;
             }
-#if PT_LEAF_ONE
-            return;
-#else
             // a second leaf found while this one was postponed (scenes with alpha-tested geometry visit many
-            // leaves per ray — 20 in the atrium — and are 2.5 % faster chaining them; the others are not)
-            if ((PT_LEAF_SECOND || (ALPHA && PT_LEAF_SECOND_ALPHA)) && cur < 0)
+            // leaves per ray — 20 in the atrium — and are 2.5 % faster chaining them; the others are 2.3-2.5 %
+            // faster leaving it to the next round of the warp)
+            if (ALPHA && cur < 0)
             {
                 leaf = cur;
                 cur = PT_CHILD_POP;
             }
-#endif
         }
     }
 };
@@ -668,7 +536,7 @@ PT_DEV void traverse(const DeviceScene &s, vec3 org, vec3 dir, float tmin, float
                      TraversalStats &st)
 {
     unsigned long long stack[PT_STACK_SIZE];
-    Traverser<CLOSEST, ALPHA, STATS, 0, CULL> tr;
+    Traverser<CLOSEST, ALPHA, STATS, CULL> tr;
     tr.stack = stack;
     tr.cullDir = dir;
     tr.st = st;
@@ -721,15 +589,6 @@ PT_DEV void traverse(const DeviceScene &s, vec3 org, vec3 dir, float tmin, float
 //     that sub-tree, and its result is merged into the owner's with the same (t, triangle id)
 //     order the serial traversal uses — the answer is identical, the tail up to 32x shorter.
 // ---------------------------------------------------------------------------------------------
-// the prefetch stages of tracePersistent as calls (0) or inlined at their call sites (1)
-#ifndef PT_INLINE_PREFETCH
-#define PT_INLINE_PREFETCH 1
-#endif
-#if PT_INLINE_PREFETCH
-#define PT_PREFETCH_INLINE __attribute__((always_inline))
-#else
-#define PT_PREFETCH_INLINE
-#endif
 #ifndef PT_FETCH_CHUNK
 #define PT_FETCH_CHUNK 32u
 #endif
@@ -769,8 +628,9 @@ PT_DEV void tracePersistent(const DeviceScene &s, uint32_t n, uint32_t *workCoun
 
     uint32_t nxCount = 0; // warp-uniform: lanes [0, nxCount) hold the slot indices of the batch after the buffer
     uint32_t nxSlot = 0;
+    // (both stages are force-inlined: as calls they forced a local-memory copy of the kernel parameter block, DESIGN.md §3)
     // stage 1: request the slot indices of the next batch of the warp's chunk
-    auto prefetchSlots = [&]() PT_PREFETCH_INLINE {
+    auto prefetchSlots = [&]() __attribute__((always_inline)) {
         nxCount = 0;
         if (exhausted)
             return;
@@ -794,7 +654,7 @@ PT_DEV void tracePersistent(const DeviceScene &s, uint32_t n, uint32_t *workCoun
         wBase += nxCount;
     };
     // stage 2: request the rays of the batch whose slot indices arrived meanwhile, then stage 1 again
-    auto prefetch = [&]() PT_PREFETCH_INLINE {
+    auto prefetch = [&]() __attribute__((always_inline)) {
         pfPos = 0;
         pfCount = nxCount;
         if (lane < nxCount)
@@ -861,9 +721,6 @@ PT_DEV void tracePersistent(const DeviceScene &s, uint32_t n, uint32_t *workCoun
                     tr.nodeStep(s);
                 tr.postponeLeaf(s.triPos);
                 tr.popStep();
-#if PT_POP_TWICE
-                tr.popStep(); // an entry culled by the current best costs no extra trip
-#endif
             } while (__popc(__ballot_sync(FULL, (tr.atInternal() || tr.needsPop()) && !tr.hasLeaf())) > PT_NODE_LOOP_LANES);
             tr.leafStep(s);
             if (!drain)
@@ -944,11 +801,6 @@ PT_DEV void tracePersistent(const DeviceScene &s, uint32_t n, uint32_t *workCoun
                 r.org.z = __shfl_sync(FULL, tr.r.org.z, donor);
                 r.idx = __shfl_sync(FULL, tr.r.idx, donor), r.idy = __shfl_sync(FULL, tr.r.idy, donor);
                 r.idz = __shfl_sync(FULL, tr.r.idz, donor);
-#if PT_BOX_FMA
-                r.oidNx = __shfl_sync(FULL, tr.r.oidNx, donor), r.oidNy = __shfl_sync(FULL, tr.r.oidNy, donor);
-                r.oidNz = __shfl_sync(FULL, tr.r.oidNz, donor), r.oidFx = __shfl_sync(FULL, tr.r.oidFx, donor);
-                r.oidFy = __shfl_sync(FULL, tr.r.oidFy, donor), r.oidFz = __shfl_sync(FULL, tr.r.oidFz, donor);
-#endif
                 r.Sx = __shfl_sync(FULL, tr.r.Sx, donor), r.Sy = __shfl_sync(FULL, tr.r.Sy, donor);
                 r.Sz = __shfl_sync(FULL, tr.r.Sz, donor);
                 r.kx = __shfl_sync(FULL, tr.r.kx, donor), r.ky = __shfl_sync(FULL, tr.r.ky, donor);

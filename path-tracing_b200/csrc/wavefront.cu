@@ -55,22 +55,6 @@ namespace
 #define PT_SHADE_GRID_PER_SM 4 // k_shade blocks per SM = the resident ones (grid-stride loop over the hits).  Measured 4 / 8 / 16 / 64: alone the kernel
                                // likes MORE blocks (chess 55.2 / 54.3 / 53.4 / 50.2 ms), the two overlapping pools fewer (2368 / 2360 / 2352 / 2341 Mrays/s)
 #endif
-// k_shade register diet: the geometry the code after the BSDF sample needs is reduced to its results before the material fetch
-#ifndef PT_SHADE_DIET
-#define PT_SHADE_DIET 1
-#endif
-#ifndef PT_SHADE_LATE_READS
-#define PT_SHADE_LATE_READS 0 // measured: re-reading differentials / throughput / radiance where they are used exposes their latency, k_shade +12 % (chess)
-#endif
-// the ray-load lambda of k_extend (which also regenerates ended paths) as a call (0) or inlined at its two call sites (1)
-#ifndef PT_INLINE_LOADRAY
-#define PT_INLINE_LOADRAY 1
-#endif
-#if PT_INLINE_LOADRAY
-#define PT_LOADRAY_INLINE __attribute__((always_inline))
-#else
-#define PT_LOADRAY_INLINE
-#endif
 
 constexpr uint32_t kMaxRestarts = 1024; // the reference's restart loop is unbounded; see oracle
 // path state word (PathRecord::thr.w): bounce [0, 8), NaN/Inf restarts of the frame [8, 19), sample of the frame [19, 32)
@@ -280,15 +264,14 @@ template <bool ALPHA, bool STATS> __global__ void __launch_bounds__(128, PT_TRAC
     uint32_t hits = 0, rays = 0, samples = 0, restarts = 0;
     uint32_t *regenOut = cur ? rc.ps.regenQ[0] : rc.ps.regenQ[1];
     unsigned long long stack[PT_STACK_SIZE];
-    __shared__ unsigned long long sharedStack[(PT_SMEM_STACK > 0 ? PT_SMEM_STACK : 1) * PT_TRACE_THREADS];
-    Traverser<true, ALPHA, STATS, PT_SMEM_STACK> tr;
+    Traverser<true, ALPHA, STATS> tr;
     tr.stack = stack;
-    tr.sstack = sharedStack + threadIdx.x;
     tr.st = TraversalStats { 0, 0, 0 };
     tracePersistent(
         rc.scene, n, &rc.qc->extendWork, tr, 0.00001f,
         [&](uint32_t i) { return activeSlot(rc, cur, i, nCont); },
-        [&](uint32_t entry) PT_LOADRAY_INLINE {
+        // force-inlined: as a call it forced a local-memory copy of the kernel parameter block (DESIGN.md §3)
+        [&](uint32_t entry) __attribute__((always_inline)) {
             if (entry & kRegen)
                 return regeneratePath(rc, entry, samples, restarts);
             RayPacket p;
@@ -299,7 +282,7 @@ template <bool ALPHA, bool STATS> __global__ void __launch_bounds__(128, PT_TRAC
             p.tmax = 10000.0f;
             return p;
         },
-        [&](Traverser<true, ALPHA, STATS, PT_SMEM_STACK> &t, uint32_t slot) {
+        [&](Traverser<true, ALPHA, STATS> &t, uint32_t slot) {
             rays++;
             if (t.hit.tri == 0xffffffffu)
             {
@@ -417,12 +400,12 @@ template <bool ALPHA, bool STATS> __global__ void __launch_bounds__(128, PT_SHAD
         const uint32_t slot = hitQueue[i];
         const float4 hitv = rc.ps.rec[slot].hit;
         const float4 rayO = rc.ps.rec[slot].rayO, rayD = rc.ps.rec[slot].rayD;
-#if !PT_SHADE_LATE_READS
+        // read with the rest of the record: reading throughput, radiance and the differentials again where they are
+        // used exposed the loads' latency at the end of every hit (measured: k_shade +12 %, chess)
         float4 thr4 = rc.ps.rec[slot].thr;
         float4 rad4 = rc.ps.rec[slot].rad;
         vec3 throughput = V3(thr4), radiance = V3(rad4);
         uint32_t state = __float_as_uint(thr4.w);
-#endif
         const vec3 rayDir = V3(rayD);
         const uint32_t tri = __float_as_uint(hitv.x);
 
@@ -434,7 +417,7 @@ template <bool ALPHA, bool STATS> __global__ void __launch_bounds__(128, PT_SHAD
         // ---- closestHit.rchit:54-83 with baked world-space data ---------------------------------
         const float4 q0 = __ldg(s.triPos + 3 * (size_t)tri), q1 = __ldg(s.triPos + 3 * (size_t)tri + 1);
         const float4 q2 = __ldg(s.triPos + 3 * (size_t)tri + 2);
-        const TriShade &ts = s.triShade[PT_SHADE_INDEX(tri, q0.w)];
+        const TriShade &ts = s.triShade[__float_as_uint(q0.w)];
         const float4 a0 = __ldg(&ts.a[0]), a1 = __ldg(&ts.a[1]), a2 = __ldg(&ts.a[2]), a3 = __ldg(&ts.a[3]);
         const float4 a4 = __ldg(&ts.a[4]), a5 = __ldg(&ts.a[5]), a6 = __ldg(&ts.a[6]), a7 = __ldg(&ts.a[7]);
         const float4 a8 = __ldg(&ts.a[8]);
@@ -451,15 +434,10 @@ template <bool ALPHA, bool STATS> __global__ void __launch_bounds__(128, PT_SHAD
         vec3 tangent = normalize(t0r * bary.x + t1r * bary.y + t2r * bary.z);
         vec3 bitangent = normalize(b0r * bary.x + b1r * bary.y + b2r * bary.z);
         const vec3 edge1 = p1 - p0, edge2 = p2 - p0;
-#if PT_SHADE_UNIT_NORMALS
         // normalised once per triangle by k_bake (same functions, same operands)
         const float4 a9 = __ldg(&ts.a[9]), a10 = __ldg(&ts.a[10]), a11 = __ldg(&ts.a[11]);
         const vec3 n0 = V3(a9.x, a9.y, a9.z), n1 = V3(a9.w, a10.x, a10.y), n2 = V3(a10.z, a10.w, a11.x);
         vec3 geometricNormal = V3(a11.y, a11.z, a11.w);
-#else
-        const vec3 n0 = normalize(n0r), n1 = normalize(n1r), n2 = normalize(n2r);
-        vec3 geometricNormal = normalize(cross(edge1, edge2));
-#endif
         const bool inside = dot(geometricNormal, rayDir) > 0.0f;
         if (inside)
         {
@@ -481,18 +459,15 @@ template <bool ALPHA, bool STATS> __global__ void __launch_bounds__(128, PT_SHAD
         vec3 dpdx, dpdy;
         computeDpDxy(position, rd.rxOrigin, rd.rxDirection, rd.ryOrigin, rd.ryDirection, normal, dpdx, dpdy);
         const float4 derivatives = computeDerivatives(dpdx, dpdy, dpdu, dpdv);
-#if PT_SHADE_DIET
         // Register diet: what the code AFTER the BSDF sample needs of the geometry is reduced to its results now — the
         // ray origin of either outcome (reflected / refracted: same operations as the one call the shader makes, for
         // both values of its flag) and the normal's screen-space derivatives — so that the triangle's corners, vertex
-        // normals, barycentrics and uv derivatives are dead while the material and the BSDF are evaluated; the ray
-        // differentials are re-read from the path record where they are propagated.
+        // normals, barycentrics and uv derivatives are dead while the material and the BSDF are evaluated.
         const vec3 originReflected = offsetRayOriginShadowTerminator(position, p0, p1, p2, n0, n1, n2, bary, false);
         const vec3 originRefracted = offsetRayOriginShadowTerminator(position, p0, p1, p2, n0, n1, n2, bary, true);
         const vec3 originThrough = offsetRayOriginSelfIntersection(position, -geometricNormal);
         const vec3 dndx = dndu * derivatives.x + dndv * derivatives.y;
         const vec3 dndy = dndu * derivatives.z + dndv * derivatives.w;
-#endif
 
         // ---- material, closestHit.rchit:101-117 -------------------------------------------------
         MaterialSample material = sampleMaterial(s, materialId, texCoords.x, texCoords.y, derivatives, inside,
@@ -523,11 +498,7 @@ template <bool ALPHA, bool STATS> __global__ void __launch_bounds__(128, PT_SHAD
             bsdf.Color.z *= powf(material.AttenuationColor.z, e);
         }
         const bool isRefracted = bsdf.Direction.z < 0.0f;
-#if PT_SHADE_DIET
         const vec3 rayOrigin = isRefracted ? originRefracted : originReflected;
-#else
-        const vec3 rayOrigin = offsetRayOriginShadowTerminator(position, p0, p1, p2, n0, n1, n2, bary, isRefracted);
-#endif
 
         float lightPdf, lightSmplPdf;
         const float l0 = rnd(rng);
@@ -538,38 +509,12 @@ template <bool ALPHA, bool STATS> __global__ void __launch_bounds__(128, PT_SHAD
         const vec3 lightBsdf = evaluateBSDF(material, V, L, lightSmplPdf);
 
         const vec3 newDir = normalize(mul(TBN, bsdf.Direction));
-#if PT_SHADE_DIET
         const vec3 newPos = isRefracted ? originThrough : rayOrigin;
-#else
-        const vec3 newPos = isRefracted ? offsetRayOriginSelfIntersection(position, -geometricNormal) : rayOrigin;
-#endif
         const vec3 directLight = light.Color * light.Attenuation * lightBsdf;
 
-#if PT_SHADE_LATE_READS
-        {
-            // __ldcg is an asm volatile load: a second read of the record (an L2 hit), not the registers of the first
-            // one kept alive across the BSDF
-            const float4 *dv = &rc.ps.rec[slot].diff0;
-            const float4 e0 = __ldcg(dv), e1 = __ldcg(dv + 1), e2 = __ldcg(dv + 2);
-            rd.rxOrigin = V3(e0.x, e0.y, e0.z);
-            rd.rxDirection = V3(e0.w, e1.x, e1.y);
-            rd.ryOrigin = V3(e1.z, e1.w, e2.x);
-            rd.ryDirection = V3(e2.y, e2.z, e2.w);
-        }
-#endif
-#if PT_SHADE_DIET
         propagateDifferentials(normal, rayOrigin, -rayDir, newDir, dndx, dndy, material.Eta, isRefracted, rd);
-#else
-        propagateDifferentials(derivatives, normal, rayOrigin, -rayDir, newDir, dndu, dndv, material.Eta, isRefracted, rd);
-#endif
 
         // ---- raygen.rgen:71-96 ----------------------------------------------------------------
-#if PT_SHADE_LATE_READS
-        // throughput, radiance and the bounce state are first needed here: read now (same line as rayO / rayD)
-        const float4 thr4 = __ldcg(&rc.ps.rec[slot].thr), rad4 = __ldcg(&rc.ps.rec[slot].rad);
-        vec3 throughput = V3(thr4), radiance = V3(rad4);
-        uint32_t state = __float_as_uint(thr4.w);
-#endif
         radiance += throughput * material.EmissiveColor;
         bool done = false;
         if (bsdf.Pdf == -1.0f)
@@ -642,10 +587,8 @@ template <bool ALPHA, bool STATS> __global__ void __launch_bounds__(128, PT_TRAC
         rc.qc->hit = 0;
     }
     unsigned long long stack[PT_STACK_SIZE];
-    __shared__ unsigned long long sharedStack[(PT_SMEM_STACK > 0 ? PT_SMEM_STACK : 1) * PT_TRACE_THREADS];
-    Traverser<false, ALPHA, STATS, PT_SMEM_STACK> tr;
+    Traverser<false, ALPHA, STATS> tr;
     tr.stack = stack;
-    tr.sstack = sharedStack + threadIdx.x;
     tr.st = TraversalStats { 0, 0, 0 };
     tracePersistent(
         rc.scene, n, &rc.qc->shadowWork, tr, 0.00001f,
@@ -659,7 +602,7 @@ template <bool ALPHA, bool STATS> __global__ void __launch_bounds__(128, PT_TRAC
             p.tmax = o.w;
             return p;
         },
-        [&](Traverser<false, ALPHA, STATS, PT_SMEM_STACK> &t, uint32_t slot) {
+        [&](Traverser<false, ALPHA, STATS> &t, uint32_t slot) {
             if (t.hit.tri == 0xffffffffu)
             {
                 const float4 c = rc.ps.rec[slot].shC;
@@ -716,7 +659,7 @@ __device__ __forceinline__ pt_hit toPtHit(const DeviceScene &s, const Hit &h)
         r.t = r.u = r.v = 0.0f;
         return r;
     }
-    const float4 a8 = __ldg(&s.triShade[PT_SHADE_INDEX(h.tri, __ldg(s.triPos + 3 * (size_t)h.tri).w)].a[8]);
+    const float4 a8 = __ldg(&s.triShade[__float_as_uint(__ldg(s.triPos + 3 * (size_t)h.tri).w)].a[8]);
     r.instance = __float_as_uint(a8.y);
     r.geometry = __float_as_uint(a8.z);
     r.primitive = __float_as_uint(a8.w);
@@ -820,7 +763,7 @@ __global__ void k_debug(DeviceScene s, CameraMatrices cam, uint32_t width, uint3
     const vec3 bary = V3(1.0f - hit.b1 - hit.b2, hit.b1, hit.b2);
     const float4 q0 = __ldg(s.triPos + 3 * (size_t)tri), q1 = __ldg(s.triPos + 3 * (size_t)tri + 1);
     const float4 q2 = __ldg(s.triPos + 3 * (size_t)tri + 2);
-    const TriShade &ts = s.triShade[PT_SHADE_INDEX(tri, q0.w)];
+    const TriShade &ts = s.triShade[__float_as_uint(q0.w)];
     const float4 a0 = __ldg(&ts.a[0]), a1 = __ldg(&ts.a[1]), a2 = __ldg(&ts.a[2]), a3 = __ldg(&ts.a[3]);
     const float4 a4 = __ldg(&ts.a[4]), a5 = __ldg(&ts.a[5]), a6 = __ldg(&ts.a[6]), a7 = __ldg(&ts.a[7]);
     const float4 a8 = __ldg(&ts.a[8]);

@@ -2,8 +2,9 @@
 # Builds a variant of libpt_core.so with extra nvcc flags into scratch/variants/<name>/ (A/B
 # experiments on the GPU box: PT_CORE_LIB=scratch/variants/<name>/libpt_core.so python bench.py ...).
 #   tools/build_variant.sh <name> [-f "file1 file2"] <extra nvcc flags ...>
-# -f lists the sources the flags apply to (default: wavefront — the only one most switches touch); the
-# other objects are taken from the in-tree build (run make there first).
+# -f lists the sources the flags apply to (default: wavefront — the only one the numeric tuning parameters
+# such as -DPT_NODE_LOOP_LANES=8 or -DPT_TRACE_MIN_BLOCKS=6 touch); the other objects are taken from the
+# in-tree build (run make there first).
 set -e
 name=$1; shift
 files="wavefront"
