@@ -411,6 +411,29 @@ PT_API pt_status pt_scene_update(pt_context *ctx, const pt_scene_update_desc *de
  * call; the accumulated image is not reset. */
 PT_API pt_status pt_set_sampler(pt_context *ctx, uint32_t max_anisotropy);
 
+/* Light sampling of next-event estimation (an extension: the reference has no counterpart).
+ *   PT_LIGHT_SAMPLING_REFERENCE     the reference's: one analytic light (point or directional) per hit (default).
+ *   PT_LIGHT_SAMPLING_EMISSIVE_MIS  also samples the scene's emissive triangles (opaque geometry whose material has
+ *                                   emissive_intensity > 0 and a non-black emissive colour or texture), in proportion to
+ *                                   area x luminance, and weights emission found by BSDF sampling with the power
+ *                                   heuristic.  Every path vertex, and with it rays_closest / hits, is that of the
+ *                                   reference mode; only the collected radiance differs.  A scene without emitters
+ *                                   renders bit for bit as in the reference mode.  Semantics: DESIGN.md section 3g.
+ * Takes effect at the next render call; the accumulated image is not reset. */
+typedef enum pt_light_sampling {
+    PT_LIGHT_SAMPLING_REFERENCE = 0,
+    PT_LIGHT_SAMPLING_EMISSIVE_MIS = 1,
+} pt_light_sampling;
+PT_API pt_status pt_set_light_sampling(pt_context *ctx, uint32_t mode);
+
+/* The emitter table of PT_LIGHT_SAMPLING_EMISSIVE_MIS (built now if it is out of date): *out_count emitters; entry k is
+ * flat triangle flat_ids[k] (flattening order: instance, mesh in model, primitive) with integer weight weights[k], drawn
+ * through the alias entry (alias_threshold[k], alias_index[k]): a uniform bucket k and a uniform 32-bit fraction x keep k
+ * when x < alias_threshold[k], else take alias_index[k].  Arrays may be NULL (count only); otherwise they hold capacity
+ * entries, and PT_ERR_INVALID_ARGUMENT is returned when capacity < count. */
+PT_API pt_status pt_emitter_table(pt_context *ctx, uint32_t *out_count, uint32_t *flat_ids, uint32_t *weights,
+                                  uint32_t *alias_threshold, uint32_t *alias_index, uint32_t capacity);
+
 /* Replaces Renderer::UpdateTexture(index) (PT/Renderer/Renderer.cpp:441-471): replace the
  * content of one texture slot (slot = PT_SCENE_TEXTURE_OFFSET + scene texture index). */
 PT_API pt_status pt_texture_upload(pt_context *ctx, uint32_t slot, const pt_texture_desc *texture);

@@ -48,7 +48,12 @@ ABI_SYMBOLS = [
     "pt_test_shading",
     "pt_test_texture",
     "pt_debug_render",
+    "pt_set_light_sampling",
+    "pt_emitter_table",
 ]
+
+# pt_light_sampling, include/pt_core.h
+LIGHT_SAMPLING = {"reference": 0, "emissive_mis": 1}
 
 
 class PtError(RuntimeError):
@@ -255,6 +260,8 @@ def lib():
     L.pt_render_samples.argtypes = [vp, vp, u32, u32, vp, u32]
     L.pt_render_frames.argtypes = [vp, vp, u32, u32, u32, vp, u32]
     L.pt_set_sampler.argtypes = [vp, u32]
+    L.pt_set_light_sampling.argtypes = [vp, u32]
+    L.pt_emitter_table.argtypes = [vp, vp, vp, vp, vp, vp, u32]
     L.pt_accum_device_ptr.argtypes = [vp, C.POINTER(vp), C.POINTER(C.c_size_t), C.POINTER(vp)]
     L.pt_readback.argtypes = [vp, vp, C.c_size_t]
     L.pt_postprocess.argtypes = [vp, vp, u32, u32, vp, C.c_size_t]
@@ -480,6 +487,23 @@ class Renderer:
 
     def set_kernel_timing(self, enable: bool):
         self._check(self._L.pt_set_kernel_timing(self._h, 1 if enable else 0))
+
+    def set_light_sampling(self, mode: str):
+        """Light sampling of next-event estimation: "reference" (default: the reference's analytic lights) or
+        "emissive_mis" (also the scene's emissive triangles, with multiple importance sampling; DESIGN.md §3g).
+        Takes effect at the next render; the accumulation is not reset."""
+        if mode not in LIGHT_SAMPLING:
+            raise ValueError(f"light sampling must be one of {sorted(LIGHT_SAMPLING)}, not {mode!r}")
+        self._check(self._L.pt_set_light_sampling(self._h, LIGHT_SAMPLING[mode]))
+
+    def emitter_table(self) -> dict:
+        """The emitter table of the "emissive_mis" mode (built now if out of date): uint32 arrays flat_ids (flattened
+        triangle ids), weights (integer selection weights) and the alias entries alias_threshold, alias_index."""
+        n = C.c_uint32(0)
+        self._check(self._L.pt_emitter_table(self._h, C.byref(n), None, None, None, None, 0))
+        t = {k: np.zeros(n.value, np.uint32) for k in ("flat_ids", "weights", "alias_threshold", "alias_index")}
+        self._check(self._L.pt_emitter_table(self._h, C.byref(n), *(t[k].ctypes.data for k in t), n.value))
+        return t
 
     def debug_render(self, params: sc.RenderParams, width: int, height: int, mode="color", raygen_flags: int = 0,
                      hit_group_flags: int = 0) -> np.ndarray:

@@ -1184,6 +1184,7 @@ void testComposeTransform(const float *meshRows, const float *instanceRows, floa
 
 void freeScene(Context *ctx)
 {
+    freeEmitters(ctx);
     freeAccel(ctx);
     if (ctx->stream)
     {
@@ -1214,6 +1215,7 @@ pt_status uploadTextureSlot(Context *ctx, uint32_t slot, const pt_texture_desc *
     // the old allocation stays owned by the scene until the next scene upload
     ctx->sceneAllocs.push_back(mem);
     ctx->hostTextures[slot] = t;
+    ctx->emittersValid = false; // an emissive texture may have changed
     PT_CUDA_CHECK(ctx, cudaMemcpyAsync(const_cast<DevTexture *>(ctx->scene.textures) + slot, &t, sizeof(t),
                                        cudaMemcpyHostToDevice, ctx->stream));
     PT_CUDA_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
@@ -1480,6 +1482,7 @@ pt_status updateScene(Context *ctx, const pt_scene_update_desc *d)
     }
     if (d->instance_transforms || d->bone_transforms)
     {
+        ctx->emittersValid = false; // the emitters' corners move with the geometry
         if (d->instance_transforms)
             for (uint32_t i = 0; i < d->instance_count; i++)
                 std::memcpy(ctx->topo.instances[i].transform, d->instance_transforms + 12 * (size_t)i, 48);

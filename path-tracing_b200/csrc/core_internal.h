@@ -63,7 +63,7 @@ struct __align__(128) PathRecord
     float4 shC;   // contribution.xyz (throughput * DirectLight / pdf), -
     float4 decal; // rgb, dist (scenes with alpha-tested geometry)
     float decalA;
-    uint32_t pad[3];
+    uint32_t pad[3]; // pad[0]: bsdf.Pdf of the previous bounce (k_shade_emissive, emissive-MIS light sampling)
     float4 spare[3];
 };
 static_assert(sizeof(PathRecord) == 256, "PathRecord must be two 128-byte lines");
@@ -80,6 +80,18 @@ struct PathState
 };
 
 #define PT_MAX_POOLS 8
+
+// Emissive triangles for next-event estimation (emitters.cu; PT_LIGHT_SAMPLING_EMISSIVE_MIS only).  Emitter k of the table
+// is flat triangle flatIds[k]; it is drawn with probability weight[k] / sum(weight) through the alias table.
+struct EmitterTable
+{
+    const float4 *rec;          // [count][4]: p0.xyz, p1.x | p1.yz, p2.xy | p2.z, uv0, uv1.x | uv1.y, uv2, material id (bits)
+    const uint2 *alias;         // [count]: (threshold of the 32-bit fraction, alias index)
+    const float *emitterPdf;    // [count]: P(select) / area of emitter k
+    const float *pdfOverArea;   // [flat triangles]: the same by flat id, 0 for triangles that are never sampled
+    uint32_t count;
+    float pEmitter;             // probability of the emitter branch of a light sample
+};
 
 // host copy of the tables instances are flattened from (kept for pt_scene_update)
 struct SceneTopology
@@ -137,6 +149,16 @@ struct Context
     float splitThreshold = 4.0f;
     uint64_t triangleCount = 0, referenceCount = 0;
     uint32_t bvhMaxDepth = 0; // levels of the wide BVH (the traversal stack holds at most 3 entries per level)
+
+    // light sampling (pt_set_light_sampling) and the emitter table, built at the first render that needs it after the
+    // scene, a texture or the sampler changed; nothing of it exists in the default mode
+    uint32_t lightSampling = PT_LIGHT_SAMPLING_REFERENCE;
+    bool emittersValid = false;
+    EmitterTable emitters = {};
+    std::vector<void *> emitterAllocs;
+    std::vector<uint32_t> emitterIds, emitterWeights;
+    std::vector<uint2> emitterAlias;
+    float emitterBuildMs = 0;
 
     // target
     uint32_t width = 0, height = 0;
@@ -230,6 +252,10 @@ pt_status uploadScene(Context *ctx, const pt_scene_desc *desc);
 void freeScene(Context *ctx);
 pt_status uploadTextureSlot(Context *ctx, uint32_t slot, const pt_texture_desc *tex);
 pt_status updateScene(Context *ctx, const pt_scene_update_desc *desc);
+
+// emitters.cu
+pt_status buildEmitters(Context *ctx);
+void freeEmitters(Context *ctx);
 
 // textures.cu
 pt_status createTexture(Context *ctx, const pt_texture_desc &desc, DevTexture &out, void **outAlloc, bool scalable = false);

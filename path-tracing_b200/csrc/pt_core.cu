@@ -464,6 +464,49 @@ pt_status pt_set_sampler(pt_context *ctx, uint32_t max_anisotropy)
         return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_set_sampler", "max_anisotropy must be in 1..16");
     ctx->maxAnisotropy = max_anisotropy;
     ctx->scene.maxAnisotropy = max_anisotropy; // the scene struct travels to every kernel by value
+    ctx->emittersValid = false;                // emitter weights are textureGrad fetches
+    return PT_OK;
+}
+
+pt_status pt_set_light_sampling(pt_context *ctx, uint32_t mode)
+{
+    if (!ctx)
+        return PT_ERR_INVALID_ARGUMENT;
+    if (mode != PT_LIGHT_SAMPLING_REFERENCE && mode != PT_LIGHT_SAMPLING_EMISSIVE_MIS)
+        return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_set_light_sampling", "unknown light-sampling mode");
+    ctx->lightSampling = mode;
+    return PT_OK;
+}
+
+pt_status pt_emitter_table(pt_context *ctx, uint32_t *out_count, uint32_t *flat_ids, uint32_t *weights,
+                           uint32_t *alias_threshold, uint32_t *alias_index, uint32_t capacity)
+{
+    if (!ctx || !out_count)
+        return PT_ERR_INVALID_ARGUMENT;
+    if (!ctx->hasScene)
+        return fail(ctx, PT_ERR_NO_SCENE, "pt_emitter_table", "no scene uploaded");
+    DeviceGuard guard(ctx->device);
+    if (!ctx->emittersValid)
+    {
+        const pt_status st = buildEmitters(ctx);
+        if (st != PT_OK)
+            return st;
+    }
+    const uint32_t n = ctx->emitters.count;
+    *out_count = n;
+    if ((flat_ids || weights || alias_threshold || alias_index) && capacity < n)
+        return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_emitter_table", "capacity is below the emitter count");
+    for (uint32_t k = 0; k < n; k++)
+    {
+        if (flat_ids)
+            flat_ids[k] = ctx->emitterIds[k];
+        if (weights)
+            weights[k] = ctx->emitterWeights[k];
+        if (alias_threshold)
+            alias_threshold[k] = ctx->emitterAlias[k].x;
+        if (alias_index)
+            alias_index[k] = ctx->emitterAlias[k].y;
+    }
     return PT_OK;
 }
 

@@ -540,5 +540,48 @@ PT_DEV LightSample sampleLight(const LightBlock *lb, vec3 u, vec3 position, floa
     return r;
 }
 
+// ---------------------------------------------------------------------------------------------
+// emissive-triangle light sampling (PT_LIGHT_SAMPLING_EMISSIVE_MIS, DESIGN.md §3g) — an extension, no GLSL
+// counterpart; tests/emissive_oracle.cpp defines the same functions
+// ---------------------------------------------------------------------------------------------
+// The emissive colour x intensity (q0) and emissive texture slot of a material; false when it cannot emit: intensity 0, or
+// a zero colour with one of the black built-in 1x1 textures (slots 4, 6, 7)
+PT_DEV bool emissiveSource(const DeviceScene &s, uint32_t materialId, float4 &q0, uint32_t &slot)
+{
+    const uint32_t type = materialId & 0xffu, index = materialId >> 8;
+    if (type > 2)
+        return false;
+    const MaterialRaw *m = (type == 0 ? s.materials[0] : type == 1 ? s.materials[1] : s.materials[2]) + index;
+    q0 = __ldg(&m->q[0]);
+    const float4 q4 = __ldg(&m->q[4]);
+    slot = __float_as_uint(type == 0 ? q4.w : q4.z);
+    const bool blackTexture = slot == 4 || slot == 6 || slot == 7;
+    return q0.w > 0.0f && (q0.x != 0.0f || q0.y != 0.0f || q0.z != 0.0f || !blackTexture);
+}
+
+// w = a^2 / (a^2 + b^2) for pdfs a, b >= 0: finite and in [0, 1] for every input, zero and infinite pdfs included
+PT_DEV float powerHeuristic(float a, float b)
+{
+    if (!(a > 0.0f))
+        return 0.0f;
+    if (!(b > 0.0f))
+        return 1.0f;
+    if (isinf(a))
+        return isinf(b) ? 0.5f : 1.0f;
+    const float r = b / a;
+    return 1.0f / (1.0f + r * r);
+}
+
+PT_DEV uint32_t xorshift(uint32_t &s)
+{
+    s ^= s << 13;
+    s ^= s >> 17;
+    s ^= s << 5;
+    return s;
+}
+
+// the secondary stream of a light sample: a hash of the main stream's state, which is not advanced by it
+PT_DEV uint32_t lightSampleRng(uint32_t rng) { return jenkinsHash(rng ^ 0x68bc21ebu); }
+
 
 } // namespace pt

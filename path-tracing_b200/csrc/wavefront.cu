@@ -381,6 +381,39 @@ __device__ __forceinline__ MaterialSample sampleMaterial(const DeviceScene &s, u
 }
 
 // ---------------------------------------------------------------------------------------------
+// emissive-MIS light sampling (DESIGN.md §3g): a uniform point on emitter k of the table, seen from `position`.  Returns the
+// light sample in sampleLight's form (Color = emission, Attenuation = 1 until the MIS weight is known) and its pdf in
+// solid angle; pdf 0 when the point cannot be seen (grazing, or a degenerate triangle).
+// ---------------------------------------------------------------------------------------------
+__device__ __forceinline__ LightSample sampleEmitter(const DeviceScene &s, const EmitterTable &em, uint32_t k, float r1, float r2,
+                                                     vec3 position, float &pdf)
+{
+    const float4 e0 = __ldg(em.rec + 4 * (size_t)k), e1 = __ldg(em.rec + 4 * (size_t)k + 1);
+    const float4 e2 = __ldg(em.rec + 4 * (size_t)k + 2), e3 = __ldg(em.rec + 4 * (size_t)k + 3);
+    const vec3 p0 = V3(e0.x, e0.y, e0.z), p1 = V3(e0.w, e1.x, e1.y), p2 = V3(e1.z, e1.w, e2.x);
+    const float su = sqrtf(r1);
+    const float b0 = 1.0f - su, b1 = su * (1.0f - r2), b2 = su * r2;
+    const vec3 y = p0 * b0 + p1 * b1 + p2 * b2;
+    const float u = e2.y * b0 + e2.w * b1 + e3.y * b2, v = e2.z * b0 + e3.x * b1 + e3.z * b2;
+    const vec3 ng = normalize(cross(p1 - p0, p2 - p0));
+    // the shadow ray's target leaves the emitter towards the shading point, so the emitter cannot occlude itself
+    const vec3 target = offsetRayOriginSelfIntersection(y, dot(ng, position - y) >= 0.0f ? ng : -ng);
+    LightSample r;
+    r.Distance = length(position - target);
+    r.Direction = normalize(position - target);
+    float4 q0;
+    uint32_t slot;
+    emissiveSource(s, __float_as_uint(e3.w), q0, slot);
+    r.Color = (V3(textureLod0(s, s.textures[slot], u, v)) + V3(q0)) * q0.w;
+    r.Attenuation = 1.0f;
+    const float cosLight = fabsf(dot(ng, r.Direction));
+    pdf = em.pEmitter * __ldg(em.emitterPdf + k) * (r.Distance * r.Distance) / cosLight;
+    if (!(pdf > 0.0f) || isinf(pdf))
+        pdf = 0.0f;
+    return r;
+}
+
+// ---------------------------------------------------------------------------------------------
 // shade: closestHit.rchit, then the raygen bounce logic (misses are finished by k_extend)
 // ---------------------------------------------------------------------------------------------
 template <bool ALPHA, bool STATS> __global__ void __launch_bounds__(128, PT_SHADE_MIN_BLOCKS) k_shade(RenderConst rc, int cur)
@@ -566,6 +599,239 @@ template <bool ALPHA, bool STATS> __global__ void __launch_bounds__(128, PT_SHAD
             rc.ps.rec[slot].diff0 = make_float4(rd.rxOrigin.x, rd.rxOrigin.y, rd.rxOrigin.z, rd.rxDirection.x);
             rc.ps.rec[slot].diff1 = make_float4(rd.rxDirection.y, rd.rxDirection.z, rd.ryOrigin.x, rd.ryOrigin.y);
             rc.ps.rec[slot].diff2 = make_float4(rd.ryOrigin.z, rd.ryDirection.x, rd.ryDirection.y, rd.ryDirection.z);
+        }
+    }
+    if (STATS)
+        warpAdd(&rc.counters->texels, texels);
+}
+
+// ---------------------------------------------------------------------------------------------
+// k_shade with emissive-triangle light sampling and MIS (pt_set_light_sampling, DESIGN.md §3g): the same closest-hit and
+// bounce logic, the same main rng stream, plus the emitter branch of the light sample, the MIS weight of emission found
+// by BSDF sampling and the previous bounce's BSDF pdf in the path record.  A copy rather than a template parameter of
+// k_shade: folding both into one body changed k_shade's machine code.
+// ---------------------------------------------------------------------------------------------
+template <bool ALPHA, bool STATS>
+__global__ void __launch_bounds__(128, PT_SHADE_MIN_BLOCKS) k_shade_emissive(RenderConst rc, int cur, EmitterTable em)
+{
+    const uint32_t n = rc.qc->hit;
+    const uint32_t stride = gridDim.x * blockDim.x;
+    const DeviceScene &s = rc.scene;
+    uint32_t texels = 0;
+    // the queue positions of k_extend, which has completed (stream order)
+    if (blockIdx.x == 0 && threadIdx.x == 0)
+        rc.qc->extendWork = 0;
+    const uint32_t *hitQueue = rc.sortHits ? rc.ps.hitQSorted : rc.ps.hitQ;
+    // (requesting the next hit's path record into L2 one loop iteration ahead was measured: no gain,
+    // the kernel is bound by issue latency at 16 warps per SM, not by the record's DRAM latency)
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
+    {
+        const uint32_t slot = hitQueue[i];
+        const float4 hitv = rc.ps.rec[slot].hit;
+        const float4 rayO = rc.ps.rec[slot].rayO, rayD = rc.ps.rec[slot].rayD;
+        // read with the rest of the record: reading throughput, radiance and the differentials again where they are
+        // used exposed the loads' latency at the end of every hit (measured: k_shade +12 %, chess)
+        float4 thr4 = rc.ps.rec[slot].thr;
+        float4 rad4 = rc.ps.rec[slot].rad;
+        vec3 throughput = V3(thr4), radiance = V3(rad4);
+        uint32_t state = __float_as_uint(thr4.w);
+        const vec3 rayDir = V3(rayD);
+        const uint32_t tri = __float_as_uint(hitv.x);
+
+        uint32_t rng = __float_as_uint(rayD.w);
+        float maxRoughness = rayO.w;
+        const float rayTmax = hitv.y;
+        const vec3 bary = V3(1.0f - hitv.z - hitv.w, hitv.z, hitv.w);
+
+        // ---- closestHit.rchit:54-83 with baked world-space data ---------------------------------
+        const float4 q0 = __ldg(s.triPos + 3 * (size_t)tri), q1 = __ldg(s.triPos + 3 * (size_t)tri + 1);
+        const float4 q2 = __ldg(s.triPos + 3 * (size_t)tri + 2);
+        const TriShade &ts = s.triShade[__float_as_uint(q0.w)];
+        const float4 a0 = __ldg(&ts.a[0]), a1 = __ldg(&ts.a[1]), a2 = __ldg(&ts.a[2]), a3 = __ldg(&ts.a[3]);
+        const float4 a4 = __ldg(&ts.a[4]), a5 = __ldg(&ts.a[5]), a6 = __ldg(&ts.a[6]), a7 = __ldg(&ts.a[7]);
+        const float4 a8 = __ldg(&ts.a[8]);
+        const uint32_t materialId = __float_as_uint(q2.w);
+        const vec3 p0 = V3(q0), p1 = V3(q1), p2 = V3(q2);
+        const vec3 n0r = V3(a0.x, a0.y, a0.z), n1r = V3(a0.w, a1.x, a1.y), n2r = V3(a1.z, a1.w, a2.x);
+        const vec3 t0r = V3(a2.y, a2.z, a2.w), t1r = V3(a3.x, a3.y, a3.z), t2r = V3(a3.w, a4.x, a4.y);
+        const vec3 b0r = V3(a4.z, a4.w, a5.x), b1r = V3(a5.y, a5.z, a5.w), b2r = V3(a6.x, a6.y, a6.z);
+        const vec2 uv0 = V2(a6.w, a7.x), uv1 = V2(a7.y, a7.z), uv2 = V2(a7.w, a8.x);
+        // MIS weight of the emission this BSDF-sampled ray found (bounce >= 1 on a triangle the light sampling can pick)
+        float emissionWeight = 1.0f;
+        if ((state & 0xffu) != 0)
+        {
+            const float pdfOverArea = __ldg(em.pdfOverArea + __float_as_uint(q0.w));
+            if (pdfOverArea > 0.0f)
+            {
+                const float4 a11 = __ldg(&ts.a[11]);
+                const float cosLight = fabsf(a11.y * rayDir.x + a11.z * rayDir.y + a11.w * rayDir.z);
+                const float pdfLight = em.pEmitter * pdfOverArea * (rayTmax * rayTmax) / cosLight;
+                emissionWeight = powerHeuristic(__uint_as_float(rc.ps.rec[slot].pad[0]), pdfLight);
+            }
+        }
+
+        const vec3 position = p0 * bary.x + p1 * bary.y + p2 * bary.z;
+        const vec2 texCoords = uv0 * bary.x + uv1 * bary.y + uv2 * bary.z;
+        vec3 normal = normalize(n0r * bary.x + n1r * bary.y + n2r * bary.z);
+        vec3 tangent = normalize(t0r * bary.x + t1r * bary.y + t2r * bary.z);
+        vec3 bitangent = normalize(b0r * bary.x + b1r * bary.y + b2r * bary.z);
+        const vec3 edge1 = p1 - p0, edge2 = p2 - p0;
+        // normalised once per triangle by k_bake (same functions, same operands)
+        const float4 a9 = __ldg(&ts.a[9]), a10 = __ldg(&ts.a[10]), a11 = __ldg(&ts.a[11]);
+        const vec3 n0 = V3(a9.x, a9.y, a9.z), n1 = V3(a9.w, a10.x, a10.y), n2 = V3(a10.z, a10.w, a11.x);
+        vec3 geometricNormal = V3(a11.y, a11.z, a11.w);
+        const bool inside = dot(geometricNormal, rayDir) > 0.0f;
+        if (inside)
+        {
+            geometricNormal = -geometricNormal;
+            normal = -normal;
+            tangent = -tangent;
+            bitangent = -bitangent;
+        }
+
+        // ---- tracing.glsl:2-28 -------------------------------------------------------------
+        vec3 dpdu, dpdv, dndu, dndv;
+        computeDpnDuv(edge1, edge2, n1 - n0, n2 - n0, uv1 - uv0, uv2 - uv0, tangent, bitangent, dpdu, dpdv, dndu, dndv);
+        const float4 d0 = rc.ps.rec[slot].diff0, d1 = rc.ps.rec[slot].diff1, d2 = rc.ps.rec[slot].diff2;
+        RayDifferentials rd;
+        rd.rxOrigin = V3(d0.x, d0.y, d0.z);
+        rd.rxDirection = V3(d0.w, d1.x, d1.y);
+        rd.ryOrigin = V3(d1.z, d1.w, d2.x);
+        rd.ryDirection = V3(d2.y, d2.z, d2.w);
+        vec3 dpdx, dpdy;
+        computeDpDxy(position, rd.rxOrigin, rd.rxDirection, rd.ryOrigin, rd.ryDirection, normal, dpdx, dpdy);
+        const float4 derivatives = computeDerivatives(dpdx, dpdy, dpdu, dpdv);
+        // Register diet: what the code AFTER the BSDF sample needs of the geometry is reduced to its results now — the
+        // ray origin of either outcome (reflected / refracted: same operations as the one call the shader makes, for
+        // both values of its flag) and the normal's screen-space derivatives — so that the triangle's corners, vertex
+        // normals, barycentrics and uv derivatives are dead while the material and the BSDF are evaluated.
+        const vec3 originReflected = offsetRayOriginShadowTerminator(position, p0, p1, p2, n0, n1, n2, bary, false);
+        const vec3 originRefracted = offsetRayOriginShadowTerminator(position, p0, p1, p2, n0, n1, n2, bary, true);
+        const vec3 originThrough = offsetRayOriginSelfIntersection(position, -geometricNormal);
+        const vec3 dndx = dndu * derivatives.x + dndv * derivatives.y;
+        const vec3 dndy = dndu * derivatives.z + dndv * derivatives.w;
+
+        // ---- material, closestHit.rchit:101-117 -------------------------------------------------
+        MaterialSample material = sampleMaterial(s, materialId, texCoords.x, texCoords.y, derivatives, inside,
+                                                 (rc.hitFlags & PT_HIT_FLAGS_DX_NORMAL_TEXTURES) != 0,
+                                                 STATS ? &texels : nullptr);
+        if (ALPHA)
+        {
+            const float4 dec = rc.ps.rec[slot].decal;
+            if (dec.w != -1.0f && rayTmax > dec.w)
+                material.Color = mix(material.Color, V3(dec), rc.ps.rec[slot].decalA);
+        }
+        maxRoughness = fmaxf(material.Roughness, maxRoughness);
+        material.Roughness = fmaxf(maxRoughness, 0.01f);
+
+        const mat3 geometryTBN = mat3 { tangent, bitangent, normal };
+        const vec3 N = normalize(normal + mul(geometryTBN, material.Normal));
+        const mat3 TBN = computeTangentSpace(N);
+        // TBN is orthonormal: inverse(TBN) == transpose(TBN)
+        const vec3 V = normalize(mulT(TBN, normalize(-rayDir)));
+
+        BSDFSample bsdf = sampleBSDF(material, V, rng);
+
+        if (inside)
+        {
+            const float e = rayTmax / material.AttenuationDistance;
+            bsdf.Color.x *= powf(material.AttenuationColor.x, e);
+            bsdf.Color.y *= powf(material.AttenuationColor.y, e);
+            bsdf.Color.z *= powf(material.AttenuationColor.z, e);
+        }
+        const bool isRefracted = bsdf.Direction.z < 0.0f;
+        const vec3 rayOrigin = isRefracted ? originRefracted : originReflected;
+
+        float lightPdf, lightSmplPdf;
+        const float l0 = rnd(rng);
+        const float l1 = rnd(rng);
+        const float l2 = rnd(rng);
+        LightSample light = sampleLight(s.lights, V3(l0, l1, l2), rayOrigin, lightPdf);
+        bool emitterSample = false;
+        // the branch, the alias draw (bucket, 32-bit fraction) and the point come from a secondary stream
+        uint32_t rng2 = lightSampleRng(rng);
+        if (rnd(rng2) < em.pEmitter)
+        {
+            const uint32_t hi = xorshift(rng2), lo = xorshift(rng2);
+            const uint32_t bucket = __umulhi(hi, em.count);
+            const uint2 entry = __ldg(em.alias + bucket);
+            const uint32_t k = lo < entry.x ? bucket : entry.y;
+            const float r1 = rnd(rng2);
+            const float r2 = rnd(rng2);
+            light = sampleEmitter(s, em, k, r1, r2, rayOrigin, lightPdf);
+            emitterSample = true;
+            // the last bounce: the reference mode never collects emission one vertex further, so neither does this
+            if ((state & 0xffu) + 1 >= rc.bounceCount)
+                lightPdf = 0.0f;
+        }
+        else
+            lightPdf = lightPdf * (1.0f - em.pEmitter);
+        const vec3 L = normalize(mulT(TBN, -light.Direction));
+        const vec3 lightBsdf = evaluateBSDF(material, V, L, lightSmplPdf);
+        if (emitterSample)
+            light.Attenuation = powerHeuristic(lightPdf, lightSmplPdf);
+
+        const vec3 newDir = normalize(mul(TBN, bsdf.Direction));
+        const vec3 newPos = isRefracted ? originThrough : rayOrigin;
+        const vec3 directLight = light.Color * light.Attenuation * lightBsdf;
+
+        propagateDifferentials(normal, rayOrigin, -rayDir, newDir, dndx, dndy, material.Eta, isRefracted, rd);
+
+        // ---- raygen.rgen:71-96 ----------------------------------------------------------------
+        radiance += throughput * (material.EmissiveColor * emissionWeight);
+        bool done = false;
+        if (bsdf.Pdf == -1.0f)
+            done = true; // raygen.rgen:71 cannot tell this from a miss
+        else
+        {
+            if (lightPdf > 0.0f)
+            {
+                const vec3 c = throughput * directLight / lightPdf;
+                // a contribution of exactly +-0 cannot change the radiance: the occlusion query is skipped.  A non-finite
+                // emitter sample is dropped: it must not cause a NaN/Inf restart the reference mode would not make.
+                if (!(c.x == 0.0f && c.y == 0.0f && c.z == 0.0f) &&
+                    !(emitterSample && (bad(c.x) || bad(c.y) || bad(c.z))))
+                {
+                    const vec3 sd = -normalize(light.Direction);
+                    rc.ps.rec[slot].shO = make_float4(newPos.x, newPos.y, newPos.z, light.Distance);
+                    rc.ps.rec[slot].shD = make_float4(sd.x, sd.y, sd.z, 0.0f);
+                    rc.ps.rec[slot].shC = make_float4(c.x, c.y, c.z, 0.0f);
+                    rc.ps.shadowQueue[atomicAggInc(&rc.qc->shadow)] = slot;
+                }
+            }
+            if (bsdf.Pdf > 0.001f)
+                throughput *= bsdf.Color / bsdf.Pdf;
+            const float prob = fminf(maxComponent(throughput), 1.0f);
+            if (prob < 0.001f)
+                done = true;
+            else if (prob < rnd(rng))
+                done = true;
+            else
+                throughput = throughput / prob;
+        }
+        const uint32_t bounce = (state & 0xffu) + 1;
+        if (bounce >= rc.bounceCount)
+            done = true;
+        state = (state & ~0xffu) | bounce;
+        // continuing paths go straight to the next iteration's queue (in shading = triangle order, so
+        // the next extend starts from spatially coherent origins); ended ones to its regen queue
+        // (their shadow ray, if any, is resolved by k_shadow before that)
+        if (done)
+            (cur ? rc.ps.regenQ[0] : rc.ps.regenQ[1])[atomicAggInc(&rc.qc->regen[cur ^ 1])] = slot | kRegen;
+        else
+            (cur ? rc.ps.contQ[0] : rc.ps.contQ[1])[atomicAggInc(&rc.qc->cont[cur ^ 1])] = slot;
+
+        rc.ps.rec[slot].rad = make_float4(radiance.x, radiance.y, radiance.z, rad4.w);
+        // the rng state outlives the path (a NaN/Inf restart continues the stream, raygen.rgen:99-112)
+        rc.ps.rec[slot].rayD = make_float4(newDir.x, newDir.y, newDir.z, __uint_as_float(rng));
+        if (!done)
+        {
+            rc.ps.rec[slot].thr = make_float4(throughput.x, throughput.y, throughput.z, __uint_as_float(state));
+            rc.ps.rec[slot].rayO = make_float4(newPos.x, newPos.y, newPos.z, maxRoughness);
+            rc.ps.rec[slot].diff0 = make_float4(rd.rxOrigin.x, rd.rxOrigin.y, rd.rxOrigin.z, rd.rxDirection.x);
+            rc.ps.rec[slot].diff1 = make_float4(rd.rxDirection.y, rd.rxDirection.z, rd.ryOrigin.x, rd.ryOrigin.y);
+            rc.ps.rec[slot].diff2 = make_float4(rd.ryOrigin.z, rd.ryDirection.x, rd.ryDirection.y, rd.ryDirection.z);
+            rc.ps.rec[slot].pad[0] = __float_as_uint(bsdf.Pdf);
         }
     }
     if (STATS)
@@ -946,6 +1212,12 @@ pt_status renderFrames(Context *ctx, const pt_render_params *params, uint32_t fi
         return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_render_frames", "samples_per_frame must be in 1..8192");
     if (tiles == nullptr)
         tileCount = 0;
+    if (ctx->lightSampling == PT_LIGHT_SAMPLING_EMISSIVE_MIS && !ctx->emittersValid)
+    {
+        const pt_status st = buildEmitters(ctx);
+        if (st != PT_OK)
+            return st;
+    }
 
     // ---- pixel list of the tile set: 8x4 pixel blocks, so that consecutive work items are
     //      neighbouring pixels and a warp's fresh primary rays are coherent -----------------------
@@ -1085,6 +1357,15 @@ pt_status renderFrames(Context *ctx, const pt_render_params *params, uint32_t fi
 
     const bool alpha = ctx->scene.hasAlpha != 0;
     const bool statsOn = ctx->collectTraversalStats;
+    // emissive-MIS light sampling: without emitters it is the reference mode, which k_shade renders bit for bit
+    const bool emissive = ctx->lightSampling == PT_LIGHT_SAMPLING_EMISSIVE_MIS && ctx->emitters.count > 0;
+    EmitterTable emitters = ctx->emitters;
+    {
+        // the emitter branch's probability: 1 when no analytic light can contribute, 1/2 otherwise
+        const LightBlock &lb = ctx->hostLights;
+        const bool analytic = lb.count > 0 || lb.dirColor.x != 0.0f || lb.dirColor.y != 0.0f || lb.dirColor.z != 0.0f;
+        emitters.pEmitter = analytic ? 0.5f : 1.0f;
+    }
     // Hits are shaded in triangle order (radix sort of the hit queue on the upper bits of the
     // leaf-order = Morton-order triangle index): neighbouring lanes then shade neighbouring
     // triangles — same material branch, same texture region, shared cache lines.  16 key bits
@@ -1217,7 +1498,10 @@ pt_status renderFrames(Context *ctx, const pt_render_params *params, uint32_t fi
                                                                    rc.ps.hitQ, rc.ps.hitQSorted, (int)rc.slotCount, 0,
                                                                    (int)keyBits + 1, st));
             }
-            PT_DISPATCH(k_shade, pl.gridShade, 128, rc, cur);
+            if (emissive)
+                PT_DISPATCH(k_shade_emissive, pl.gridShade, 128, rc, cur, emitters);
+            else
+                PT_DISPATCH(k_shade, pl.gridShade, 128, rc, cur);
             end(st);
             begin(PT_KERNEL_SHADOW, st);
             PT_DISPATCH(k_shadow, pl.gridShadow, 128, rc, cur);
