@@ -508,6 +508,32 @@ enum { PT_OUTPUT_RGBA8_SRGB = 0, PT_OUTPUT_RGBAF32 = 1 };
 PT_API pt_status pt_postprocess(pt_context *ctx, const pt_postprocess_params *params, uint32_t total_samples,
                                 uint32_t output_format, void *out_pixels, size_t out_bytes);
 
+/* ---- denoiser (DESIGN §3h) ------------------------------------------------ */
+
+/* Edge-avoiding a-trous wavelet filter (SVGF's spatial filter, Schied et al. 2017) guided by the
+ * pixel-centre primary hit's base colour, shading normal and hit distance. */
+typedef struct pt_denoise_params {
+    uint32_t iterations;   /* a-trous levels K, 0..8 (step 2^k); 0 = the mean radiance, unchanged */
+    float sigma_luminance; /* colour edge-stopping, in standard deviations (SVGF sigma_l; suggested 4)  */
+    float sigma_normal;    /* exponent of the normal weight (suggested 128)                           */
+    float sigma_depth;     /* depth edge-stopping (suggested 1)                                       */
+} pt_denoise_params;
+
+/* Denoises accumulation / total_samples of the current target. Writes width*height RGBA floats of mean radiance
+ * (A = 1) to out_rgba if it is not NULL, and keeps the result on the device for pt_postprocess_denoised.
+ * params supplies the camera the image was rendered with (the guides are traced with it); lens_radius > 0 is
+ * PT_ERR_UNSUPPORTED (pinhole guides cannot describe a defocused image). The accumulation buffer is not modified. */
+PT_API pt_status pt_denoise(pt_context *ctx, const pt_render_params *params, const pt_denoise_params *denoise,
+                            uint32_t total_samples, float *out_rgba, size_t out_bytes);
+
+/* The guide buffers of the last pt_denoise: per pixel (albedo.rgb, hit distance t; t = -1 on a miss) and
+ * (shading normal.xyz, 0). For tests and for callers with their own denoiser. Either pointer may be NULL. */
+PT_API pt_status pt_denoise_guides(pt_context *ctx, float *out_albedo_t, float *out_normal, size_t out_bytes);
+
+/* pt_postprocess's chain (exposure, bloom, tone map, output format) on the last pt_denoise result. */
+PT_API pt_status pt_postprocess_denoised(pt_context *ctx, const pt_postprocess_params *params, uint32_t output_format,
+                                         void *out_pixels, size_t out_bytes);
+
 /* Waits for all queued work of the context. */
 PT_API pt_status pt_synchronize(pt_context *ctx);
 

@@ -50,6 +50,9 @@ ABI_SYMBOLS = [
     "pt_debug_render",
     "pt_set_light_sampling",
     "pt_emitter_table",
+    "pt_denoise",
+    "pt_denoise_guides",
+    "pt_postprocess_denoised",
 ]
 
 # pt_light_sampling, include/pt_core.h
@@ -71,6 +74,12 @@ class PostProcessParams(C.Structure):
     """pt_postprocess_params = Renderer::PostProcessSettings (Path-Tracing/Renderer/Renderer.h:68-73) + tone-mapping mode."""
 
     _fields_ = [("exposure", C.c_float), ("bloom_threshold", C.c_float), ("bloom_intensity", C.c_float), ("tone_mapping", C.c_uint32)]
+
+
+class DenoiseParams(C.Structure):
+    """pt_denoise_params: a-trous levels and the edge-stopping parameters of the denoiser (DESIGN.md §3h)."""
+
+    _fields_ = [("iterations", C.c_uint32), ("sigma_luminance", C.c_float), ("sigma_normal", C.c_float), ("sigma_depth", C.c_float)]
 
 
 class SceneUpdateDesc(C.Structure):
@@ -280,6 +289,9 @@ def lib():
     L.pt_test_shading.argtypes = [vp, u32, vp, vp, u32]
     L.pt_test_texture.argtypes = [vp, u32, vp, vp, u32, i32]
     L.pt_debug_render.argtypes = [vp, vp, vp, u32, u32, vp]
+    L.pt_denoise.argtypes = [vp, vp, vp, u32, vp, C.c_size_t]
+    L.pt_denoise_guides.argtypes = [vp, vp, vp, C.c_size_t]
+    L.pt_postprocess_denoised.argtypes = [vp, vp, u32, vp, C.c_size_t]
     _lib = L
     return L
 
@@ -401,17 +413,39 @@ class Renderer:
         return out
 
     def postprocess(self, exposure: float = 1.0, bloom_threshold: float = 1.0, bloom_intensity: float = 0.1, hdr: bool = False,
-                    total_samples: int | None = None) -> np.ndarray:
+                    total_samples: int | None = None, denoised: bool = False) -> np.ndarray:
         """What the reference's "Render" button writes (Renderer::RecordPostProcessCommands +
         RecordSaveOutputCommands + OutputSaver): exposure, bloom, tone mapping and the output-format
         conversion of the accumulated image.  (H, W, 4) uint8 sRGB, or float32 with hdr (the .hdr output,
-        not tone-mapped)."""
+        not tone-mapped).  denoised=True runs the same chain on the result of the last denoise() instead."""
         p = PostProcessParams(exposure, bloom_threshold, bloom_intensity, TONE_MAPPING_HDR if hdr else TONE_MAPPING_SDR)
         out = np.empty((self.height, self.width, 4), np.float32 if hdr else np.uint8)
+        fmt = OUTPUT_RGBAF32 if hdr else OUTPUT_RGBA8_SRGB
+        if denoised:
+            self._check(self._L.pt_postprocess_denoised(self._h, C.addressof(p), fmt, out.ctypes.data, out.nbytes))
+            return out
         n = self.total_samples if total_samples is None else total_samples
-        self._check(self._L.pt_postprocess(self._h, C.addressof(p), int(n), OUTPUT_RGBAF32 if hdr else OUTPUT_RGBA8_SRGB,
-                                           out.ctypes.data, out.nbytes))
+        self._check(self._L.pt_postprocess(self._h, C.addressof(p), int(n), fmt, out.ctypes.data, out.nbytes))
         return out
+
+    def denoise(self, params: sc.RenderParams | None = None, iterations: int = 5, sigma_luminance: float = 4.0,
+                sigma_normal: float = 128.0, sigma_depth: float = 1.0, total_samples: int | None = None) -> np.ndarray:
+        """Edge-avoiding a-trous denoiser (DESIGN.md §3h) of accumulation / total_samples, guided by the first hit of the
+        camera in params (default: the settings rendered with): (H, W, 4) float32 mean radiance, A = 1.  The result
+        stays on the device for postprocess(denoised=True) and the save_* writers; the accumulation is unchanged."""
+        p = (params or self.params).to_c()
+        d = DenoiseParams(int(iterations), sigma_luminance, sigma_normal, sigma_depth)
+        n = self.total_samples if total_samples is None else total_samples
+        out = np.empty((self.height, self.width, 4), np.float32)
+        self._check(self._L.pt_denoise(self._h, C.addressof(p), C.addressof(d), int(n), out.ctypes.data, out.nbytes))
+        return out
+
+    def denoise_guides(self) -> dict:
+        """The guides of the last denoise(): "albedo" (H, W, 3), "t" (H, W; -1 on a miss) and "normal" (H, W, 3)."""
+        at = np.empty((self.height, self.width, 4), np.float32)
+        nrm = np.empty((self.height, self.width, 4), np.float32)
+        self._check(self._L.pt_denoise_guides(self._h, at.ctypes.data, nrm.ctypes.data, at.nbytes))
+        return {"albedo": at[..., :3], "t": at[..., 3], "normal": nrm[..., :3]}
 
     def save_png(self, path: str, **postprocess_args):
         """OutputSaver::WriteImage for OutputFormat::Png (Path-Tracing/Renderer/OutputSaver.cpp:227-253):

@@ -165,6 +165,12 @@ struct Context
     float4 *accum = nullptr;
     PathState ps = {};
     std::vector<void *> targetAllocs;
+    // denoiser buffers (denoise.cu), one target allocation made at the first pt_denoise: guides (albedo, t) and (N, 0), the
+    // result, the filter's (N, t) taps, two ping-pong (irradiance, variance) images and the depth gradient
+    float4 *denoiseAlbedoT = nullptr, *denoiseNormal = nullptr, *denoised = nullptr, *denoiseNT = nullptr;
+    float4 *denoisePing = nullptr, *denoisePong = nullptr;
+    float2 *denoiseGrad = nullptr;
+    bool denoiseValid = false; // a pt_denoise result exists for the current accumulation
     size_t slotPoolSize = (size_t)1 << 23;     // paths in flight, all pools together (PT_SLOTS)
     size_t sbufBudgetBytes = (size_t)8 << 30;  // sample-buffer budget (PT_SBUF_MB)
     uint32_t slotCapacity = 0; // size of the slot pool
@@ -270,10 +276,17 @@ pt_status debugRender(Context *ctx, const pt_render_params *params, const pt_deb
                       float *out);
 pt_status traceClosest(Context *ctx, const pt_ray *rays, uint64_t n, pt_hit *out);
 pt_status traceOcclusion(Context *ctx, const pt_ray *rays, uint64_t n, uint8_t *out);
+// k_denoise_guides over the render target's extent, queued on ctx->stream
+void launchDenoiseGuides(Context *ctx, const pt_render_params *params, float4 *albedoT, float4 *normal);
+
+// denoise.cu
+pt_status denoise(Context *ctx, const pt_render_params *params, const pt_denoise_params *dn, uint32_t totalSamples, float *out,
+                  size_t outBytes);
 
 // postprocess.cu
-pt_status postProcess(Context *ctx, const pt_postprocess_params *params, uint32_t totalSamples, uint32_t outputFormat,
-                      void *out, size_t outBytes);
+// src / divisor is the image the chain starts from: the accumulation and its sample count, or the denoised mean and 1
+pt_status postProcess(Context *ctx, const char *what, const pt_postprocess_params *params, const float4 *src, float divisor,
+                      uint32_t outputFormat, void *out, size_t outBytes);
 
 // unit_kernels.cu
 void testComposeTransform(const float *meshRows, const float *instanceRows, float P[12], float N[9]);

@@ -164,21 +164,21 @@ __global__ void __launch_bounds__(256) k_post_output(const uint2 *__restrict__ c
 
 } // namespace
 
-pt_status postProcess(Context *ctx, const pt_postprocess_params *p, uint32_t totalSamples, uint32_t outputFormat, void *out,
-                      size_t outBytes)
+pt_status postProcess(Context *ctx, const char *what, const pt_postprocess_params *p, const float4 *src, float divisor,
+                      uint32_t outputFormat, void *out, size_t outBytes)
 {
     if (!p || !out)
-        return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_postprocess", "NULL argument");
+        return fail(ctx, PT_ERR_INVALID_ARGUMENT, what, "NULL argument");
     if (!ctx->accum)
-        return fail(ctx, PT_ERR_NO_TARGET, "pt_postprocess", "pt_render_begin has not been called");
+        return fail(ctx, PT_ERR_NO_TARGET, what, "pt_render_begin has not been called");
     if (outputFormat != PT_OUTPUT_RGBA8_SRGB && outputFormat != PT_OUTPUT_RGBAF32)
-        return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_postprocess", "unknown output format");
+        return fail(ctx, PT_ERR_INVALID_ARGUMENT, what, "unknown output format");
     if (p->tone_mapping > PT_TONE_MAPPING_HDR)
-        return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_postprocess", "unknown tone-mapping mode");
+        return fail(ctx, PT_ERR_INVALID_ARGUMENT, what, "unknown tone-mapping mode");
     const uint32_t W = ctx->width, H = ctx->height;
     const size_t n = (size_t)W * H, need = n * (outputFormat == PT_OUTPUT_RGBA8_SRGB ? 4 : 16);
     if (outBytes < need)
-        return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_postprocess", "output buffer too small");
+        return fail(ctx, PT_ERR_INVALID_ARGUMENT, what, "output buffer too small");
 
     // floor(log2(max(w, h))) + 1 levels (PT/Renderer/Image.cpp:14-17)
     uint32_t levels = 1;
@@ -213,7 +213,7 @@ pt_status postProcess(Context *ctx, const pt_postprocess_params *p, uint32_t tot
         cursor += (size_t)bloom[l].w * bloom[l].h;
     }
     const uint32_t wide = (uint32_t)std::min<size_t>((n + 255) / 256, (size_t)ctx->smCount * 8);
-    k_post_prefilter<<<wide, 256, 0, st>>>(ctx->accum, (uint32_t)n, (float)totalSamples, p->exposure, p->bloom_threshold, color,
+    k_post_prefilter<<<wide, 256, 0, st>>>(src, (uint32_t)n, divisor, p->exposure, p->bloom_threshold, color,
                                            bloom[0].px);
     const dim3 block(32, 8);
     for (uint32_t i = 0; i + 1 < maxMip; i++)

@@ -28,6 +28,10 @@ static void freeTarget(Context *ctx)
         cudaFree(p);
     ctx->targetAllocs.clear();
     ctx->accum = nullptr;
+    ctx->denoiseAlbedoT = ctx->denoiseNormal = ctx->denoised = ctx->denoiseNT = nullptr;
+    ctx->denoisePing = ctx->denoisePong = nullptr;
+    ctx->denoiseGrad = nullptr;
+    ctx->denoiseValid = false;
     ctx->ps = PathState {};
     ctx->slotCapacity = 0;
     ctx->pixelList = nullptr;
@@ -262,6 +266,7 @@ pt_status pt_render_begin(pt_context *ctx, uint32_t width, uint32_t height)
         ctx->slotCapacity = (uint32_t)slots;
     }
     PT_CUDA_CHECK(ctx, cudaMemsetAsync(ctx->accum, 0, n * sizeof(float4), ctx->stream));
+    ctx->denoiseValid = false;
     return PT_OK;
 }
 
@@ -327,7 +332,49 @@ pt_status pt_postprocess(pt_context *ctx, const pt_postprocess_params *params, u
     if (!ctx)
         return PT_ERR_INVALID_ARGUMENT;
     DeviceGuard guard(ctx->device);
-    return postProcess(ctx, params, total_samples, output_format, out_pixels, out_bytes);
+    return postProcess(ctx, "pt_postprocess", params, ctx->accum, (float)total_samples, output_format, out_pixels, out_bytes);
+}
+
+pt_status pt_denoise(pt_context *ctx, const pt_render_params *params, const pt_denoise_params *denoise_params,
+                     uint32_t total_samples, float *out_rgba, size_t out_bytes)
+{
+    if (!ctx)
+        return PT_ERR_INVALID_ARGUMENT;
+    DeviceGuard guard(ctx->device);
+    return denoise(ctx, params, denoise_params, total_samples, out_rgba, out_bytes);
+}
+
+pt_status pt_denoise_guides(pt_context *ctx, float *out_albedo_t, float *out_normal, size_t out_bytes)
+{
+    if (!ctx)
+        return PT_ERR_INVALID_ARGUMENT;
+    if (!ctx->accum)
+        return fail(ctx, PT_ERR_NO_TARGET, "pt_denoise_guides", "pt_render_begin has not been called");
+    if (!ctx->denoiseValid)
+        return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_denoise_guides", "no pt_denoise since the last pt_render_begin");
+    const size_t need = (size_t)ctx->width * ctx->height * sizeof(float4);
+    if (out_bytes < need)
+        return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_denoise_guides", "output buffer too small");
+    DeviceGuard guard(ctx->device);
+    if (out_albedo_t)
+        PT_CUDA_CHECK(ctx, cudaMemcpyAsync(out_albedo_t, ctx->denoiseAlbedoT, need, cudaMemcpyDeviceToHost, ctx->stream));
+    if (out_normal)
+        PT_CUDA_CHECK(ctx, cudaMemcpyAsync(out_normal, ctx->denoiseNormal, need, cudaMemcpyDeviceToHost, ctx->stream));
+    PT_CUDA_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
+    return PT_OK;
+}
+
+pt_status pt_postprocess_denoised(pt_context *ctx, const pt_postprocess_params *params, uint32_t output_format, void *out_pixels,
+                                  size_t out_bytes)
+{
+    if (!ctx)
+        return PT_ERR_INVALID_ARGUMENT;
+    if (!ctx->accum)
+        return fail(ctx, PT_ERR_NO_TARGET, "pt_postprocess_denoised", "pt_render_begin has not been called");
+    if (!ctx->denoiseValid)
+        return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_postprocess_denoised", "no pt_denoise since the last pt_render_begin");
+    DeviceGuard guard(ctx->device);
+    return postProcess(ctx, "pt_postprocess_denoised", params, ctx->denoised, 1.0f, output_format, out_pixels, out_bytes);
 }
 
 pt_status pt_synchronize(pt_context *ctx)

@@ -995,36 +995,34 @@ __device__ __forceinline__ vec3 debugLightContribution(vec3 lightDir, vec3 light
     return (kD * color / PT_PI + specular) * radiance * NdotL;
 }
 
-template <bool ALPHA_PRIMARY, bool ALPHA_SHADOW, bool CULL>
-__global__ void k_debug(DeviceScene s, CameraMatrices cam, uint32_t width, uint32_t height, uint32_t missFlags, pt_debug_params dbg,
-                        float4 *out)
+// The pixel-centre primary hit of k_debug and k_denoise_guides (debugRaygen.rgen + debugClosestHit.rchit:163-265 on the
+// baked world-space triangle): the surface, its material (textureGrad with the ray-differential derivatives, the decal mixed
+// into the base colour on alpha scenes) and the normal-mapped shading normal N.  flags are PT_DEBUG_HIT_* bits.
+struct PrimarySurface
 {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= width * height)
-        return;
-    const uint32_t px = i % width, py = i / width;
-    const PrimaryRays pr = constructPrimaryRay((float)px, (float)py, (float)width, (float)height, cam, V2(0.5f, 0.5f),
-                                               V2(0.0f, 0.0f), 0.0f, 0.0f);
+    PrimaryRays pr;
     Hit hit;
+    vec3 bary, p0, p1, p2, n0r, n1r, n2r, position, normal, N;
+    vec2 texCoords;
+    float4 ids; // TriShade a[8]: -, instance, geometry, primitive (bits)
+    float4 derivatives;
+    MaterialSample material;
+};
+
+// false on a miss (sf.pr and sf.hit are set)
+template <bool ALPHA_PRIMARY, bool CULL>
+__device__ __forceinline__ bool tracePrimarySurface(const DeviceScene &s, const CameraMatrices &cam, uint32_t px, uint32_t py,
+                                                    uint32_t width, uint32_t height, uint32_t flags, PrimarySurface &sf)
+{
+    sf.pr = constructPrimaryRay((float)px, (float)py, (float)width, (float)height, cam, V2(0.5f, 0.5f), V2(0.0f, 0.0f), 0.0f, 0.0f);
+    const PrimaryRays &pr = sf.pr;
+    Hit &hit = sf.hit;
     Decal decal;
     TraversalStats st;
     traverse<true, ALPHA_PRIMARY, false, CULL>(s, pr.origin, pr.direction, 0.00001f, 10000.0f, hit, decal, st);
     if (hit.tri == 0xffffffffu)
-    {
-        // debugMiss.rmiss:17-36 (no hdrToLdr here)
-        vec3 c = V3(0.2f, 0.2f, 0.2f);
-        if ((missFlags & PT_MISS_FLAGS_SKYBOX_2D) && s.hasSky2D)
-        {
-            const float longitude = atan2f(pr.direction.z, pr.direction.x), latitude = asinf(-pr.direction.y);
-            c = V3(textureLod0(s, s.sky2D, longitude / 2.0f / PT_PI + 0.5f, latitude / PT_PI + 0.5f));
-        }
-        else if ((missFlags & PT_MISS_FLAGS_SKYBOX_CUBE) && s.skyCubeSlot)
-            c = V3(sampleCube(s, s.skyCubeSlot, pr.direction));
-        out[i] = make_float4(c.x, c.y, c.z, 1.0f);
-        return;
-    }
+        return false;
 
-    // debugClosestHit.rchit:163-265 on the baked world-space triangle
     const uint32_t tri = hit.tri;
     const vec3 bary = V3(1.0f - hit.b1 - hit.b2, hit.b1, hit.b2);
     const float4 q0 = __ldg(s.triPos + 3 * (size_t)tri), q1 = __ldg(s.triPos + 3 * (size_t)tri + 1);
@@ -1044,7 +1042,6 @@ __global__ void k_debug(DeviceScene s, CameraMatrices cam, uint32_t width, uint3
     const vec3 normal = normalize(n0r * bary.x + n1r * bary.y + n2r * bary.z);
     const vec3 tangent = normalize(t0r * bary.x + t1r * bary.y + t2r * bary.z);
     const vec3 bitangent = normalize(b0r * bary.x + b1r * bary.y + b2r * bary.z);
-    const vec3 n0 = normalize(n0r), n1 = normalize(n1r), n2 = normalize(n2r);
 
     // tracing.glsl:2-28
     vec3 dpdu, dpdv;
@@ -1073,16 +1070,61 @@ __global__ void k_debug(DeviceScene s, CameraMatrices cam, uint32_t width, uint3
         dpdx = (pr.origin + tx * pr.rxDirection) - position;
         dpdy = (pr.origin + ty * pr.ryDirection) - position;
     }
-    const uint32_t flags = dbg.hit_group_flags;
     const float4 derivatives =
         (flags & PT_DEBUG_HIT_DISABLE_MIP_MAPS) ? make_float4(0.0f, 0.0f, 0.0f, 0.0f) : computeDerivatives(dpdx, dpdy, dpdu, dpdv);
     MaterialSample material = sampleMaterial(s, materialId, texCoords.x, texCoords.y, derivatives, false,
                                              (flags & PT_DEBUG_HIT_DX_NORMAL_TEXTURES) != 0, nullptr, flags);
     if (ALPHA_PRIMARY && decal.dist != -1.0f && hit.t > decal.dist)
         material.Color = mix(material.Color, V3(decal.r, decal.g, decal.b), decal.a);
-    const vec3 V = -normalize(pr.direction);
     const mat3 TBN = mat3 { tangent, bitangent, normal };
-    const vec3 N = normalize(normal + mul(TBN, material.Normal));
+    sf.N = normalize(normal + mul(TBN, material.Normal));
+    sf.bary = bary;
+    sf.p0 = p0;
+    sf.p1 = p1;
+    sf.p2 = p2;
+    sf.n0r = n0r;
+    sf.n1r = n1r;
+    sf.n2r = n2r;
+    sf.position = position;
+    sf.normal = normal;
+    sf.texCoords = texCoords;
+    sf.ids = a8;
+    sf.derivatives = derivatives;
+    sf.material = material;
+    return true;
+}
+
+template <bool ALPHA_PRIMARY, bool ALPHA_SHADOW, bool CULL>
+__global__ void k_debug(DeviceScene s, CameraMatrices cam, uint32_t width, uint32_t height, uint32_t missFlags, pt_debug_params dbg,
+                        float4 *out)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= width * height)
+        return;
+    const uint32_t px = i % width, py = i / width;
+    const uint32_t flags = dbg.hit_group_flags;
+    PrimarySurface sf;
+    if (!tracePrimarySurface<ALPHA_PRIMARY, CULL>(s, cam, px, py, width, height, flags, sf))
+    {
+        // debugMiss.rmiss:17-36 (no hdrToLdr here)
+        const PrimaryRays &pr = sf.pr;
+        vec3 c = V3(0.2f, 0.2f, 0.2f);
+        if ((missFlags & PT_MISS_FLAGS_SKYBOX_2D) && s.hasSky2D)
+        {
+            const float longitude = atan2f(pr.direction.z, pr.direction.x), latitude = asinf(-pr.direction.y);
+            c = V3(textureLod0(s, s.sky2D, longitude / 2.0f / PT_PI + 0.5f, latitude / PT_PI + 0.5f));
+        }
+        else if ((missFlags & PT_MISS_FLAGS_SKYBOX_CUBE) && s.skyCubeSlot)
+            c = V3(sampleCube(s, s.skyCubeSlot, pr.direction));
+        out[i] = make_float4(c.x, c.y, c.z, 1.0f);
+        return;
+    }
+    const vec3 bary = sf.bary, p0 = sf.p0, p1 = sf.p1, p2 = sf.p2, position = sf.position, N = sf.N;
+    const vec3 n0 = normalize(sf.n0r), n1 = normalize(sf.n1r), n2 = normalize(sf.n2r);
+    const vec2 texCoords = sf.texCoords;
+    const float4 derivatives = sf.derivatives, a8 = sf.ids;
+    const MaterialSample &material = sf.material;
+    const vec3 V = -normalize(sf.pr.direction);
 
     vec3 result;
     switch (dbg.render_mode)
@@ -1138,6 +1180,27 @@ __global__ void k_debug(DeviceScene s, CameraMatrices cam, uint32_t width, uint3
     }
     }
     out[i] = make_float4(result.x, result.y, result.z, 1.0f);
+}
+
+// Guides of the denoiser (denoise.cu): k_debug's primary surface with its default flags, per pixel (base colour, hit
+// distance t; t = -1 on a miss) and (shading normal N, 0)
+template <bool ALPHA>
+__global__ void k_denoise_guides(DeviceScene s, CameraMatrices cam, uint32_t width, uint32_t height, uint32_t flags, float4 *albedoT,
+                                 float4 *normal)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= width * height)
+        return;
+    PrimarySurface sf;
+    if (!tracePrimarySurface<ALPHA, false>(s, cam, i % width, i / width, width, height, flags, sf))
+    {
+        albedoT[i] = make_float4(0.0f, 0.0f, 0.0f, -1.0f);
+        normal[i] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+        return;
+    }
+    const vec3 c = sf.material.Color;
+    albedoT[i] = make_float4(c.x, c.y, c.z, sf.hit.t);
+    normal[i] = make_float4(sf.N.x, sf.N.y, sf.N.z, 0.0f);
 }
 
 template <bool ALPHA> __global__ void k_trace_closest(DeviceScene s, const pt_ray *rays, uint64_t n, pt_hit *out)
@@ -1649,6 +1712,17 @@ pt_status debugRender(Context *ctx, const pt_render_params *params, const pt_deb
     cudaFreeAsync(dOut, ctx->stream);
     PT_CUDA_CHECK(ctx, err);
     return checkStackOverflow(ctx, "pt_debug_render");
+}
+
+void launchDenoiseGuides(Context *ctx, const pt_render_params *params, float4 *albedoT, float4 *normal)
+{
+    const uint32_t width = ctx->width, height = ctx->height;
+    const uint32_t grid = (uint32_t)(((size_t)width * height + 127) / 128);
+    const uint32_t flags = (params->hit_flags & PT_HIT_FLAGS_DX_NORMAL_TEXTURES) ? PT_DEBUG_HIT_DX_NORMAL_TEXTURES : 0u;
+    if (ctx->scene.hasAlpha)
+        k_denoise_guides<true><<<grid, 128, 0, ctx->stream>>>(ctx->scene, toCamera(params), width, height, flags, albedoT, normal);
+    else
+        k_denoise_guides<false><<<grid, 128, 0, ctx->stream>>>(ctx->scene, toCamera(params), width, height, flags, albedoT, normal);
 }
 
 pt_status traceClosest(Context *ctx, const pt_ray *rays, uint64_t n, pt_hit *out)
