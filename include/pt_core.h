@@ -534,6 +534,50 @@ PT_API pt_status pt_denoise_guides(pt_context *ctx, float *out_albedo_t, float *
 PT_API pt_status pt_postprocess_denoised(pt_context *ctx, const pt_postprocess_params *params, uint32_t output_format,
                                          void *out_pixels, size_t out_bytes);
 
+/* ---- adaptive sampling (DESIGN §3i) --------------------------------------- */
+
+/* Each pixel keeps its sample count and Welford statistics (mean, M2) of its samples' luminance
+ * l = (0.2126 r + 0.7152 g) + 0.0722 b.  A pixel is converged when M2 <= t^2 (mean^2 + 0.01) n (n - 1), i.e. the
+ * relative standard error of its mean is at most t = threshold.  Pixels move in 8x4 blocks aligned at (0, 0): a block
+ * is active while its count is below min_samples, or below max_samples with a pixel that is not converged. */
+typedef struct pt_adaptive_params {
+    uint32_t min_samples;    /* >= 2: every pixel's samples before its error is first judged           */
+    uint32_t max_samples;    /* >= min_samples: per-pixel cap                                          */
+    uint32_t batch;          /* >= 1: samples between two judgements                                   */
+    uint32_t min_pass_items; /* 0 = 2^21: a pass renders at least this many (pixel, sample) items      */
+    float threshold;         /* >= 0, finite: relative standard error at which a block stops           */
+} pt_adaptive_params;
+
+typedef struct pt_adaptive_info {
+    uint32_t passes;
+    uint32_t min_count, max_count;   /* over the frame after the call                              */
+    uint32_t unconverged_pixels;     /* pixels that stopped at max_samples without meeting threshold */
+    uint64_t samples;                /* (pixel, sample) items rendered by this call                 */
+} pt_adaptive_info;
+
+/* Renders until no block is active.  Each pass takes the smallest count n among the active blocks and the next larger
+ * one, `next`, and renders samples [n, n + k) of the A pixels of the active blocks at n, with
+ * k = min(max_samples, next, max(n + batch, min_samples, n + ceil(min_pass_items / A))) - n.  Sample s of a pixel is the
+ * sample s of pt_render_samples (first_sample 0, the whole frame), so a pixel with n samples holds exactly the
+ * accumulation of a uniform n-sample render.  A later call on the same target continues with its own parameters (a lower
+ * threshold or a higher cap refines further).  A target holds a uniform render or an adaptive one: this call fails with
+ * PT_ERR_INVALID_ARGUMENT after pt_render_samples / pt_render_frames wrote to the target, and those fail on a target
+ * holding an adaptive render, until pt_render_begin.  pt_stats covers the whole call.  Blocking. */
+PT_API pt_status pt_render_adaptive(pt_context *ctx, const pt_render_params *params, const pt_adaptive_params *adaptive,
+                                    pt_adaptive_info *out_info /* may be NULL */);
+
+/* Per pixel (row-major, `pixels` >= width * height): the sample count, and (mean luminance, M2). Either pointer may be NULL. */
+PT_API pt_status pt_adaptive_readback(pt_context *ctx, uint32_t *out_counts, float *out_mean_m2, size_t pixels);
+
+/* pt_postprocess's chain on the mean image accum / count of an adaptive render (the divisor is 1). */
+PT_API pt_status pt_postprocess_adaptive(pt_context *ctx, const pt_postprocess_params *params, uint32_t output_format,
+                                         void *out_pixels, size_t out_bytes);
+
+/* pt_denoise's filter on the mean image accum / count of an adaptive render (the divisor is 1); the result is kept for
+ * pt_postprocess_denoised like pt_denoise's. */
+PT_API pt_status pt_denoise_adaptive(pt_context *ctx, const pt_render_params *params, const pt_denoise_params *denoise,
+                                     float *out_rgba, size_t out_bytes);
+
 /* Waits for all queued work of the context. */
 PT_API pt_status pt_synchronize(pt_context *ctx);
 

@@ -53,6 +53,10 @@ ABI_SYMBOLS = [
     "pt_denoise",
     "pt_denoise_guides",
     "pt_postprocess_denoised",
+    "pt_render_adaptive",
+    "pt_adaptive_readback",
+    "pt_postprocess_adaptive",
+    "pt_denoise_adaptive",
 ]
 
 # pt_light_sampling, include/pt_core.h
@@ -80,6 +84,20 @@ class DenoiseParams(C.Structure):
     """pt_denoise_params: a-trous levels and the edge-stopping parameters of the denoiser (DESIGN.md §3h)."""
 
     _fields_ = [("iterations", C.c_uint32), ("sigma_luminance", C.c_float), ("sigma_normal", C.c_float), ("sigma_depth", C.c_float)]
+
+
+class AdaptiveParams(C.Structure):
+    """pt_adaptive_params: per-pixel sample counts of an adaptive render (DESIGN.md §3i)."""
+
+    _fields_ = [("min_samples", C.c_uint32), ("max_samples", C.c_uint32), ("batch", C.c_uint32), ("min_pass_items", C.c_uint32),
+                ("threshold", C.c_float)]
+
+
+class AdaptiveInfo(C.Structure):
+    """pt_adaptive_info: what one pt_render_adaptive call did."""
+
+    _fields_ = [("passes", C.c_uint32), ("min_count", C.c_uint32), ("max_count", C.c_uint32), ("unconverged_pixels", C.c_uint32),
+                ("samples", C.c_uint64)]
 
 
 class SceneUpdateDesc(C.Structure):
@@ -292,6 +310,10 @@ def lib():
     L.pt_denoise.argtypes = [vp, vp, vp, u32, vp, C.c_size_t]
     L.pt_denoise_guides.argtypes = [vp, vp, vp, C.c_size_t]
     L.pt_postprocess_denoised.argtypes = [vp, vp, u32, vp, C.c_size_t]
+    L.pt_render_adaptive.argtypes = [vp, vp, vp, vp]
+    L.pt_adaptive_readback.argtypes = [vp, vp, vp, C.c_size_t]
+    L.pt_postprocess_adaptive.argtypes = [vp, vp, u32, vp, C.c_size_t]
+    L.pt_denoise_adaptive.argtypes = [vp, vp, vp, vp, C.c_size_t]
     _lib = L
     return L
 
@@ -306,6 +328,7 @@ class Renderer:
         self._h = h
         self.width = self.height = 0
         self.total_samples = 0
+        self.adaptive = False  # the target holds an adaptive render (render_adaptive) until on_resize
         self.params: sc.RenderParams | None = None
 
     # -- plumbing ---------------------------------------------------------------------------
@@ -376,6 +399,7 @@ class Renderer:
         self._check(self._L.pt_render_begin(self._h, width, height))
         self.width, self.height = width, height
         self.total_samples = 0
+        self.adaptive = False
 
     def set_settings(self, params: sc.RenderParams):
         self.params = params
@@ -405,6 +429,34 @@ class Renderer:
         if first_sample is None:
             self.total_samples += frames * samples_per_frame
 
+    def render_adaptive(self, min_samples: int = 16, max_samples: int = 1024, batch: int = 16, threshold: float = 0.02,
+                        min_pass_items: int = 0, params: sc.RenderParams | None = None) -> dict:
+        """Adaptive sampling (DESIGN.md §3i): samples 8x4 pixel blocks until the relative standard error of every pixel's
+        mean luminance is at most threshold, each pixel between min_samples and max_samples.  A pixel with n samples holds
+        exactly the accumulation of an n-sample render(); a second call refines the same target.  While the target holds
+        the adaptive render, postprocess(), denoise() and the save_* writers use the mean image accumulation / count.
+        Returns pt_adaptive_info as a dict."""
+        p = (params or self.params).to_c()
+        a = AdaptiveParams(int(min_samples), int(max_samples), int(batch), int(min_pass_items), float(threshold))
+        info = AdaptiveInfo()
+        self._check(self._L.pt_render_adaptive(self._h, C.addressof(p), C.addressof(a), C.addressof(info)))
+        self.adaptive = True
+        return {n: int(getattr(info, n)) for n, _ in AdaptiveInfo._fields_}
+
+    def sample_counts(self) -> np.ndarray:
+        """(H, W) uint32 sample count of every pixel of the adaptive render."""
+        out = np.empty((self.height, self.width), np.uint32)
+        self._check(self._L.pt_adaptive_readback(self._h, out.ctypes.data, None, out.size))
+        return out
+
+    def adaptive_statistics(self) -> dict:
+        """Per pixel of the adaptive render: "count" (H, W) uint32, and the Welford statistics of its samples' luminance,
+        "mean" and "m2" (H, W) float32 (the sample variance is m2 / (count - 1))."""
+        counts = np.empty((self.height, self.width), np.uint32)
+        mm = np.empty((self.height, self.width, 2), np.float32)
+        self._check(self._L.pt_adaptive_readback(self._h, counts.ctypes.data, mm.ctypes.data, counts.size))
+        return {"count": counts, "mean": mm[..., 0], "m2": mm[..., 1]}
+
     def read_accumulation(self, out: np.ndarray | None = None) -> np.ndarray:
         if out is None:
             out = np.empty((self.height, self.width, 4), np.float32)
@@ -417,12 +469,16 @@ class Renderer:
         """What the reference's "Render" button writes (Renderer::RecordPostProcessCommands +
         RecordSaveOutputCommands + OutputSaver): exposure, bloom, tone mapping and the output-format
         conversion of the accumulated image.  (H, W, 4) uint8 sRGB, or float32 with hdr (the .hdr output,
-        not tone-mapped).  denoised=True runs the same chain on the result of the last denoise() instead."""
+        not tone-mapped).  denoised=True runs the same chain on the result of the last denoise() instead; after
+        render_adaptive() the chain runs on accumulation / per-pixel count and total_samples is not used."""
         p = PostProcessParams(exposure, bloom_threshold, bloom_intensity, TONE_MAPPING_HDR if hdr else TONE_MAPPING_SDR)
         out = np.empty((self.height, self.width, 4), np.float32 if hdr else np.uint8)
         fmt = OUTPUT_RGBAF32 if hdr else OUTPUT_RGBA8_SRGB
         if denoised:
             self._check(self._L.pt_postprocess_denoised(self._h, C.addressof(p), fmt, out.ctypes.data, out.nbytes))
+            return out
+        if self.adaptive:
+            self._check(self._L.pt_postprocess_adaptive(self._h, C.addressof(p), fmt, out.ctypes.data, out.nbytes))
             return out
         n = self.total_samples if total_samples is None else total_samples
         self._check(self._L.pt_postprocess(self._h, C.addressof(p), int(n), fmt, out.ctypes.data, out.nbytes))
@@ -432,11 +488,15 @@ class Renderer:
                 sigma_normal: float = 128.0, sigma_depth: float = 1.0, total_samples: int | None = None) -> np.ndarray:
         """Edge-avoiding a-trous denoiser (DESIGN.md §3h) of accumulation / total_samples, guided by the first hit of the
         camera in params (default: the settings rendered with): (H, W, 4) float32 mean radiance, A = 1.  The result
-        stays on the device for postprocess(denoised=True) and the save_* writers; the accumulation is unchanged."""
+        stays on the device for postprocess(denoised=True) and the save_* writers; the accumulation is unchanged.  After
+        render_adaptive() the filter runs on accumulation / per-pixel count and total_samples is not used."""
         p = (params or self.params).to_c()
         d = DenoiseParams(int(iterations), sigma_luminance, sigma_normal, sigma_depth)
         n = self.total_samples if total_samples is None else total_samples
         out = np.empty((self.height, self.width, 4), np.float32)
+        if self.adaptive:
+            self._check(self._L.pt_denoise_adaptive(self._h, C.addressof(p), C.addressof(d), out.ctypes.data, out.nbytes))
+            return out
         self._check(self._L.pt_denoise(self._h, C.addressof(p), C.addressof(d), int(n), out.ctypes.data, out.nbytes))
         return out
 
@@ -514,6 +574,8 @@ class Renderer:
     def set_tuning(self, key: str, value: int):
         """Scheduling knobs (pools, slots, sort_hits, sbuf_mb); results do not depend on them."""
         self._check(self._L.pt_set_tuning(self._h, key.encode(), int(value)))
+        if key == "slots" and self.width:  # the target is re-created empty
+            self.adaptive = False
 
     def set_sampler(self, max_anisotropy: int):
         """Sampler state (Renderer.cpp:103-112): maximum anisotropy of the material fetches, 1 = isotropic (default) .. 16 (the reference's)."""

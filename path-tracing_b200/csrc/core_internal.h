@@ -93,6 +93,25 @@ struct EmitterTable
     float pEmitter;             // probability of the emitter branch of a light sample
 };
 
+// Adaptive sampling (DESIGN.md §3i): Welford statistics of the luminance of a pixel's samples, in sample order
+struct __align__(16) AdaptivePixel
+{
+    uint32_t count; // samples the pixel has
+    float mean, m2;
+    uint32_t pad;
+};
+
+// what k_adaptive_blocks / k_adaptive_select / k_adaptive_scatter report to the host after an evaluation
+struct AdaptiveSummary
+{
+    uint32_t n;            // smallest count among the active blocks (0xffffffff: none is active)
+    uint32_t next;         // next larger count among them (0xffffffff: none)
+    uint32_t pixels;       // A: pixels of the active blocks at count n = the pass's pixel list
+    uint32_t minCount, maxCount;
+    uint32_t unconverged;  // pixels of blocks at or above max_samples that miss the threshold
+    uint32_t pad[2];
+};
+
 // host copy of the tables instances are flattened from (kept for pt_scene_update)
 struct SceneTopology
 {
@@ -171,6 +190,19 @@ struct Context
     float4 *denoisePing = nullptr, *denoisePong = nullptr;
     float2 *denoiseGrad = nullptr;
     bool denoiseValid = false; // a pt_denoise result exists for the current accumulation
+    // what the accumulation holds since the last pt_render_begin: nothing, a uniform render (pt_render_samples /
+    // pt_render_frames) or an adaptive one (pt_render_adaptive); the two never mix, so per-pixel counts stay known
+    enum class TargetContent { Empty, Uniform, Adaptive } targetContent = TargetContent::Empty;
+    // adaptive sampling (adaptive.cu), one target allocation made at the first pt_render_adaptive: per pixel (count, mean
+    // luminance, M2), per 8x4 block three words and the scan's scratch, and the pass summary; the mean image accum / count
+    // at the first read
+    AdaptivePixel *adaptivePixels = nullptr;
+    uint32_t *adaptiveBlocks = nullptr;
+    uint32_t *adaptiveCounts = nullptr, *adaptiveOffsets = nullptr; // per block: pixels selected for the pass, their scan
+    void *adaptiveScanTemp = nullptr;
+    size_t adaptiveScanBytes = 0;
+    AdaptiveSummary *adaptiveSummary = nullptr;
+    float4 *adaptiveMean = nullptr;
     size_t slotPoolSize = (size_t)1 << 23;     // paths in flight, all pools together (PT_SLOTS)
     size_t sbufBudgetBytes = (size_t)8 << 30;  // sample-buffer budget (PT_SBUF_MB)
     uint32_t slotCapacity = 0; // size of the slot pool
@@ -271,6 +303,19 @@ pt_texture_desc defaultTexture(const uint32_t *rgba, bool srgb);
 pt_status allocSortTemp(Context *ctx, size_t slots);
 pt_status renderFrames(Context *ctx, const pt_render_params *params, uint32_t firstSample, uint32_t frameCount, uint32_t samplesPerFrame,
                         const pt_tile *tiles, uint32_t tileCount);
+// the pieces of renderFrames, in its order: the sample buffer for sampleCount samples of ctx->pixelCount pixels (roundMax =
+// samples per round), the counters and the start event, the rounds over ctx->pixelList (k_resolve, or k_resolve_adaptive when
+// `adaptive`), and the stop event, the timing and the stack check
+pt_status sizeSampleBuffer(Context *ctx, uint32_t sampleCount, uint32_t &roundMax);
+pt_status resetRenderStats(Context *ctx);
+pt_status renderRounds(Context *ctx, const pt_render_params *params, uint32_t firstSample, uint32_t sampleCount, uint32_t samplesPerFrame,
+                       uint32_t roundMax, bool adaptive);
+pt_status finishRender(Context *ctx, const char *what);
+
+// adaptive.cu
+pt_status renderAdaptive(Context *ctx, const pt_render_params *params, const pt_adaptive_params *ap, pt_adaptive_info *info);
+// accum / count into ctx->adaptiveMean (allocated here), queued on ctx->stream
+pt_status adaptiveMeanImage(Context *ctx, const char *what);
 pt_status firstHitAov(Context *ctx, const pt_render_params *params, uint32_t width, uint32_t height, pt_hit *out);
 pt_status debugRender(Context *ctx, const pt_render_params *params, const pt_debug_params *debug, uint32_t width, uint32_t height,
                       float *out);
@@ -280,11 +325,17 @@ pt_status traceOcclusion(Context *ctx, const pt_ray *rays, uint64_t n, uint8_t *
 void launchDenoiseGuides(Context *ctx, const pt_render_params *params, float4 *albedoT, float4 *normal);
 
 // denoise.cu
-pt_status denoise(Context *ctx, const pt_render_params *params, const pt_denoise_params *dn, uint32_t totalSamples, float *out,
-                  size_t outBytes);
+// src / divisor as in postProcess; src is read after the argument checks, so ctx->accum may still be NULL there.
+// checkDenoise / checkPostProcess are those argument checks alone (no device work), run first by both functions
+pt_status checkDenoise(Context *ctx, const char *what, const pt_render_params *params, const pt_denoise_params *dn, float divisor,
+                       const float *out, size_t outBytes);
+pt_status denoise(Context *ctx, const char *what, const pt_render_params *params, const pt_denoise_params *dn, const float4 *src,
+                  float divisor, float *out, size_t outBytes);
 
 // postprocess.cu
 // src / divisor is the image the chain starts from: the accumulation and its sample count, or the denoised mean and 1
+pt_status checkPostProcess(Context *ctx, const char *what, const pt_postprocess_params *params, uint32_t outputFormat, const void *out,
+                           size_t outBytes);
 pt_status postProcess(Context *ctx, const char *what, const pt_postprocess_params *params, const float4 *src, float divisor,
                       uint32_t outputFormat, void *out, size_t outBytes);
 

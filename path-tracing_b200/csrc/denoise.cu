@@ -178,29 +178,37 @@ __global__ void __launch_bounds__(256) k_atrous(const float4 *__restrict__ src, 
 
 } // namespace
 
-pt_status denoise(Context *ctx, const pt_render_params *params, const pt_denoise_params *dn, uint32_t totalSamples, float *out,
-                  size_t outBytes)
+pt_status checkDenoise(Context *ctx, const char *what, const pt_render_params *params, const pt_denoise_params *dn, float divisor,
+                       const float *out, size_t outBytes)
 {
     if (!params || !dn)
-        return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_denoise", "NULL argument");
+        return fail(ctx, PT_ERR_INVALID_ARGUMENT, what, "NULL argument");
     if (!ctx->hasScene)
-        return fail(ctx, PT_ERR_NO_SCENE, "pt_denoise", "no scene uploaded");
+        return fail(ctx, PT_ERR_NO_SCENE, what, "no scene uploaded");
     if (!ctx->accum)
-        return fail(ctx, PT_ERR_NO_TARGET, "pt_denoise", "pt_render_begin has not been called");
+        return fail(ctx, PT_ERR_NO_TARGET, what, "pt_render_begin has not been called");
     if (params->lens_radius > 0.0f)
-        return fail(ctx, PT_ERR_UNSUPPORTED, "pt_denoise", "lens_radius > 0: pinhole guides cannot describe a defocused image");
-    if (totalSamples == 0)
-        return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_denoise", "total_samples must be at least 1");
+        return fail(ctx, PT_ERR_UNSUPPORTED, what, "lens_radius > 0: pinhole guides cannot describe a defocused image");
+    if (divisor == 0.0f)
+        return fail(ctx, PT_ERR_INVALID_ARGUMENT, what, "total_samples must be at least 1");
     if (dn->iterations > 8)
-        return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_denoise", "iterations must be in 0..8");
+        return fail(ctx, PT_ERR_INVALID_ARGUMENT, what, "iterations must be in 0..8");
     for (const float s : { dn->sigma_luminance, dn->sigma_normal, dn->sigma_depth })
         if (!std::isfinite(s) || s < 0.0f)
-            return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_denoise", "sigmas must be finite and non-negative");
+            return fail(ctx, PT_ERR_INVALID_ARGUMENT, what, "sigmas must be finite and non-negative");
+    if (out && outBytes < (size_t)ctx->width * ctx->height * sizeof(float4))
+        return fail(ctx, PT_ERR_INVALID_ARGUMENT, what, "output buffer too small");
+    return PT_OK;
+}
+
+pt_status denoise(Context *ctx, const char *what, const pt_render_params *params, const pt_denoise_params *dn, const float4 *src,
+                  float divisor, float *out, size_t outBytes)
+{
+    const pt_status checked = checkDenoise(ctx, what, params, dn, divisor, out, outBytes);
+    if (checked != PT_OK)
+        return checked;
     const uint32_t W = ctx->width, H = ctx->height;
     const size_t n = (size_t)W * H;
-    if (out && outBytes < n * sizeof(float4))
-        return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_denoise", "output buffer too small");
-
     if (!ctx->denoised)
     {
         // belongs to the target: freeTarget releases it with the accumulation
@@ -220,7 +228,7 @@ pt_status denoise(Context *ctx, const pt_render_params *params, const pt_denoise
     cudaStream_t st = ctx->stream;
     launchDenoiseGuides(ctx, params, ctx->denoiseAlbedoT, ctx->denoiseNormal);
     const dim3 block(32, 8), grid((W + 31) / 32, (H + 7) / 8);
-    k_denoise_prepare<<<grid, block, 0, st>>>(ctx->accum, (float)totalSamples, ctx->denoiseAlbedoT, ctx->denoiseNormal, W, H,
+    k_denoise_prepare<<<grid, block, 0, st>>>(src, divisor, ctx->denoiseAlbedoT, ctx->denoiseNormal, W, H,
                                               ctx->denoiseNT, ctx->denoisePing, ctx->denoiseGrad, ctx->denoised);
     const uint32_t K = dn->iterations;
     if (K > 0)
@@ -243,7 +251,7 @@ pt_status denoise(Context *ctx, const pt_render_params *params, const pt_denoise
         err = cudaStreamSynchronize(st);
     PT_CUDA_CHECK(ctx, err);
     ctx->stats.kernel_launches = 2 + (K > 0 ? 1 + K : 0);
-    const pt_status s = checkStackOverflow(ctx, "pt_denoise");
+    const pt_status s = checkStackOverflow(ctx, what);
     if (s == PT_OK)
         ctx->denoiseValid = true;
     return s;

@@ -164,8 +164,8 @@ __global__ void __launch_bounds__(256) k_post_output(const uint2 *__restrict__ c
 
 } // namespace
 
-pt_status postProcess(Context *ctx, const char *what, const pt_postprocess_params *p, const float4 *src, float divisor,
-                      uint32_t outputFormat, void *out, size_t outBytes)
+pt_status checkPostProcess(Context *ctx, const char *what, const pt_postprocess_params *p, uint32_t outputFormat, const void *out,
+                           size_t outBytes)
 {
     if (!p || !out)
         return fail(ctx, PT_ERR_INVALID_ARGUMENT, what, "NULL argument");
@@ -175,10 +175,20 @@ pt_status postProcess(Context *ctx, const char *what, const pt_postprocess_param
         return fail(ctx, PT_ERR_INVALID_ARGUMENT, what, "unknown output format");
     if (p->tone_mapping > PT_TONE_MAPPING_HDR)
         return fail(ctx, PT_ERR_INVALID_ARGUMENT, what, "unknown tone-mapping mode");
-    const uint32_t W = ctx->width, H = ctx->height;
-    const size_t n = (size_t)W * H, need = n * (outputFormat == PT_OUTPUT_RGBA8_SRGB ? 4 : 16);
+    const size_t need = (size_t)ctx->width * ctx->height * (outputFormat == PT_OUTPUT_RGBA8_SRGB ? 4 : 16);
     if (outBytes < need)
         return fail(ctx, PT_ERR_INVALID_ARGUMENT, what, "output buffer too small");
+    return PT_OK;
+}
+
+pt_status postProcess(Context *ctx, const char *what, const pt_postprocess_params *p, const float4 *src, float divisor,
+                      uint32_t outputFormat, void *out, size_t outBytes)
+{
+    const pt_status checked = checkPostProcess(ctx, what, p, outputFormat, out, outBytes);
+    if (checked != PT_OK)
+        return checked;
+    const uint32_t W = ctx->width, H = ctx->height;
+    const size_t n = (size_t)W * H, need = n * (outputFormat == PT_OUTPUT_RGBA8_SRGB ? 4 : 16);
 
     // floor(log2(max(w, h))) + 1 levels (PT/Renderer/Image.cpp:14-17)
     uint32_t levels = 1;

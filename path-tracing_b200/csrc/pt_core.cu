@@ -32,6 +32,14 @@ static void freeTarget(Context *ctx)
     ctx->denoisePing = ctx->denoisePong = nullptr;
     ctx->denoiseGrad = nullptr;
     ctx->denoiseValid = false;
+    ctx->targetContent = Context::TargetContent::Empty;
+    ctx->adaptivePixels = nullptr;
+    ctx->adaptiveBlocks = nullptr;
+    ctx->adaptiveCounts = ctx->adaptiveOffsets = nullptr;
+    ctx->adaptiveScanTemp = nullptr;
+    ctx->adaptiveScanBytes = 0;
+    ctx->adaptiveSummary = nullptr;
+    ctx->adaptiveMean = nullptr;
     ctx->ps = PathState {};
     ctx->slotCapacity = 0;
     ctx->pixelList = nullptr;
@@ -267,6 +275,7 @@ pt_status pt_render_begin(pt_context *ctx, uint32_t width, uint32_t height)
     }
     PT_CUDA_CHECK(ctx, cudaMemsetAsync(ctx->accum, 0, n * sizeof(float4), ctx->stream));
     ctx->denoiseValid = false;
+    ctx->targetContent = Context::TargetContent::Empty;
     return PT_OK;
 }
 
@@ -341,7 +350,7 @@ pt_status pt_denoise(pt_context *ctx, const pt_render_params *params, const pt_d
     if (!ctx)
         return PT_ERR_INVALID_ARGUMENT;
     DeviceGuard guard(ctx->device);
-    return denoise(ctx, params, denoise_params, total_samples, out_rgba, out_bytes);
+    return denoise(ctx, "pt_denoise", params, denoise_params, ctx->accum, (float)total_samples, out_rgba, out_bytes);
 }
 
 pt_status pt_denoise_guides(pt_context *ctx, float *out_albedo_t, float *out_normal, size_t out_bytes)
@@ -375,6 +384,87 @@ pt_status pt_postprocess_denoised(pt_context *ctx, const pt_postprocess_params *
         return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_postprocess_denoised", "no pt_denoise since the last pt_render_begin");
     DeviceGuard guard(ctx->device);
     return postProcess(ctx, "pt_postprocess_denoised", params, ctx->denoised, 1.0f, output_format, out_pixels, out_bytes);
+}
+
+pt_status pt_render_adaptive(pt_context *ctx, const pt_render_params *params, const pt_adaptive_params *adaptive,
+                             pt_adaptive_info *out_info)
+{
+    if (!ctx)
+        return PT_ERR_INVALID_ARGUMENT;
+    DeviceGuard guard(ctx->device);
+    return renderAdaptive(ctx, params, adaptive, out_info);
+}
+
+// the target must hold an adaptive render for the adaptive read functions
+static pt_status checkAdaptiveTarget(Context *ctx, const char *what)
+{
+    if (!ctx->accum)
+        return fail(ctx, PT_ERR_NO_TARGET, what, "pt_render_begin has not been called");
+    if (ctx->targetContent != Context::TargetContent::Adaptive)
+        return fail(ctx, PT_ERR_INVALID_ARGUMENT, what, "no pt_render_adaptive since the last pt_render_begin");
+    return PT_OK;
+}
+
+pt_status pt_adaptive_readback(pt_context *ctx, uint32_t *out_counts, float *out_mean_m2, size_t pixels)
+{
+    if (!ctx)
+        return PT_ERR_INVALID_ARGUMENT;
+    const pt_status s = checkAdaptiveTarget(ctx, "pt_adaptive_readback");
+    if (s != PT_OK)
+        return s;
+    const size_t n = (size_t)ctx->width * ctx->height;
+    if (pixels < n)
+        return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_adaptive_readback", "output buffer too small");
+    DeviceGuard guard(ctx->device);
+    const AdaptivePixel *px = ctx->adaptivePixels;
+    if (out_counts)
+        PT_CUDA_CHECK(ctx, cudaMemcpy2DAsync(out_counts, sizeof(uint32_t), &px->count, sizeof(AdaptivePixel), sizeof(uint32_t), n,
+                                             cudaMemcpyDeviceToHost, ctx->stream));
+    if (out_mean_m2)
+        PT_CUDA_CHECK(ctx, cudaMemcpy2DAsync(out_mean_m2, 2 * sizeof(float), &px->mean, sizeof(AdaptivePixel), 2 * sizeof(float), n,
+                                             cudaMemcpyDeviceToHost, ctx->stream));
+    PT_CUDA_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
+    return PT_OK;
+}
+
+pt_status pt_postprocess_adaptive(pt_context *ctx, const pt_postprocess_params *params, uint32_t output_format, void *out_pixels,
+                                  size_t out_bytes)
+{
+    if (!ctx)
+        return PT_ERR_INVALID_ARGUMENT;
+    const char *what = "pt_postprocess_adaptive";
+    pt_status s = checkPostProcess(ctx, what, params, output_format, out_pixels, out_bytes);
+    if (s == PT_OK)
+        s = checkAdaptiveTarget(ctx, what);
+    if (s != PT_OK)
+        return s;
+    DeviceGuard guard(ctx->device);
+    s = adaptiveMeanImage(ctx, what);
+    if (s == PT_OK)
+        s = postProcess(ctx, what, params, ctx->adaptiveMean, 1.0f, output_format, out_pixels, out_bytes);
+    if (s == PT_OK)
+        ctx->stats.kernel_launches++; // k_adaptive_mean
+    return s;
+}
+
+pt_status pt_denoise_adaptive(pt_context *ctx, const pt_render_params *params, const pt_denoise_params *denoise_params,
+                              float *out_rgba, size_t out_bytes)
+{
+    if (!ctx)
+        return PT_ERR_INVALID_ARGUMENT;
+    const char *what = "pt_denoise_adaptive";
+    pt_status s = checkDenoise(ctx, what, params, denoise_params, 1.0f, out_rgba, out_bytes);
+    if (s == PT_OK)
+        s = checkAdaptiveTarget(ctx, what);
+    if (s != PT_OK)
+        return s;
+    DeviceGuard guard(ctx->device);
+    s = adaptiveMeanImage(ctx, what);
+    if (s == PT_OK)
+        s = denoise(ctx, what, params, denoise_params, ctx->adaptiveMean, 1.0f, out_rgba, out_bytes);
+    if (s == PT_OK)
+        ctx->stats.kernel_launches++; // k_adaptive_mean
+    return s;
 }
 
 pt_status pt_synchronize(pt_context *ctx)

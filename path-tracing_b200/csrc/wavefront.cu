@@ -913,6 +913,34 @@ __global__ void __launch_bounds__(256) k_resolve(RenderConst rc)
     }
 }
 
+// k_resolve's additions (same order, same expressions) plus the Welford update of the pixel's luminance statistics per
+// sample (DESIGN.md §3i); a dropped frame (parked as 0) is a sample of luminance 0, as in the accumulation
+__global__ void __launch_bounds__(256) k_resolve_adaptive(RenderConst rc, AdaptivePixel *state)
+{
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t pi = blockIdx.x * blockDim.x + threadIdx.x; pi < rc.pixelCount; pi += stride)
+    {
+        const uint32_t pixel = __ldg(rc.pixelList + pi);
+        float4 a = rc.accum[pixel];
+        AdaptivePixel st = state[pixel];
+        for (uint32_t s = 0; s < rc.roundSamples; s++)
+        {
+            const float4 r = __ldcs(rc.sbuf + (size_t)s * rc.pixelCount + pi);
+            a.x = r.x + a.x;
+            a.y = r.y + a.y;
+            a.z = r.z + a.z;
+            const float l = (0.2126f * r.x + 0.7152f * r.y) + 0.0722f * r.z;
+            st.count += 1;
+            const float d = l - st.mean;
+            st.mean += d / (float)st.count;
+            st.m2 += d * (l - st.mean);
+        }
+        a.w = 1.0f;
+        rc.accum[pixel] = a;
+        state[pixel] = st;
+    }
+}
+
 // ---------------------------------------------------------------------------------------------
 // standalone queries
 // ---------------------------------------------------------------------------------------------
@@ -1260,6 +1288,59 @@ pt_status allocSortTemp(Context *ctx, size_t slots)
     return PT_OK;
 }
 
+// ---- pixel list of the tile set: 8x4 pixel blocks, so that consecutive work items are
+//      neighbouring pixels and a warp's fresh primary rays are coherent -----------------------
+static pt_status buildPixelList(Context *ctx, const pt_tile *tiles, uint32_t tileCount)
+{
+    const uint32_t W = ctx->width, H = ctx->height;
+    const pt_tile whole = { 0, 0, W, H };
+    std::vector<pt_tile> want(tileCount ? tiles : &whole, tileCount ? tiles + tileCount : &whole + 1);
+    const bool same = ctx->pixelListValid && want.size() == ctx->pixelTiles.size() &&
+                      (want.empty() || std::memcmp(want.data(), ctx->pixelTiles.data(), want.size() * sizeof(pt_tile)) == 0);
+    if (!same)
+    {
+        // the tiles must be disjoint: a pixel listed twice would be sampled twice and k_resolve would race on it.
+        // The total area is checked BEFORE any pixel is listed (many large tiles cannot exhaust host memory),
+        // overlap with one bit per pixel while listing.
+        uint64_t area = 0;
+        for (const pt_tile &in : want)
+        {
+            const pt_tile t = { std::min(in.x0, W), std::min(in.y0, H), std::min(in.x1, W), std::min(in.y1, H) };
+            if (t.x1 > t.x0 && t.y1 > t.y0)
+                area += (uint64_t)(t.x1 - t.x0) * (t.y1 - t.y0);
+            if (area > (uint64_t)W * H)
+                return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_render_samples", "tiles overlap (their area exceeds the frame)");
+        }
+        std::vector<uint32_t> list;
+        list.reserve((size_t)area);
+        std::vector<bool> covered((size_t)W * H, false);
+        for (const pt_tile &in : want)
+        {
+            const pt_tile t = { std::min(in.x0, W), std::min(in.y0, H), std::min(in.x1, W), std::min(in.y1, H) };
+            for (uint32_t y = t.y0; y < t.y1; y++)
+                for (uint32_t x = t.x0; x < t.x1; x++)
+                {
+                    if (covered[(size_t)y * W + x])
+                        return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_render_samples", "tiles overlap");
+                    covered[(size_t)y * W + x] = true;
+                }
+            for (uint32_t by = t.y0; by < t.y1; by += 4)
+                for (uint32_t bx = t.x0; bx < t.x1; bx += 8)
+                    for (uint32_t y = by; y < std::min(by + 4, t.y1); y++)
+                        for (uint32_t x = bx; x < std::min(bx + 8, t.x1); x++)
+                            list.push_back(y * W + x);
+        }
+        if (!list.empty())
+            PT_CUDA_CHECK(ctx, cudaMemcpyAsync(ctx->pixelList, list.data(), list.size() * 4, cudaMemcpyHostToDevice,
+                                               ctx->stream));
+        PT_CUDA_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
+        ctx->pixelTiles = want;
+        ctx->pixelCount = (uint32_t)list.size();
+        ctx->pixelListValid = true;
+    }
+    return PT_OK;
+}
+
 pt_status renderFrames(Context *ctx, const pt_render_params *params, uint32_t firstSample, uint32_t sampleCount, uint32_t samplesPerFrame,
                         const pt_tile *tiles, uint32_t tileCount)
 {
@@ -1273,6 +1354,9 @@ pt_status renderFrames(Context *ctx, const pt_render_params *params, uint32_t fi
         return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_render_samples", "bounce_count must be in 1..255");
     if (samplesPerFrame == 0 || samplesPerFrame > kMaxSamplesPerFrame)
         return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_render_frames", "samples_per_frame must be in 1..8192");
+    if (ctx->targetContent == Context::TargetContent::Adaptive)
+        return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_render_samples",
+                    "the target holds an adaptive render (per-pixel sample counts); call pt_render_begin first");
     if (tiles == nullptr)
         tileCount = 0;
     if (ctx->lightSampling == PT_LIGHT_SAMPLING_EMISSIVE_MIS && !ctx->emittersValid)
@@ -1282,60 +1366,25 @@ pt_status renderFrames(Context *ctx, const pt_render_params *params, uint32_t fi
             return st;
     }
 
-    // ---- pixel list of the tile set: 8x4 pixel blocks, so that consecutive work items are
-    //      neighbouring pixels and a warp's fresh primary rays are coherent -----------------------
-    const uint32_t W = ctx->width, H = ctx->height;
-    {
-        const pt_tile whole = { 0, 0, W, H };
-        std::vector<pt_tile> want(tileCount ? tiles : &whole, tileCount ? tiles + tileCount : &whole + 1);
-        const bool same = ctx->pixelListValid && want.size() == ctx->pixelTiles.size() &&
-                          (want.empty() || std::memcmp(want.data(), ctx->pixelTiles.data(), want.size() * sizeof(pt_tile)) == 0);
-        if (!same)
-        {
-            // the tiles must be disjoint: a pixel listed twice would be sampled twice and k_resolve would race on it.
-            // The total area is checked BEFORE any pixel is listed (many large tiles cannot exhaust host memory),
-            // overlap with one bit per pixel while listing.
-            uint64_t area = 0;
-            for (const pt_tile &in : want)
-            {
-                const pt_tile t = { std::min(in.x0, W), std::min(in.y0, H), std::min(in.x1, W), std::min(in.y1, H) };
-                if (t.x1 > t.x0 && t.y1 > t.y0)
-                    area += (uint64_t)(t.x1 - t.x0) * (t.y1 - t.y0);
-                if (area > (uint64_t)W * H)
-                    return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_render_samples", "tiles overlap (their area exceeds the frame)");
-            }
-            std::vector<uint32_t> list;
-            list.reserve((size_t)area);
-            std::vector<bool> covered((size_t)W * H, false);
-            for (const pt_tile &in : want)
-            {
-                const pt_tile t = { std::min(in.x0, W), std::min(in.y0, H), std::min(in.x1, W), std::min(in.y1, H) };
-                for (uint32_t y = t.y0; y < t.y1; y++)
-                    for (uint32_t x = t.x0; x < t.x1; x++)
-                    {
-                        if (covered[(size_t)y * W + x])
-                            return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_render_samples", "tiles overlap");
-                        covered[(size_t)y * W + x] = true;
-                    }
-                for (uint32_t by = t.y0; by < t.y1; by += 4)
-                    for (uint32_t bx = t.x0; bx < t.x1; bx += 8)
-                        for (uint32_t y = by; y < std::min(by + 4, t.y1); y++)
-                            for (uint32_t x = bx; x < std::min(bx + 8, t.x1); x++)
-                                list.push_back(y * W + x);
-            }
-            if (!list.empty())
-                PT_CUDA_CHECK(ctx, cudaMemcpyAsync(ctx->pixelList, list.data(), list.size() * 4, cudaMemcpyHostToDevice,
-                                                   ctx->stream));
-            PT_CUDA_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
-            ctx->pixelTiles = want;
-            ctx->pixelCount = (uint32_t)list.size();
-            ctx->pixelListValid = true;
-        }
-    }
-    const uint32_t pixels = ctx->pixelCount;
-
-    // ---- rounds: as many samples per round as the sample buffer budget allows ---------------------
+    const pt_status listed = buildPixelList(ctx, tiles, tileCount);
+    if (listed != PT_OK)
+        return listed;
+    if (sampleCount > 0)
+        ctx->targetContent = Context::TargetContent::Uniform;
     uint32_t roundMax = 0;
+    pt_status st = sizeSampleBuffer(ctx, sampleCount, roundMax);
+    if (st == PT_OK)
+        st = resetRenderStats(ctx);
+    if (st == PT_OK)
+        st = renderRounds(ctx, params, firstSample, sampleCount, samplesPerFrame, roundMax, false);
+    return st == PT_OK ? finishRender(ctx, "pt_render_samples") : st;
+}
+
+pt_status sizeSampleBuffer(Context *ctx, uint32_t sampleCount, uint32_t &roundMax)
+{
+    const uint32_t pixels = ctx->pixelCount;
+    // ---- rounds: as many samples per round as the sample buffer budget allows ---------------------
+    roundMax = 0;
     if (pixels > 0 && sampleCount > 0)
     {
         size_t freeB = 0, totalB = 0;
@@ -1356,7 +1405,11 @@ pt_status renderFrames(Context *ctx, const pt_render_params *params, uint32_t fi
             ctx->sbufCapacity = need;
         }
     }
+    return PT_OK;
+}
 
+pt_status resetRenderStats(Context *ctx)
+{
     ctx->stats.kernel_launches = 0;
     ctx->stats.wavefront_iterations = 0;
     for (int k = 0; k < PT_KERNEL_CLASS_COUNT; k++)
@@ -1366,6 +1419,14 @@ pt_status renderFrames(Context *ctx, const pt_render_params *params, uint32_t fi
     }
     PT_CUDA_CHECK(ctx, cudaMemsetAsync(ctx->dCounters, 0, sizeof(DeviceCounters), ctx->stream));
     PT_CUDA_CHECK(ctx, cudaEventRecord(ctx->evStart, ctx->stream));
+    return PT_OK;
+}
+
+pt_status renderRounds(Context *ctx, const pt_render_params *params, uint32_t firstSample, uint32_t sampleCount, uint32_t samplesPerFrame,
+                       uint32_t roundMax, bool adaptive)
+{
+    const uint32_t W = ctx->width, H = ctx->height;
+    const uint32_t pixels = ctx->pixelCount;
 
     // optional per-launch CUDA-event timing (pt_set_kernel_timing): (class, start, stop) triples
     struct Timed
@@ -1615,7 +1676,11 @@ pt_status renderFrames(Context *ctx, const pt_render_params *params, uint32_t fi
         }
         // every pool has been synchronised with the host: the round's samples are all parked
         begin(PT_KERNEL_FINISH, ctx->stream);
-        k_resolve<<<std::min((pixels + 255) / 256, (uint32_t)ctx->smCount * 8), 256, 0, ctx->stream>>>(base);
+        const uint32_t resolveGrid = std::min((pixels + 255) / 256, (uint32_t)ctx->smCount * 8);
+        if (adaptive)
+            k_resolve_adaptive<<<resolveGrid, 256, 0, ctx->stream>>>(base, ctx->adaptivePixels);
+        else
+            k_resolve<<<resolveGrid, 256, 0, ctx->stream>>>(base);
         end(ctx->stream);
         ctx->stats.kernel_launches++;
     }
@@ -1629,12 +1694,18 @@ pt_status renderFrames(Context *ctx, const pt_render_params *params, uint32_t fi
             ctx->stats.kernel_ms[t.cls] += ms;
         }
     }
+    // what is still queued runs on ctx->stream only: every pool has been synchronised with the host
+    finished = true;
+    return PT_OK;
+}
+
+pt_status finishRender(Context *ctx, const char *what)
+{
     PT_CUDA_CHECK(ctx, cudaEventRecord(ctx->evStop, ctx->stream));
     PT_CUDA_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
     PT_CUDA_CHECK(ctx, cudaGetLastError());
     PT_CUDA_CHECK(ctx, cudaEventElapsedTime(&ctx->stats.last_render_ms, ctx->evStart, ctx->evStop));
-    finished = true;
-    return checkStackOverflow(ctx, "pt_render_samples");
+    return checkStackOverflow(ctx, what);
 }
 
 pt_status checkStackOverflow(Context *ctx, const char *what)
