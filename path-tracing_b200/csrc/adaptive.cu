@@ -1,7 +1,7 @@
 // adaptive.cu — adaptive sampling: converged 8x4 pixel blocks stop early (DESIGN.md §3i).
 //
 // Per pixel the target keeps (count, mean, M2), Welford statistics of the luminance of its samples, which
-// k_resolve_adaptive (wavefront.cu) updates in sample order while it accumulates.  A pass:
+// k_resolve<true> (wavefront.cu) updates in sample order while it accumulates.  A pass:
 //   k_adaptive_blocks   the stop rule per 8x4 block; the smallest count n among the active blocks
 //   k_adaptive_select   per block its pixel count if it is active at count n, and the next larger count among the active
 //   + exclusive scan    blocks; a device-wide scan of those counts places each block's pixels in ascending block order

@@ -63,7 +63,7 @@ struct __align__(128) PathRecord
     float4 shC;   // contribution.xyz (throughput * DirectLight / pdf), -
     float4 decal; // rgb, dist (scenes with alpha-tested geometry)
     float decalA;
-    uint32_t pad[3]; // pad[0]: bsdf.Pdf of the previous bounce (k_shade_emissive, emissive-MIS light sampling)
+    uint32_t pad[3]; // pad[0]: bsdf.Pdf of the previous bounce (k_shade<A, S, true>, emissive-MIS light sampling)
     float4 spare[3];
 };
 static_assert(sizeof(PathRecord) == 256, "PathRecord must be two 128-byte lines");
@@ -304,8 +304,8 @@ pt_status allocSortTemp(Context *ctx, size_t slots);
 pt_status renderFrames(Context *ctx, const pt_render_params *params, uint32_t firstSample, uint32_t frameCount, uint32_t samplesPerFrame,
                         const pt_tile *tiles, uint32_t tileCount);
 // the pieces of renderFrames, in its order: the sample buffer for sampleCount samples of ctx->pixelCount pixels (roundMax =
-// samples per round), the counters and the start event, the rounds over ctx->pixelList (k_resolve, or k_resolve_adaptive when
-// `adaptive`), and the stop event, the timing and the stack check
+// samples per round), the counters and the start event, the rounds over ctx->pixelList (k_resolve<adaptive>, which with
+// `adaptive` also updates the pixels' statistics), and the stop event, the timing and the stack check
 pt_status sizeSampleBuffer(Context *ctx, uint32_t sampleCount, uint32_t &roundMax);
 pt_status resetRenderStats(Context *ctx);
 pt_status renderRounds(Context *ctx, const pt_render_params *params, uint32_t firstSample, uint32_t sampleCount, uint32_t samplesPerFrame,

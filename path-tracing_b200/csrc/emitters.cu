@@ -3,7 +3,7 @@
 // k_emitters finds the emissive triangles and their power, area x luminance of the emission averaged over the triangle;
 // the host quantises the powers to integer weights and builds a Walker / Vose alias table from them with integer
 // arithmetic in a fixed order, so the table is exact and the same on every GPU and in the CPU reference
-// (tests/emissive_oracle.cpp buildEmitterTable, same definitions); k_emitter_records gathers the 64-byte records k_shade_emissive samples points from.
+// (tests/emissive_oracle.cpp buildEmitterTable, same definitions); k_emitter_records gathers the 64-byte records k_shade<A, S, true> samples points from.
 // Built at the first render in the mode after an upload, an update that moves geometry, a texture upload or a sampler change.
 #include "core_internal.h"
 #include "shading.cuh"

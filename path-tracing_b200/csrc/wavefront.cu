@@ -414,205 +414,14 @@ __device__ __forceinline__ LightSample sampleEmitter(const DeviceScene &s, const
 }
 
 // ---------------------------------------------------------------------------------------------
-// shade: closestHit.rchit, then the raygen bounce logic (misses are finished by k_extend)
+// shade: closestHit.rchit, then the raygen bounce logic (misses are finished by k_extend).
+// EMISSIVE adds emissive-triangle light sampling and MIS (pt_set_light_sampling, DESIGN.md §3g) to the same closest-hit
+// and bounce logic and the same main rng stream: the emitter branch of the light sample, the MIS weight of emission found
+// by BSDF sampling and the previous bounce's BSDF pdf in the path record; em is read only when EMISSIVE.  The body stays
+// in the kernel: moving it into a force-inlined __device__ function changed the machine code of both modes.
 // ---------------------------------------------------------------------------------------------
-template <bool ALPHA, bool STATS> __global__ void __launch_bounds__(128, PT_SHADE_MIN_BLOCKS) k_shade(RenderConst rc, int cur)
-{
-    const uint32_t n = rc.qc->hit;
-    const uint32_t stride = gridDim.x * blockDim.x;
-    const DeviceScene &s = rc.scene;
-    uint32_t texels = 0;
-    // the queue positions of k_extend, which has completed (stream order)
-    if (blockIdx.x == 0 && threadIdx.x == 0)
-        rc.qc->extendWork = 0;
-    const uint32_t *hitQueue = rc.sortHits ? rc.ps.hitQSorted : rc.ps.hitQ;
-    // (requesting the next hit's path record into L2 one loop iteration ahead was measured: no gain,
-    // the kernel is bound by issue latency at 16 warps per SM, not by the record's DRAM latency)
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
-    {
-        const uint32_t slot = hitQueue[i];
-        const float4 hitv = rc.ps.rec[slot].hit;
-        const float4 rayO = rc.ps.rec[slot].rayO, rayD = rc.ps.rec[slot].rayD;
-        // read with the rest of the record: reading throughput, radiance and the differentials again where they are
-        // used exposed the loads' latency at the end of every hit (measured: k_shade +12 %, chess)
-        float4 thr4 = rc.ps.rec[slot].thr;
-        float4 rad4 = rc.ps.rec[slot].rad;
-        vec3 throughput = V3(thr4), radiance = V3(rad4);
-        uint32_t state = __float_as_uint(thr4.w);
-        const vec3 rayDir = V3(rayD);
-        const uint32_t tri = __float_as_uint(hitv.x);
-
-        uint32_t rng = __float_as_uint(rayD.w);
-        float maxRoughness = rayO.w;
-        const float rayTmax = hitv.y;
-        const vec3 bary = V3(1.0f - hitv.z - hitv.w, hitv.z, hitv.w);
-
-        // ---- closestHit.rchit:54-83 with baked world-space data ---------------------------------
-        const float4 q0 = __ldg(s.triPos + 3 * (size_t)tri), q1 = __ldg(s.triPos + 3 * (size_t)tri + 1);
-        const float4 q2 = __ldg(s.triPos + 3 * (size_t)tri + 2);
-        const TriShade &ts = s.triShade[__float_as_uint(q0.w)];
-        const float4 a0 = __ldg(&ts.a[0]), a1 = __ldg(&ts.a[1]), a2 = __ldg(&ts.a[2]), a3 = __ldg(&ts.a[3]);
-        const float4 a4 = __ldg(&ts.a[4]), a5 = __ldg(&ts.a[5]), a6 = __ldg(&ts.a[6]), a7 = __ldg(&ts.a[7]);
-        const float4 a8 = __ldg(&ts.a[8]);
-        const uint32_t materialId = __float_as_uint(q2.w);
-        const vec3 p0 = V3(q0), p1 = V3(q1), p2 = V3(q2);
-        const vec3 n0r = V3(a0.x, a0.y, a0.z), n1r = V3(a0.w, a1.x, a1.y), n2r = V3(a1.z, a1.w, a2.x);
-        const vec3 t0r = V3(a2.y, a2.z, a2.w), t1r = V3(a3.x, a3.y, a3.z), t2r = V3(a3.w, a4.x, a4.y);
-        const vec3 b0r = V3(a4.z, a4.w, a5.x), b1r = V3(a5.y, a5.z, a5.w), b2r = V3(a6.x, a6.y, a6.z);
-        const vec2 uv0 = V2(a6.w, a7.x), uv1 = V2(a7.y, a7.z), uv2 = V2(a7.w, a8.x);
-
-        const vec3 position = p0 * bary.x + p1 * bary.y + p2 * bary.z;
-        const vec2 texCoords = uv0 * bary.x + uv1 * bary.y + uv2 * bary.z;
-        vec3 normal = normalize(n0r * bary.x + n1r * bary.y + n2r * bary.z);
-        vec3 tangent = normalize(t0r * bary.x + t1r * bary.y + t2r * bary.z);
-        vec3 bitangent = normalize(b0r * bary.x + b1r * bary.y + b2r * bary.z);
-        const vec3 edge1 = p1 - p0, edge2 = p2 - p0;
-        // normalised once per triangle by k_bake (same functions, same operands)
-        const float4 a9 = __ldg(&ts.a[9]), a10 = __ldg(&ts.a[10]), a11 = __ldg(&ts.a[11]);
-        const vec3 n0 = V3(a9.x, a9.y, a9.z), n1 = V3(a9.w, a10.x, a10.y), n2 = V3(a10.z, a10.w, a11.x);
-        vec3 geometricNormal = V3(a11.y, a11.z, a11.w);
-        const bool inside = dot(geometricNormal, rayDir) > 0.0f;
-        if (inside)
-        {
-            geometricNormal = -geometricNormal;
-            normal = -normal;
-            tangent = -tangent;
-            bitangent = -bitangent;
-        }
-
-        // ---- tracing.glsl:2-28 -------------------------------------------------------------
-        vec3 dpdu, dpdv, dndu, dndv;
-        computeDpnDuv(edge1, edge2, n1 - n0, n2 - n0, uv1 - uv0, uv2 - uv0, tangent, bitangent, dpdu, dpdv, dndu, dndv);
-        const float4 d0 = rc.ps.rec[slot].diff0, d1 = rc.ps.rec[slot].diff1, d2 = rc.ps.rec[slot].diff2;
-        RayDifferentials rd;
-        rd.rxOrigin = V3(d0.x, d0.y, d0.z);
-        rd.rxDirection = V3(d0.w, d1.x, d1.y);
-        rd.ryOrigin = V3(d1.z, d1.w, d2.x);
-        rd.ryDirection = V3(d2.y, d2.z, d2.w);
-        vec3 dpdx, dpdy;
-        computeDpDxy(position, rd.rxOrigin, rd.rxDirection, rd.ryOrigin, rd.ryDirection, normal, dpdx, dpdy);
-        const float4 derivatives = computeDerivatives(dpdx, dpdy, dpdu, dpdv);
-        // Register diet: what the code AFTER the BSDF sample needs of the geometry is reduced to its results now — the
-        // ray origin of either outcome (reflected / refracted: same operations as the one call the shader makes, for
-        // both values of its flag) and the normal's screen-space derivatives — so that the triangle's corners, vertex
-        // normals, barycentrics and uv derivatives are dead while the material and the BSDF are evaluated.
-        const vec3 originReflected = offsetRayOriginShadowTerminator(position, p0, p1, p2, n0, n1, n2, bary, false);
-        const vec3 originRefracted = offsetRayOriginShadowTerminator(position, p0, p1, p2, n0, n1, n2, bary, true);
-        const vec3 originThrough = offsetRayOriginSelfIntersection(position, -geometricNormal);
-        const vec3 dndx = dndu * derivatives.x + dndv * derivatives.y;
-        const vec3 dndy = dndu * derivatives.z + dndv * derivatives.w;
-
-        // ---- material, closestHit.rchit:101-117 -------------------------------------------------
-        MaterialSample material = sampleMaterial(s, materialId, texCoords.x, texCoords.y, derivatives, inside,
-                                                 (rc.hitFlags & PT_HIT_FLAGS_DX_NORMAL_TEXTURES) != 0,
-                                                 STATS ? &texels : nullptr);
-        if (ALPHA)
-        {
-            const float4 dec = rc.ps.rec[slot].decal;
-            if (dec.w != -1.0f && rayTmax > dec.w)
-                material.Color = mix(material.Color, V3(dec), rc.ps.rec[slot].decalA);
-        }
-        maxRoughness = fmaxf(material.Roughness, maxRoughness);
-        material.Roughness = fmaxf(maxRoughness, 0.01f);
-
-        const mat3 geometryTBN = mat3 { tangent, bitangent, normal };
-        const vec3 N = normalize(normal + mul(geometryTBN, material.Normal));
-        const mat3 TBN = computeTangentSpace(N);
-        // TBN is orthonormal: inverse(TBN) == transpose(TBN)
-        const vec3 V = normalize(mulT(TBN, normalize(-rayDir)));
-
-        BSDFSample bsdf = sampleBSDF(material, V, rng);
-
-        if (inside)
-        {
-            const float e = rayTmax / material.AttenuationDistance;
-            bsdf.Color.x *= powf(material.AttenuationColor.x, e);
-            bsdf.Color.y *= powf(material.AttenuationColor.y, e);
-            bsdf.Color.z *= powf(material.AttenuationColor.z, e);
-        }
-        const bool isRefracted = bsdf.Direction.z < 0.0f;
-        const vec3 rayOrigin = isRefracted ? originRefracted : originReflected;
-
-        float lightPdf, lightSmplPdf;
-        const float l0 = rnd(rng);
-        const float l1 = rnd(rng);
-        const float l2 = rnd(rng);
-        const LightSample light = sampleLight(s.lights, V3(l0, l1, l2), rayOrigin, lightPdf);
-        const vec3 L = normalize(mulT(TBN, -light.Direction));
-        const vec3 lightBsdf = evaluateBSDF(material, V, L, lightSmplPdf);
-
-        const vec3 newDir = normalize(mul(TBN, bsdf.Direction));
-        const vec3 newPos = isRefracted ? originThrough : rayOrigin;
-        const vec3 directLight = light.Color * light.Attenuation * lightBsdf;
-
-        propagateDifferentials(normal, rayOrigin, -rayDir, newDir, dndx, dndy, material.Eta, isRefracted, rd);
-
-        // ---- raygen.rgen:71-96 ----------------------------------------------------------------
-        radiance += throughput * material.EmissiveColor;
-        bool done = false;
-        if (bsdf.Pdf == -1.0f)
-            done = true; // raygen.rgen:71 cannot tell this from a miss
-        else
-        {
-            if (lightPdf > 0.0f)
-            {
-                const vec3 c = throughput * directLight / lightPdf;
-                // a contribution of exactly +-0 cannot change the radiance: the occlusion query is skipped
-                if (!(c.x == 0.0f && c.y == 0.0f && c.z == 0.0f))
-                {
-                    const vec3 sd = -normalize(light.Direction);
-                    rc.ps.rec[slot].shO = make_float4(newPos.x, newPos.y, newPos.z, light.Distance);
-                    rc.ps.rec[slot].shD = make_float4(sd.x, sd.y, sd.z, 0.0f);
-                    rc.ps.rec[slot].shC = make_float4(c.x, c.y, c.z, 0.0f);
-                    rc.ps.shadowQueue[atomicAggInc(&rc.qc->shadow)] = slot;
-                }
-            }
-            if (bsdf.Pdf > 0.001f)
-                throughput *= bsdf.Color / bsdf.Pdf;
-            const float prob = fminf(maxComponent(throughput), 1.0f);
-            if (prob < 0.001f)
-                done = true;
-            else if (prob < rnd(rng))
-                done = true;
-            else
-                throughput = throughput / prob;
-        }
-        const uint32_t bounce = (state & 0xffu) + 1;
-        if (bounce >= rc.bounceCount)
-            done = true;
-        state = (state & ~0xffu) | bounce;
-        // continuing paths go straight to the next iteration's queue (in shading = triangle order, so
-        // the next extend starts from spatially coherent origins); ended ones to its regen queue
-        // (their shadow ray, if any, is resolved by k_shadow before that)
-        if (done)
-            (cur ? rc.ps.regenQ[0] : rc.ps.regenQ[1])[atomicAggInc(&rc.qc->regen[cur ^ 1])] = slot | kRegen;
-        else
-            (cur ? rc.ps.contQ[0] : rc.ps.contQ[1])[atomicAggInc(&rc.qc->cont[cur ^ 1])] = slot;
-
-        rc.ps.rec[slot].rad = make_float4(radiance.x, radiance.y, radiance.z, rad4.w);
-        // the rng state outlives the path (a NaN/Inf restart continues the stream, raygen.rgen:99-112)
-        rc.ps.rec[slot].rayD = make_float4(newDir.x, newDir.y, newDir.z, __uint_as_float(rng));
-        if (!done)
-        {
-            rc.ps.rec[slot].thr = make_float4(throughput.x, throughput.y, throughput.z, __uint_as_float(state));
-            rc.ps.rec[slot].rayO = make_float4(newPos.x, newPos.y, newPos.z, maxRoughness);
-            rc.ps.rec[slot].diff0 = make_float4(rd.rxOrigin.x, rd.rxOrigin.y, rd.rxOrigin.z, rd.rxDirection.x);
-            rc.ps.rec[slot].diff1 = make_float4(rd.rxDirection.y, rd.rxDirection.z, rd.ryOrigin.x, rd.ryOrigin.y);
-            rc.ps.rec[slot].diff2 = make_float4(rd.ryOrigin.z, rd.ryDirection.x, rd.ryDirection.y, rd.ryDirection.z);
-        }
-    }
-    if (STATS)
-        warpAdd(&rc.counters->texels, texels);
-}
-
-// ---------------------------------------------------------------------------------------------
-// k_shade with emissive-triangle light sampling and MIS (pt_set_light_sampling, DESIGN.md §3g): the same closest-hit and
-// bounce logic, the same main rng stream, plus the emitter branch of the light sample, the MIS weight of emission found
-// by BSDF sampling and the previous bounce's BSDF pdf in the path record.  A copy rather than a template parameter of
-// k_shade: folding both into one body changed k_shade's machine code.
-// ---------------------------------------------------------------------------------------------
-template <bool ALPHA, bool STATS>
-__global__ void __launch_bounds__(128, PT_SHADE_MIN_BLOCKS) k_shade_emissive(RenderConst rc, int cur, EmitterTable em)
+template <bool ALPHA, bool STATS, bool EMISSIVE>
+__global__ void __launch_bounds__(128, PT_SHADE_MIN_BLOCKS) k_shade(RenderConst rc, int cur, EmitterTable em)
 {
     const uint32_t n = rc.qc->hit;
     const uint32_t stride = gridDim.x * blockDim.x;
@@ -658,7 +467,7 @@ __global__ void __launch_bounds__(128, PT_SHADE_MIN_BLOCKS) k_shade_emissive(Ren
         const vec2 uv0 = V2(a6.w, a7.x), uv1 = V2(a7.y, a7.z), uv2 = V2(a7.w, a8.x);
         // MIS weight of the emission this BSDF-sampled ray found (bounce >= 1 on a triangle the light sampling can pick)
         float emissionWeight = 1.0f;
-        if ((state & 0xffu) != 0)
+        if (EMISSIVE && (state & 0xffu) != 0)
         {
             const float pdfOverArea = __ldg(em.pdfOverArea + __float_as_uint(q0.w));
             if (pdfOverArea > 0.0f)
@@ -748,27 +557,30 @@ __global__ void __launch_bounds__(128, PT_SHADE_MIN_BLOCKS) k_shade_emissive(Ren
         const float l2 = rnd(rng);
         LightSample light = sampleLight(s.lights, V3(l0, l1, l2), rayOrigin, lightPdf);
         bool emitterSample = false;
-        // the branch, the alias draw (bucket, 32-bit fraction) and the point come from a secondary stream
-        uint32_t rng2 = lightSampleRng(rng);
-        if (rnd(rng2) < em.pEmitter)
+        if (EMISSIVE)
         {
-            const uint32_t hi = xorshift(rng2), lo = xorshift(rng2);
-            const uint32_t bucket = __umulhi(hi, em.count);
-            const uint2 entry = __ldg(em.alias + bucket);
-            const uint32_t k = lo < entry.x ? bucket : entry.y;
-            const float r1 = rnd(rng2);
-            const float r2 = rnd(rng2);
-            light = sampleEmitter(s, em, k, r1, r2, rayOrigin, lightPdf);
-            emitterSample = true;
-            // the last bounce: the reference mode never collects emission one vertex further, so neither does this
-            if ((state & 0xffu) + 1 >= rc.bounceCount)
-                lightPdf = 0.0f;
+            // the branch, the alias draw (bucket, 32-bit fraction) and the point come from a secondary stream
+            uint32_t rng2 = lightSampleRng(rng);
+            if (rnd(rng2) < em.pEmitter)
+            {
+                const uint32_t hi = xorshift(rng2), lo = xorshift(rng2);
+                const uint32_t bucket = __umulhi(hi, em.count);
+                const uint2 entry = __ldg(em.alias + bucket);
+                const uint32_t k = lo < entry.x ? bucket : entry.y;
+                const float r1 = rnd(rng2);
+                const float r2 = rnd(rng2);
+                light = sampleEmitter(s, em, k, r1, r2, rayOrigin, lightPdf);
+                emitterSample = true;
+                // the last bounce: the reference mode never collects emission one vertex further, so neither does this
+                if ((state & 0xffu) + 1 >= rc.bounceCount)
+                    lightPdf = 0.0f;
+            }
+            else
+                lightPdf = lightPdf * (1.0f - em.pEmitter);
         }
-        else
-            lightPdf = lightPdf * (1.0f - em.pEmitter);
         const vec3 L = normalize(mulT(TBN, -light.Direction));
         const vec3 lightBsdf = evaluateBSDF(material, V, L, lightSmplPdf);
-        if (emitterSample)
+        if (EMISSIVE && emitterSample)
             light.Attenuation = powerHeuristic(lightPdf, lightSmplPdf);
 
         const vec3 newDir = normalize(mul(TBN, bsdf.Direction));
@@ -778,7 +590,7 @@ __global__ void __launch_bounds__(128, PT_SHADE_MIN_BLOCKS) k_shade_emissive(Ren
         propagateDifferentials(normal, rayOrigin, -rayDir, newDir, dndx, dndy, material.Eta, isRefracted, rd);
 
         // ---- raygen.rgen:71-96 ----------------------------------------------------------------
-        radiance += throughput * (material.EmissiveColor * emissionWeight);
+        radiance += throughput * (EMISSIVE ? material.EmissiveColor * emissionWeight : material.EmissiveColor);
         bool done = false;
         if (bsdf.Pdf == -1.0f)
             done = true; // raygen.rgen:71 cannot tell this from a miss
@@ -790,7 +602,7 @@ __global__ void __launch_bounds__(128, PT_SHADE_MIN_BLOCKS) k_shade_emissive(Ren
                 // a contribution of exactly +-0 cannot change the radiance: the occlusion query is skipped.  A non-finite
                 // emitter sample is dropped: it must not cause a NaN/Inf restart the reference mode would not make.
                 if (!(c.x == 0.0f && c.y == 0.0f && c.z == 0.0f) &&
-                    !(emitterSample && (bad(c.x) || bad(c.y) || bad(c.z))))
+                    !(EMISSIVE && emitterSample && (bad(c.x) || bad(c.y) || bad(c.z))))
                 {
                     const vec3 sd = -normalize(light.Direction);
                     rc.ps.rec[slot].shO = make_float4(newPos.x, newPos.y, newPos.z, light.Distance);
@@ -831,7 +643,8 @@ __global__ void __launch_bounds__(128, PT_SHADE_MIN_BLOCKS) k_shade_emissive(Ren
             rc.ps.rec[slot].diff0 = make_float4(rd.rxOrigin.x, rd.rxOrigin.y, rd.rxOrigin.z, rd.rxDirection.x);
             rc.ps.rec[slot].diff1 = make_float4(rd.rxDirection.y, rd.rxDirection.z, rd.ryOrigin.x, rd.ryOrigin.y);
             rc.ps.rec[slot].diff2 = make_float4(rd.ryOrigin.z, rd.ryDirection.x, rd.ryDirection.y, rd.ryDirection.z);
-            rc.ps.rec[slot].pad[0] = __float_as_uint(bsdf.Pdf);
+            if (EMISSIVE)
+                rc.ps.rec[slot].pad[0] = __float_as_uint(bsdf.Pdf);
         }
     }
     if (STATS)
@@ -894,50 +707,35 @@ template <bool ALPHA, bool STATS> __global__ void __launch_bounds__(128, PT_TRAC
 // ---------------------------------------------------------------------------------------------
 // resolve: acc += radiance, one sample after the other (raygen.rgen:115-117 over consecutive frames)
 // ---------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) k_resolve(RenderConst rc)
+// ADAPTIVE adds the Welford update of the pixel's luminance statistics per sample (DESIGN.md §3i); a dropped frame
+// (parked as 0) is a sample of luminance 0, as in the accumulation.  state is read only when ADAPTIVE.
+template <bool ADAPTIVE> __global__ void __launch_bounds__(256) k_resolve(RenderConst rc, AdaptivePixel *state)
 {
     const uint32_t stride = gridDim.x * blockDim.x;
     for (uint32_t pi = blockIdx.x * blockDim.x + threadIdx.x; pi < rc.pixelCount; pi += stride)
     {
         const uint32_t pixel = __ldg(rc.pixelList + pi);
         float4 a = rc.accum[pixel];
+        AdaptivePixel st = ADAPTIVE ? state[pixel] : AdaptivePixel {};
         for (uint32_t s = 0; s < rc.roundSamples; s++)
         {
             const float4 r = __ldcs(rc.sbuf + (size_t)s * rc.pixelCount + pi);
             a.x = r.x + a.x;
             a.y = r.y + a.y;
             a.z = r.z + a.z;
+            if (ADAPTIVE)
+            {
+                const float l = (0.2126f * r.x + 0.7152f * r.y) + 0.0722f * r.z;
+                st.count += 1;
+                const float d = l - st.mean;
+                st.mean += d / (float)st.count;
+                st.m2 += d * (l - st.mean);
+            }
         }
         a.w = 1.0f;
         rc.accum[pixel] = a;
-    }
-}
-
-// k_resolve's additions (same order, same expressions) plus the Welford update of the pixel's luminance statistics per
-// sample (DESIGN.md §3i); a dropped frame (parked as 0) is a sample of luminance 0, as in the accumulation
-__global__ void __launch_bounds__(256) k_resolve_adaptive(RenderConst rc, AdaptivePixel *state)
-{
-    const uint32_t stride = gridDim.x * blockDim.x;
-    for (uint32_t pi = blockIdx.x * blockDim.x + threadIdx.x; pi < rc.pixelCount; pi += stride)
-    {
-        const uint32_t pixel = __ldg(rc.pixelList + pi);
-        float4 a = rc.accum[pixel];
-        AdaptivePixel st = state[pixel];
-        for (uint32_t s = 0; s < rc.roundSamples; s++)
-        {
-            const float4 r = __ldcs(rc.sbuf + (size_t)s * rc.pixelCount + pi);
-            a.x = r.x + a.x;
-            a.y = r.y + a.y;
-            a.z = r.z + a.z;
-            const float l = (0.2126f * r.x + 0.7152f * r.y) + 0.0722f * r.z;
-            st.count += 1;
-            const float d = l - st.mean;
-            st.mean += d / (float)st.count;
-            st.m2 += d * (l - st.mean);
-        }
-        a.w = 1.0f;
-        rc.accum[pixel] = a;
-        state[pixel] = st;
+        if (ADAPTIVE)
+            state[pixel] = st;
     }
 }
 
@@ -1596,22 +1394,24 @@ pt_status renderRounds(Context *ctx, const pt_render_params *params, uint32_t fi
             const RenderConst &rc = pl.rc;
             const int cur = pl.cur;
             cudaStream_t st = pl.stream;
-#define PT_DISPATCH(KERNEL, GRID, BLOCK, ...)                                                                         \
+            // launches KERNEL<alpha, statsOn, ...> ARGS: the runtime flags as template arguments, then the arguments that
+            // follow ARGS, if any (", ##" drops the comma when there are none)
+#define PT_DISPATCH(KERNEL, GRID, BLOCK, ARGS, ...)                                                                   \
     do                                                                                                                \
     {                                                                                                                 \
         if (alpha && statsOn)                                                                                         \
-            KERNEL<true, true><<<GRID, BLOCK, 0, st>>>(__VA_ARGS__);                                                  \
+            KERNEL<true, true, ##__VA_ARGS__><<<GRID, BLOCK, 0, st>>> ARGS;                                           \
         else if (alpha)                                                                                               \
-            KERNEL<true, false><<<GRID, BLOCK, 0, st>>>(__VA_ARGS__);                                                 \
+            KERNEL<true, false, ##__VA_ARGS__><<<GRID, BLOCK, 0, st>>> ARGS;                                          \
         else if (statsOn)                                                                                             \
-            KERNEL<false, true><<<GRID, BLOCK, 0, st>>>(__VA_ARGS__);                                                 \
+            KERNEL<false, true, ##__VA_ARGS__><<<GRID, BLOCK, 0, st>>> ARGS;                                          \
         else                                                                                                          \
-            KERNEL<false, false><<<GRID, BLOCK, 0, st>>>(__VA_ARGS__);                                                \
+            KERNEL<false, false, ##__VA_ARGS__><<<GRID, BLOCK, 0, st>>> ARGS;                                         \
     } while (0)
             begin(PT_KERNEL_EXTEND, st);
             if (rc.sortHits)
                 PT_CUDA_CHECK(ctx, cudaMemsetAsync(rc.ps.hitKey, 0xff, (size_t)rc.slotCount * 4, st));
-            PT_DISPATCH(k_extend, pl.gridExtend, 128, rc, cur);
+            PT_DISPATCH(k_extend, pl.gridExtend, 128, (rc, cur));
             end(st);
             begin(PT_KERNEL_SHADE, st);
             if (rc.sortHits)
@@ -1623,12 +1423,12 @@ pt_status renderRounds(Context *ctx, const pt_render_params *params, uint32_t fi
                                                                    (int)keyBits + 1, st));
             }
             if (emissive)
-                PT_DISPATCH(k_shade_emissive, pl.gridShade, 128, rc, cur, emitters);
+                PT_DISPATCH(k_shade, pl.gridShade, 128, (rc, cur, emitters), true);
             else
-                PT_DISPATCH(k_shade, pl.gridShade, 128, rc, cur);
+                PT_DISPATCH(k_shade, pl.gridShade, 128, (rc, cur, emitters), false);
             end(st);
             begin(PT_KERNEL_SHADOW, st);
-            PT_DISPATCH(k_shadow, pl.gridShadow, 128, rc, cur);
+            PT_DISPATCH(k_shadow, pl.gridShadow, 128, (rc, cur));
             end(st);
 #undef PT_DISPATCH
             ctx->stats.kernel_launches += 3;
@@ -1678,9 +1478,9 @@ pt_status renderRounds(Context *ctx, const pt_render_params *params, uint32_t fi
         begin(PT_KERNEL_FINISH, ctx->stream);
         const uint32_t resolveGrid = std::min((pixels + 255) / 256, (uint32_t)ctx->smCount * 8);
         if (adaptive)
-            k_resolve_adaptive<<<resolveGrid, 256, 0, ctx->stream>>>(base, ctx->adaptivePixels);
+            k_resolve<true><<<resolveGrid, 256, 0, ctx->stream>>>(base, ctx->adaptivePixels);
         else
-            k_resolve<<<resolveGrid, 256, 0, ctx->stream>>>(base);
+            k_resolve<false><<<resolveGrid, 256, 0, ctx->stream>>>(base, nullptr);
         end(ctx->stream);
         ctx->stats.kernel_launches++;
     }

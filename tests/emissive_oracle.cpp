@@ -5,7 +5,7 @@
  * traversal, material, BSDF and sampler code are the oracle's own, and adds the emitter table and a raygen /
  * closest-hit pair with the emitter branch of the light sample and the MIS weight of emission found by BSDF sampling.
  * The reference mode is the oracle's pto_render of the same library.  The definitions are those of
- * path-tracing_b200/csrc/emitters.cu and k_shade_emissive; the emitter table is equal entry for entry. */
+ * path-tracing_b200/csrc/emitters.cu and k_shade<A, S, true>; the emitter table is equal entry for entry. */
 #include "../oracle/pt_oracle.cpp"
 
 namespace

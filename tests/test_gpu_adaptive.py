@@ -288,12 +288,12 @@ def test_adaptive_beats_uniform_at_equal_samples():
     assert (counts == 16).mean() > 0.25 and ea < 0.95 * eu, ((counts == 16).mean(), ea, eu, ea / eu)
 
 
-def test_adaptive_kernels_do_not_spill():
+def test_adaptive_kernel_instances_do_not_spill():
     test_kernel_budgets.kernel_stats()  # builds the library if the log is missing
     found = 0
     for path in (test_kernel_budgets.LOG.replace("wavefront.ptxas.log", "adaptive.ptxas.log"), test_kernel_budgets.LOG):
         text = open(path).read()
-        for m in re.finditer(r"Function properties for (\S*(k_adaptive_\w+?|k_resolve_adaptive)E\S*)\n\s+(\d+) bytes stack frame, "
+        for m in re.finditer(r"Function properties for (\S*(k_adaptive_\w+?|k_resolveILb1E)E\S*)\n\s+(\d+) bytes stack frame, "
                              r"(\d+) bytes spill stores, (\d+) bytes spill loads\nptxas info\s+: Used (\d+) registers", text):
             found += 1
             print(f"{m[2]}: {m[6]} registers, stack {m[3]} bytes, spills {m[4]} / {m[5]} bytes (stores / loads)")

@@ -3,7 +3,6 @@ emitter table against the CPU reference's (tests/emissive_oracle.cpp) entry for 
 mode within the bounds of test_gpu_configs.test_image_parity, path identity with the reference mode, and determinism
 across scheduling, tiles, scene updates and mode switches."""
 import importlib
-import re
 
 import numpy as np
 import pytest
@@ -12,7 +11,6 @@ import conftest
 import emissive_scenes as es
 from emissive_oracle import EmissiveOracleScene
 import metrics
-import test_kernel_budgets
 from scenes_small import SMALL, W, H
 
 pytestmark = pytest.mark.gpu
@@ -172,15 +170,3 @@ def test_a_scene_without_emitters_renders_as_the_reference_mode():
     s = es.room(96, 64, emitters=False)
     assert (render_room(scene=s) == render_room(scene=s, mode="reference")).all()
 
-
-def test_k_shade_emissive_register_budget():
-    """k_shade_emissive: 128 registers at most, like k_shade (four 128-thread blocks per SM); its spills are reported."""
-    test_kernel_budgets.kernel_stats()  # builds the library if the log is missing
-    text = open(test_kernel_budgets.LOG).read()
-    found = 0
-    for m in re.finditer(r"Function properties for (\S*k_shade_emissiveILb([01])ELb([01])E\S*)\n\s+(\d+) bytes stack frame, "
-                         r"(\d+) bytes spill stores, (\d+) bytes spill loads\nptxas info\s+: Used (\d+) registers", text):
-        found += 1
-        print(f"k_shade_emissive<{m[2]},{m[3]}>: {m[7]} registers, spills {m[5]} / {m[6]} bytes (stores / loads)")
-        assert int(m[7]) <= 128, m[0]
-    assert found == 4

@@ -3,7 +3,7 @@
 For each scene and threshold, in one process on one GPU: the time of one adaptive call (min 16, max 1024, batch 16 spp,
 the default min_pass_items) on a fresh target, its passes and its mean and maximum samples per pixel; relMSE and FLIP of
 its mean image against a 1024-spp render of independent samples, beside uniform renders at equal samples and at equal
-time; and, in a separate profiled call, the device time of the new kernels (k_adaptive_*, the scan, k_resolve_adaptive) as
+time; and, in a separate profiled call, the device time of the new kernels (k_adaptive_*, the scan, k_resolve<true>) as
 a share of that profiled call's wall time.  Street renders in the emissive-MIS light-sampling mode.  Prints one JSON line
 per scene and threshold and writes them to --out."""
 import argparse
@@ -65,7 +65,7 @@ def kernel_share(r, p, w, h, kw):
     kernels = {}
     for e in prof.key_averages():
         # the pass's scan is CUB's DeviceScan (the hit sort uses DeviceRadixSort kernels, which do not match)
-        for k in ("k_adaptive_blocks", "k_adaptive_select", "DeviceScan", "k_adaptive_scatter", "k_adaptive_mean", "k_resolve_adaptive"):
+        for k in ("k_adaptive_blocks", "k_adaptive_select", "DeviceScan", "k_adaptive_scatter", "k_adaptive_mean", "k_resolve<true>"):
             if k in e.key:
                 t = getattr(e, "device_time_total", None) or e.cuda_time_total
                 kernels[k] = kernels.get(k, 0.0) + t / 1e3

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Register / spill figures of ONE kernel of a .cu file without building the library (nvcc -ptx, cut the entry out, ptxas -v):
-    tools/kernel_regs.py wavefront.cu k_shadeILb0ELb0 [-DFLAG ...] [--maxrregcount N]
+    tools/kernel_regs.py wavefront.cu k_shadeILb0ELb0ELb0E [-DFLAG ...] [--maxrregcount N]
 The .maxntid / .minnctapersm directives of the entry (its __launch_bounds__) are honoured unless --maxrregcount is given."""
 import os
 import re
