@@ -730,6 +730,25 @@ PT_API pt_status pt_debug_render(pt_context *ctx, const pt_render_params *params
 PT_API pt_status pt_test_texture(pt_context *ctx, uint32_t slot, const float *in6, float *out4, uint32_t count,
                                  int32_t use_grad);
 
+/* Flags of pt_test_trace. */
+enum {
+    PT_TEST_TRACE_OCCLUSION = 0x1,  /* occlusion query (k_shadow's); otherwise closest hit (k_extend's)          */
+    PT_TEST_TRACE_PERSISTENT = 0x2, /* the render's persistent traversal (dynamic ray fetch, straggler splitting);
+                                       otherwise the per-thread traversal of pt_trace_closest / pt_trace_occlusion */
+    PT_TEST_TRACE_STATS = 0x4       /* the traversal-statistics instantiation, with the tail counters           */
+};
+
+/* Traversal probe: traces `ray_count` host rays with the traversal the render's trace kernels run, so that its hits
+ * can be compared with the standalone queries hit for hit.  Every ray must have the same tmin (the persistent traversal
+ * takes one; PT_ERR_INVALID_ARGUMENT otherwise).  out_hits gets one pt_hit per ray; for occlusion queries
+ * instance != PT_NO_HIT means occluded.  out_decals (may be NULL) gets r, g, b, a, dist per ray: the decal record of
+ * a closest-hit query on a scene with alpha-tested geometry (dist = -1: none).  blocks = 0 launches the resident grid
+ * of the render; a small count (1) sends nearly all rays through the drain mode.  out_tail (may be NULL) gets
+ * {warp_iterations, warp_drain_iterations, max_warp_drain_iterations, stack_overflows} (the first three counted with
+ * PT_TEST_TRACE_STATS | PT_TEST_TRACE_PERSISTENT only). */
+PT_API pt_status pt_test_trace(pt_context *ctx, const pt_ray *rays, uint64_t ray_count, uint32_t flags, uint32_t blocks,
+                               pt_hit *out_hits, float *out_decals, uint64_t *out_tail);
+
 #ifdef __cplusplus
 }
 #endif

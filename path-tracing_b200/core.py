@@ -47,6 +47,7 @@ ABI_SYMBOLS = [
     "pt_test_output_stride",
     "pt_test_shading",
     "pt_test_texture",
+    "pt_test_trace",
     "pt_debug_render",
     "pt_set_light_sampling",
     "pt_emitter_table",
@@ -61,6 +62,8 @@ ABI_SYMBOLS = [
 
 # pt_light_sampling, include/pt_core.h
 LIGHT_SAMPLING = {"reference": 0, "emissive_mis": 1}
+# flags of pt_test_trace, include/pt_core.h
+TEST_TRACE_OCCLUSION, TEST_TRACE_PERSISTENT, TEST_TRACE_STATS = 0x1, 0x2, 0x4
 
 
 class PtError(RuntimeError):
@@ -306,6 +309,7 @@ def lib():
     L.pt_test_output_stride.restype = u32
     L.pt_test_shading.argtypes = [vp, u32, vp, vp, u32]
     L.pt_test_texture.argtypes = [vp, u32, vp, vp, u32, i32]
+    L.pt_test_trace.argtypes = [vp, vp, u64, u32, u32, vp, vp, vp]
     L.pt_debug_render.argtypes = [vp, vp, vp, u32, u32, vp]
     L.pt_denoise.argtypes = [vp, vp, vp, u32, vp, C.c_size_t]
     L.pt_denoise_guides.argtypes = [vp, vp, vp, C.c_size_t]
@@ -562,6 +566,22 @@ class Renderer:
         out = np.zeros(len(rays), np.uint8)
         self._check(self._L.pt_trace_occlusion(self._h, rays.ctypes.data, len(rays), out.ctypes.data))
         return out
+
+    def test_trace(self, rays: np.ndarray, occlusion: bool = False, persistent: bool = True, blocks: int = 0, stats: bool = False):
+        """Rays through the traversal of the render's trace kernels (pt_test_trace): the persistent, warp-synchronous
+        one of k_extend (closest) / k_shadow (occlusion), or with persistent=False the per-thread one of trace_closest /
+        trace_occlusion.  All rays must share one tmin.  blocks = 0 is the render's resident grid.  Returns (hits,
+        decals, tail): sc.HIT records (occlusion: instance != NO_HIT = occluded), (N, 5) float32 decal records r, g, b, a,
+        dist (dist = -1: none) and a dict of the tail counters (counted with stats=True and persistent=True)."""
+        rays = np.ascontiguousarray(rays, sc.RAY)
+        hits = np.zeros(len(rays), sc.HIT)
+        decals = np.zeros((len(rays), 5), np.float32)
+        tail = np.zeros(4, np.uint64)
+        flags = (TEST_TRACE_OCCLUSION if occlusion else 0) | (TEST_TRACE_PERSISTENT if persistent else 0) | (TEST_TRACE_STATS if stats else 0)
+        self._check(self._L.pt_test_trace(self._h, rays.ctypes.data, len(rays), flags, int(blocks), hits.ctypes.data,
+                                          decals.ctypes.data, tail.ctypes.data))
+        names = ("warp_iterations", "warp_drain_iterations", "max_warp_drain_iterations", "stack_overflows")
+        return hits, decals, {k: int(v) for k, v in zip(names, tail)}
 
     def stats(self) -> dict:
         s = Stats()

@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <string>
 #include <vector>
 
@@ -285,6 +286,23 @@ inline cudaError_t poolAlloc(Context *ctx, void **ptr, size_t bytes, cudaStream_
 // traversal-stack overflows since the last call (wavefront.cu); non-zero fails the call that caused them
 pt_status checkStackOverflow(Context *ctx, const char *what);
 
+// resident 128-thread blocks per SM the register allocation of the trace kernels (k_extend, k_shadow and their probe
+// k_test_trace) must allow (tuned on the B200, see DESIGN.md)
+#ifndef PT_TRACE_MIN_BLOCKS
+#define PT_TRACE_MIN_BLOCKS 8
+#endif
+// Grid of a persistent trace launch: exactly as many 128-thread blocks as are resident on the machine (occupancy query
+// per instantiation; PT_TRACE_BLOCKS overrides), never more than `items` work items need.
+template <class Kernel> uint32_t residentTraceGrid(const Context *ctx, Kernel kernel, uint32_t items)
+{
+    int perSM = 0;
+    if (ctx->traceBlocksPerSM)
+        perSM = (int)ctx->traceBlocksPerSM;
+    else if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, kernel, 128, 0) != cudaSuccess || perSM < 1)
+        perSM = 4;
+    return std::min((items + 127) / 128, (uint32_t)(ctx->smCount * perSM));
+}
+
 // bvh_build.cu
 pt_status uploadScene(Context *ctx, const pt_scene_desc *desc);
 void freeScene(Context *ctx);
@@ -321,6 +339,9 @@ pt_status debugRender(Context *ctx, const pt_render_params *params, const pt_deb
                       float *out);
 pt_status traceClosest(Context *ctx, const pt_ray *rays, uint64_t n, pt_hit *out);
 pt_status traceOcclusion(Context *ctx, const pt_ray *rays, uint64_t n, uint8_t *out);
+// pt_test_trace: the trace kernels' persistent traversal (or the per-thread one) on host rays
+pt_status testTrace(Context *ctx, const pt_ray *rays, uint64_t n, uint32_t flags, uint32_t blocks, pt_hit *out, float *outDecals,
+                    uint64_t *outTail);
 // k_denoise_guides over the render target's extent, queued on ctx->stream
 void launchDenoiseGuides(Context *ctx, const pt_render_params *params, float4 *albedoT, float4 *normal);
 

@@ -664,6 +664,15 @@ pt_status pt_test_texture(pt_context *ctx, uint32_t slot, const float *in6, floa
     return testTexture(ctx, slot, in6, out4, count, use_grad);
 }
 
+pt_status pt_test_trace(pt_context *ctx, const pt_ray *rays, uint64_t ray_count, uint32_t flags, uint32_t blocks, pt_hit *out_hits,
+                        float *out_decals, uint64_t *out_tail)
+{
+    if (!ctx)
+        return PT_ERR_INVALID_ARGUMENT;
+    DeviceGuard guard(ctx->device);
+    return testTrace(ctx, rays, ray_count, flags, blocks, out_hits, out_decals, out_tail);
+}
+
 uint32_t pt_test_input_stride(uint32_t mode) { return testInputStride(mode); }
 uint32_t pt_test_output_stride(uint32_t mode) { return testOutputStride(mode); }
 

@@ -236,6 +236,18 @@ PT_DEV void intersectNode(const BvhNode *__restrict__ node, const RaySetup &r, f
     const float ax = __uint_as_float(w0.w) * r.idx, ay = __uint_as_float(w1.x) * r.idy, az = __uint_as_float(w1.y) * r.idz;
     const float bx = (__uint_as_float(w0.x) - r.org.x) * r.idx, by = (__uint_as_float(w0.y) - r.org.y) * r.idy;
     const float bz = (__uint_as_float(w0.z) - r.org.z) * r.idz;
+    // The rounding of fmaf(k, a, b) is ABSOLUTE, a few ulp of |b| + 255 |a| (the distances of the node's planes), not of the
+    // result: for a ray that starts near a surface inside a large node (every continuation ray) it exceeds any relative
+    // slack, and a box whose face holds the edge or vertex the ray crosses was culled — rays leaked through closed meshes,
+    // and ties at shared vertices depended on the visiting order.  Entry planes therefore move 4 units of roundoff of their
+    // axis' terms closer, exit planes as much farther, plus the same of the dominant axis kz, which bounds the rounding of
+    // the t of a triangle inside the node.  (A zero direction component makes its axis NaN, which the min / max drop.)
+    const float ex = fmaf(255.0f, fabsf(ax), fabsf(bx)), ey = fmaf(255.0f, fabsf(ay), fabsf(by));
+    const float ez = fmaf(255.0f, fabsf(az), fabsf(bz));
+    const float kErr = 2.3841858e-7f; // 4 * 2^-24
+    const float eKz = kErr * comp(V3(ex, ey, ez), r.kz);
+    const float sx = fmaf(kErr, ex, eKz), sy = fmaf(kErr, ey, eKz), sz = fmaf(kErr, ez, eKz);
+    const float bnx = bx - sx, bfx = bx + sx, bny = by - sy, bfy = by + sy, bnz = bz - sz, bfz = bz + sz;
     // entry / exit planes by the sign of the direction
     const uint32_t nxw = r.nearX ? w2.y : w1.z, fxw = r.nearX ? w1.z : w2.y;
     const uint32_t nyw = r.nearY ? w2.z : w1.w, fyw = r.nearY ? w1.w : w2.z;
@@ -243,12 +255,12 @@ PT_DEV void intersectNode(const BvhNode *__restrict__ node, const RaySetup &r, f
 #pragma unroll
     for (int i = 0; i < 4; i++)
     {
-        const float tnx = fmaf((float)((nxw >> (8 * i)) & 0xffu), ax, bx), tfx = fmaf((float)((fxw >> (8 * i)) & 0xffu), ax, bx);
-        const float tny = fmaf((float)((nyw >> (8 * i)) & 0xffu), ay, by), tfy = fmaf((float)((fyw >> (8 * i)) & 0xffu), ay, by);
-        const float tnz = fmaf((float)((nzw >> (8 * i)) & 0xffu), az, bz), tfz = fmaf((float)((fzw >> (8 * i)) & 0xffu), az, bz);
+        const float tnx = fmaf((float)((nxw >> (8 * i)) & 0xffu), ax, bnx), tfx = fmaf((float)((fxw >> (8 * i)) & 0xffu), ax, bfx);
+        const float tny = fmaf((float)((nyw >> (8 * i)) & 0xffu), ay, bny), tfy = fmaf((float)((fyw >> (8 * i)) & 0xffu), ay, bfy);
+        const float tnz = fmaf((float)((nzw >> (8 * i)) & 0xffu), az, bnz), tfz = fmaf((float)((fzw >> (8 * i)) & 0xffu), az, bfz);
         const float t0 = fmaxf(fmaxf(tnx, tny), fmaxf(tnz, tmin));
         const float t1 = fminf(fminf(tfx, tfy), fminf(tfz, tmax));
-        // conservative: the slack absorbs the rounding of the three-operation plane distance
+        // the relative slack absorbs the rounding of t0 and t1 themselves
         d[i] = (c[i] != PT_CHILD_EMPTY && t0 <= t1 * 1.0000008f) ? t0 : INFINITY;
     }
 }

@@ -38,10 +38,6 @@ namespace pt
 namespace
 {
 
-// resident 128-thread blocks per SM the register allocation must allow (tuned on the B200, see DESIGN.md)
-#ifndef PT_TRACE_MIN_BLOCKS
-#define PT_TRACE_MIN_BLOCKS 8
-#endif
 // bits of the leaf-order triangle index the hit queue is sorted by; one more bit sends unused entries
 // to the end, and CUB's onesweep sort takes one pass per 8 bits: 15 + 1 = two passes
 #ifndef PT_HIT_KEY_BITS
@@ -1365,16 +1361,8 @@ pt_status renderRounds(Context *ctx, const pt_render_params *params, uint32_t fi
             pl.cur = 0;
             pl.active = true;
             pl.gridShade = std::min((slots + 127) / 128, (uint32_t)ctx->smCount * PT_SHADE_GRID_PER_SM);
-            // persistent warps: exactly as many blocks as are resident on the machine (occupancy query per
-            // instantiation; PT_TRACE_BLOCKS overrides), never more than the rays need
-            auto residentGrid = [&](auto kernel) {
-                int perSM = 0;
-                if (ctx->traceBlocksPerSM)
-                    perSM = (int)ctx->traceBlocksPerSM;
-                else if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, kernel, 128, 0) != cudaSuccess || perSM < 1)
-                    perSM = 4;
-                return std::min((slots + 127) / 128, (uint32_t)(ctx->smCount * perSM));
-            };
+            // persistent warps: the resident grid, never more than the rays need
+            auto residentGrid = [&](auto kernel) { return residentTraceGrid(ctx, kernel, slots); };
             if (alpha && statsOn)
                 pl.gridExtend = residentGrid(k_extend<true, true>), pl.gridShadow = residentGrid(k_shadow<true, true>);
             else if (alpha)
