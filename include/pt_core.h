@@ -534,6 +534,30 @@ PT_API pt_status pt_denoise_guides(pt_context *ctx, float *out_albedo_t, float *
 PT_API pt_status pt_postprocess_denoised(pt_context *ctx, const pt_postprocess_params *params, uint32_t output_format,
                                          void *out_pixels, size_t out_bytes);
 
+/* ---- temporal denoiser (DESIGN §3j) --------------------------------------- */
+
+/* SVGF's temporal stage (Schied et al. 2017, §4.1-4.2): the demodulated irradiance of each call is accumulated into a
+ * per-pixel history reprojected from the previous call's camera, and the spatial filter runs on the result. */
+typedef struct pt_temporal_params {
+    float alpha;          /* weight of the new frame once the history is long: a = max(alpha, 1/n); 0..1 (SVGF: 0.2) */
+    float alpha_moments;  /* the same for the luminance moments, 0..1 (SVGF: 0.2)                                 */
+    uint32_t reset;       /* 1: discard the history before this frame                                              */
+} pt_temporal_params;
+
+/* One frame of temporal denoising: accumulation / total_samples of the current target is reprojected against the
+ * history of the previous call, accumulated, and filtered like pt_denoise. Output and pt_postprocess_denoised as pt_denoise.
+ * The history, the previous call's guides and its camera belong to the render target: pt_render_begin at the same extent
+ * keeps them (a moving camera restarts the accumulation every frame), an extent change, pt_scene_upload, pt_scene_update
+ * and pt_texture_upload discard them, and pt_denoise does not touch them. Other changes of the render parameters or of the
+ * light-sampling mode are the caller's to handle (with reset = 1). lens_radius > 0 is PT_ERR_UNSUPPORTED; a target holding
+ * an adaptive render is PT_ERR_INVALID_ARGUMENT. */
+PT_API pt_status pt_denoise_temporal(pt_context *ctx, const pt_render_params *params, const pt_denoise_params *denoise,
+                                     const pt_temporal_params *temporal, uint32_t total_samples, float *out_rgba, size_t out_bytes);
+
+/* The history after the last call, per pixel (row-major, `pixels` >= width * height): (integrated irradiance.rgb, history
+ * length n) and (m1, m2), the moving averages of the luminance and its square. Either may be NULL. */
+PT_API pt_status pt_denoise_temporal_history(pt_context *ctx, float *out_irradiance_n, float *out_moments, size_t pixels);
+
 /* ---- adaptive sampling (DESIGN §3i) --------------------------------------- */
 
 /* Each pixel keeps its sample count and Welford statistics (mean, M2) of its samples' luminance

@@ -54,6 +54,8 @@ ABI_SYMBOLS = [
     "pt_denoise",
     "pt_denoise_guides",
     "pt_postprocess_denoised",
+    "pt_denoise_temporal",
+    "pt_denoise_temporal_history",
     "pt_render_adaptive",
     "pt_adaptive_readback",
     "pt_postprocess_adaptive",
@@ -87,6 +89,12 @@ class DenoiseParams(C.Structure):
     """pt_denoise_params: a-trous levels and the edge-stopping parameters of the denoiser (DESIGN.md §3h)."""
 
     _fields_ = [("iterations", C.c_uint32), ("sigma_luminance", C.c_float), ("sigma_normal", C.c_float), ("sigma_depth", C.c_float)]
+
+
+class TemporalParams(C.Structure):
+    """pt_temporal_params: the moving-average weights of the temporal denoiser and its reset flag (DESIGN.md §3j)."""
+
+    _fields_ = [("alpha", C.c_float), ("alpha_moments", C.c_float), ("reset", C.c_uint32)]
 
 
 class AdaptiveParams(C.Structure):
@@ -314,6 +322,8 @@ def lib():
     L.pt_denoise.argtypes = [vp, vp, vp, u32, vp, C.c_size_t]
     L.pt_denoise_guides.argtypes = [vp, vp, vp, C.c_size_t]
     L.pt_postprocess_denoised.argtypes = [vp, vp, u32, vp, C.c_size_t]
+    L.pt_denoise_temporal.argtypes = [vp, vp, vp, vp, u32, vp, C.c_size_t]
+    L.pt_denoise_temporal_history.argtypes = [vp, vp, vp, C.c_size_t]
     L.pt_render_adaptive.argtypes = [vp, vp, vp, vp]
     L.pt_adaptive_readback.argtypes = [vp, vp, vp, C.c_size_t]
     L.pt_postprocess_adaptive.argtypes = [vp, vp, u32, vp, C.c_size_t]
@@ -503,6 +513,32 @@ class Renderer:
             return out
         self._check(self._L.pt_denoise(self._h, C.addressof(p), C.addressof(d), int(n), out.ctypes.data, out.nbytes))
         return out
+
+    def denoise_temporal(self, params: sc.RenderParams | None = None, iterations: int = 5, sigma_luminance: float = 4.0,
+                         sigma_normal: float = 128.0, sigma_depth: float = 1.0, alpha: float = 0.2, alpha_moments: float = 0.2,
+                         reset: bool = False, total_samples: int | None = None) -> np.ndarray:
+        """One frame of the temporal denoiser (DESIGN.md §3j): accumulation / total_samples is accumulated into the history
+        reprojected from the previous call's camera, then filtered like denoise().  params carries the camera of this
+        frame; the history survives on_resize() at the same extent, so an interactive loop calls on_resize(), render() and
+        denoise_temporal() per frame.  Returns (H, W, 4) float32 mean radiance, A = 1, kept on the device for
+        postprocess(denoised=True) and the save_* writers."""
+        p = (params or self.params).to_c()
+        d = DenoiseParams(int(iterations), sigma_luminance, sigma_normal, sigma_depth)
+        t = TemporalParams(alpha, alpha_moments, 1 if reset else 0)
+        n = self.total_samples if total_samples is None else total_samples
+        out = np.empty((self.height, self.width, 4), np.float32)
+        self._check(self._L.pt_denoise_temporal(self._h, C.addressof(p), C.addressof(d), C.addressof(t), int(n), out.ctypes.data,
+                                                out.nbytes))
+        return out
+
+    def temporal_history(self) -> dict:
+        """The temporal denoiser's history after the last denoise_temporal(): "irradiance" (H, W, 3) integrated demodulated
+        irradiance, "length" (H, W) history length n (0 on invalid pixels) and "moments" (H, W, 2) (m1, m2) of its
+        luminance."""
+        irr = np.empty((self.height, self.width, 4), np.float32)
+        mom = np.empty((self.height, self.width, 2), np.float32)
+        self._check(self._L.pt_denoise_temporal_history(self._h, irr.ctypes.data, mom.ctypes.data, self.width * self.height))
+        return {"irradiance": irr[..., :3], "length": irr[..., 3], "moments": mom}
 
     def denoise_guides(self) -> dict:
         """The guides of the last denoise(): "albedo" (H, W, 3), "t" (H, W; -1 on a miss) and "normal" (H, W, 3)."""

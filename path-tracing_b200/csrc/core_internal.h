@@ -191,6 +191,16 @@ struct Context
     float4 *denoisePing = nullptr, *denoisePong = nullptr;
     float2 *denoiseGrad = nullptr;
     bool denoiseValid = false; // a pt_denoise result exists for the current accumulation
+    // temporal denoiser state (temporal.cu, DESIGN §3j), one target allocation made at the first pt_denoise_temporal:
+    // two history buffers of (integrated irradiance.rgb, history length n) and (m1, m2) -- one is read while the other is
+    // written -- and the previous call's (N, t) taps (t = -1 where the pixel was invalid).  The previous camera is kept
+    // here.  It survives pt_render_begin at the same extent; scene and texture uploads and updates clear temporalValid.
+    float4 *temporalIrr[2] = {};
+    float2 *temporalMoments[2] = {};
+    float4 *temporalPrevNT = nullptr;
+    uint32_t temporalCurrent = 0; // temporalIrr / temporalMoments[temporalCurrent] hold the history after the last call
+    bool temporalValid = false;
+    float temporalPrevView[16] = {}, temporalPrevProj[16] = {};
     // what the accumulation holds since the last pt_render_begin: nothing, a uniform render (pt_render_samples /
     // pt_render_frames) or an adaptive one (pt_render_adaptive); the two never mix, so per-pixel counts stay known
     enum class TargetContent { Empty, Uniform, Adaptive } targetContent = TargetContent::Empty;
@@ -352,6 +362,20 @@ pt_status checkDenoise(Context *ctx, const char *what, const pt_render_params *p
                        const float *out, size_t outBytes);
 pt_status denoise(Context *ctx, const char *what, const pt_render_params *params, const pt_denoise_params *dn, const float4 *src,
                   float divisor, float *out, size_t outBytes);
+// the pieces of denoise(), in its order, which pt_denoise_temporal shares: the target's denoiser buffers; the guides and
+// k_denoise_prepare (ping = demodulated irradiance); k_denoise_variance of ping into pong; the K a-trous levels starting
+// from pong, the last one remodulating into ctx->denoised; and the copy to `out`, the synchronisation, the launch count
+// and the stack check
+pt_status allocDenoiseBuffers(Context *ctx);
+void launchDenoisePrepare(Context *ctx, const pt_render_params *params, const float4 *src, float divisor);
+void launchDenoiseVariance(Context *ctx, const pt_denoise_params *dn);
+void launchAtrous(Context *ctx, const pt_denoise_params *dn);
+pt_status finishDenoise(Context *ctx, const char *what, float *out, uint32_t launches);
+
+// temporal.cu
+pt_status denoiseTemporal(Context *ctx, const pt_render_params *params, const pt_denoise_params *dn, const pt_temporal_params *tp,
+                          uint32_t totalSamples, float *out, size_t outBytes);
+pt_status temporalHistory(Context *ctx, float *outIrradianceN, float *outMoments, size_t pixels);
 
 // postprocess.cu
 // src / divisor is the image the chain starts from: the accumulation and its sample count, or the denoised mean and 1

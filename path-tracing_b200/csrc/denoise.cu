@@ -201,60 +201,91 @@ pt_status checkDenoise(Context *ctx, const char *what, const pt_render_params *p
     return PT_OK;
 }
 
-pt_status denoise(Context *ctx, const char *what, const pt_render_params *params, const pt_denoise_params *dn, const float4 *src,
-                  float divisor, float *out, size_t outBytes)
+pt_status allocDenoiseBuffers(Context *ctx)
 {
-    const pt_status checked = checkDenoise(ctx, what, params, dn, divisor, out, outBytes);
-    if (checked != PT_OK)
-        return checked;
+    if (ctx->denoised)
+        return PT_OK;
+    // belongs to the target: freeTarget releases it with the accumulation
+    const size_t n = (size_t)ctx->width * ctx->height;
+    char *mem = nullptr;
+    PT_CUDA_CHECK(ctx, cudaMalloc((void **)&mem, n * (6 * sizeof(float4) + sizeof(float2))));
+    ctx->targetAllocs.push_back(mem);
+    float4 *f = reinterpret_cast<float4 *>(mem);
+    ctx->denoiseAlbedoT = f;
+    ctx->denoiseNormal = f + n;
+    ctx->denoised = f + 2 * n;
+    ctx->denoiseNT = f + 3 * n;
+    ctx->denoisePing = f + 4 * n;
+    ctx->denoisePong = f + 5 * n;
+    ctx->denoiseGrad = reinterpret_cast<float2 *>(f + 6 * n);
+    return PT_OK;
+}
+
+void launchDenoisePrepare(Context *ctx, const pt_render_params *params, const float4 *src, float divisor)
+{
     const uint32_t W = ctx->width, H = ctx->height;
-    const size_t n = (size_t)W * H;
-    if (!ctx->denoised)
-    {
-        // belongs to the target: freeTarget releases it with the accumulation
-        char *mem = nullptr;
-        PT_CUDA_CHECK(ctx, cudaMalloc((void **)&mem, n * (6 * sizeof(float4) + sizeof(float2))));
-        ctx->targetAllocs.push_back(mem);
-        float4 *f = reinterpret_cast<float4 *>(mem);
-        ctx->denoiseAlbedoT = f;
-        ctx->denoiseNormal = f + n;
-        ctx->denoised = f + 2 * n;
-        ctx->denoiseNT = f + 3 * n;
-        ctx->denoisePing = f + 4 * n;
-        ctx->denoisePong = f + 5 * n;
-        ctx->denoiseGrad = reinterpret_cast<float2 *>(f + 6 * n);
-    }
-    ctx->denoiseValid = false;
-    cudaStream_t st = ctx->stream;
     launchDenoiseGuides(ctx, params, ctx->denoiseAlbedoT, ctx->denoiseNormal);
     const dim3 block(32, 8), grid((W + 31) / 32, (H + 7) / 8);
-    k_denoise_prepare<<<grid, block, 0, st>>>(src, divisor, ctx->denoiseAlbedoT, ctx->denoiseNormal, W, H,
-                                              ctx->denoiseNT, ctx->denoisePing, ctx->denoiseGrad, ctx->denoised);
+    k_denoise_prepare<<<grid, block, 0, ctx->stream>>>(src, divisor, ctx->denoiseAlbedoT, ctx->denoiseNormal, W, H, ctx->denoiseNT,
+                                                       ctx->denoisePing, ctx->denoiseGrad, ctx->denoised);
+}
+
+void launchDenoiseVariance(Context *ctx, const pt_denoise_params *dn)
+{
+    const uint32_t W = ctx->width, H = ctx->height;
+    const dim3 block(32, 8), grid((W + 31) / 32, (H + 7) / 8);
+    k_denoise_variance<<<grid, block, 0, ctx->stream>>>(ctx->denoisePing, ctx->denoiseNT, ctx->denoiseGrad, W, H, dn->sigma_normal,
+                                                        dn->sigma_depth, ctx->denoisePong);
+}
+
+void launchAtrous(Context *ctx, const pt_denoise_params *dn)
+{
+    const uint32_t W = ctx->width, H = ctx->height;
+    const dim3 block(32, 8), grid((W + 31) / 32, (H + 7) / 8);
     const uint32_t K = dn->iterations;
-    if (K > 0)
+    float4 *a = ctx->denoisePong, *b = ctx->denoisePing;
+    for (uint32_t k = 0; k < K; k++)
     {
-        k_denoise_variance<<<grid, block, 0, st>>>(ctx->denoisePing, ctx->denoiseNT, ctx->denoiseGrad, W, H, dn->sigma_normal,
-                                                   dn->sigma_depth, ctx->denoisePong);
-        float4 *a = ctx->denoisePong, *b = ctx->denoisePing;
-        for (uint32_t k = 0; k < K; k++)
-        {
-            const bool last = k + 1 == K;
-            k_atrous<<<grid, block, 0, st>>>(a, ctx->denoiseNT, ctx->denoiseGrad, W, H, 1 << k, dn->sigma_luminance, dn->sigma_normal,
-                                             dn->sigma_depth, b, ctx->denoiseAlbedoT, last ? ctx->denoised : nullptr);
-            std::swap(a, b);
-        }
+        const bool last = k + 1 == K;
+        k_atrous<<<grid, block, 0, ctx->stream>>>(a, ctx->denoiseNT, ctx->denoiseGrad, W, H, 1 << k, dn->sigma_luminance, dn->sigma_normal,
+                                                  dn->sigma_depth, b, ctx->denoiseAlbedoT, last ? ctx->denoised : nullptr);
+        std::swap(a, b);
     }
+}
+
+pt_status finishDenoise(Context *ctx, const char *what, float *out, uint32_t launches)
+{
+    cudaStream_t st = ctx->stream;
     cudaError_t err = cudaGetLastError();
     if (err == cudaSuccess && out)
-        err = cudaMemcpyAsync(out, ctx->denoised, n * sizeof(float4), cudaMemcpyDeviceToHost, st);
+        err = cudaMemcpyAsync(out, ctx->denoised, (size_t)ctx->width * ctx->height * sizeof(float4), cudaMemcpyDeviceToHost, st);
     if (err == cudaSuccess)
         err = cudaStreamSynchronize(st);
     PT_CUDA_CHECK(ctx, err);
-    ctx->stats.kernel_launches = 2 + (K > 0 ? 1 + K : 0);
+    ctx->stats.kernel_launches = launches;
     const pt_status s = checkStackOverflow(ctx, what);
     if (s == PT_OK)
         ctx->denoiseValid = true;
     return s;
+}
+
+pt_status denoise(Context *ctx, const char *what, const pt_render_params *params, const pt_denoise_params *dn, const float4 *src,
+                  float divisor, float *out, size_t outBytes)
+{
+    pt_status s = checkDenoise(ctx, what, params, dn, divisor, out, outBytes);
+    if (s == PT_OK)
+        s = allocDenoiseBuffers(ctx);
+    if (s != PT_OK)
+        return s;
+    ctx->denoiseValid = false;
+    launchDenoisePrepare(ctx, params, src, divisor);
+    const uint32_t K = dn->iterations;
+    if (K > 0)
+    {
+        launchDenoiseVariance(ctx, dn);
+        launchAtrous(ctx, dn);
+    }
+    return finishDenoise(ctx, what, out, 2 + (K > 0 ? 1 + K : 0));
 }
 
 } // namespace pt

@@ -32,6 +32,10 @@ static void freeTarget(Context *ctx)
     ctx->denoisePing = ctx->denoisePong = nullptr;
     ctx->denoiseGrad = nullptr;
     ctx->denoiseValid = false;
+    ctx->temporalIrr[0] = ctx->temporalIrr[1] = ctx->temporalPrevNT = nullptr;
+    ctx->temporalMoments[0] = ctx->temporalMoments[1] = nullptr;
+    ctx->temporalCurrent = 0;
+    ctx->temporalValid = false;
     ctx->targetContent = Context::TargetContent::Empty;
     ctx->adaptivePixels = nullptr;
     ctx->adaptiveBlocks = nullptr;
@@ -204,6 +208,7 @@ pt_status pt_scene_upload(pt_context *ctx, const pt_scene_desc *scene)
 {
     if (!ctx)
         return PT_ERR_INVALID_ARGUMENT;
+    ctx->temporalValid = false; // the temporal denoiser's history shows the old scene
     DeviceGuard guard(ctx->device);
     return uploadScene(ctx, scene);
 }
@@ -212,6 +217,7 @@ pt_status pt_texture_upload(pt_context *ctx, uint32_t slot, const pt_texture_des
 {
     if (!ctx)
         return PT_ERR_INVALID_ARGUMENT;
+    ctx->temporalValid = false; // the temporal denoiser's history shows the old scene
     DeviceGuard guard(ctx->device);
     return uploadTextureSlot(ctx, slot, texture);
 }
@@ -331,6 +337,7 @@ pt_status pt_scene_update(pt_context *ctx, const pt_scene_update_desc *desc)
 {
     if (!ctx)
         return PT_ERR_INVALID_ARGUMENT;
+    ctx->temporalValid = false; // the temporal denoiser's history shows the old scene
     DeviceGuard guard(ctx->device);
     return updateScene(ctx, desc);
 }
@@ -384,6 +391,23 @@ pt_status pt_postprocess_denoised(pt_context *ctx, const pt_postprocess_params *
         return fail(ctx, PT_ERR_INVALID_ARGUMENT, "pt_postprocess_denoised", "no pt_denoise since the last pt_render_begin");
     DeviceGuard guard(ctx->device);
     return postProcess(ctx, "pt_postprocess_denoised", params, ctx->denoised, 1.0f, output_format, out_pixels, out_bytes);
+}
+
+pt_status pt_denoise_temporal(pt_context *ctx, const pt_render_params *params, const pt_denoise_params *denoise_params,
+                              const pt_temporal_params *temporal, uint32_t total_samples, float *out_rgba, size_t out_bytes)
+{
+    if (!ctx)
+        return PT_ERR_INVALID_ARGUMENT;
+    DeviceGuard guard(ctx->device);
+    return denoiseTemporal(ctx, params, denoise_params, temporal, total_samples, out_rgba, out_bytes);
+}
+
+pt_status pt_denoise_temporal_history(pt_context *ctx, float *out_irradiance_n, float *out_moments, size_t pixels)
+{
+    if (!ctx)
+        return PT_ERR_INVALID_ARGUMENT;
+    DeviceGuard guard(ctx->device);
+    return temporalHistory(ctx, out_irradiance_n, out_moments, pixels);
 }
 
 pt_status pt_render_adaptive(pt_context *ctx, const pt_render_params *params, const pt_adaptive_params *adaptive,
